@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the GP hot path on B200 (contract: task statement (4), SURVEY.md 8d).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2], "3-ref" of SURVEY.md 8d): SquaredExp()+SquaredExp()+WhiteNoise() (P = 19),
 N = 32768, D = 8, FP64.  One step = one NLML + gradient evaluation (log_loss_grad!, src/cost.jl:60-70) at the
@@ -18,6 +18,9 @@ next point of a fixed hyper-parameter trajectory (so nothing can be cached betwe
           component, dpotrf, dpotrs on the identity, per-hyper-parameter dK + dgemv + ddot) on the host cores: one
           calibration evaluation at N = 16384 (scale <= 8 to the metric's N) + the requested steps at the largest N
           that fits the time budget; ms_per_step is the time actually spent per executed step
+  --dump-outputs DIR : after the timed steps, rank 0 writes what its last timed evaluation returned, DIR/F.npy (shape (1,))
+          and DIR/G.npy (shape (P,)), float64.  The inputs come from fixed seeds, so two builds run with the same arguments
+          can be compared output for output.
 """
 import argparse
 import json
@@ -554,6 +557,12 @@ def config3_ext_and_training(_ffi, ctx, steps=2):
     return out
 
 
+def dump_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_gpu(args, rank, world, local_rank):
     import torch
     import gpr_sm100a as g
@@ -610,6 +619,8 @@ def run_gpu(args, rank, world, local_rank):
     t_wall = time.perf_counter() - t0
     launches = ctx.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"F": [F], "G": G})
     mh_route = mh.route()                     # product engine of the timed steps (digits of the INT8 route, 0 = DMMA)
     # device time of the K timed steps: event pair around every evaluation on the library stream, summed; max over ranks
     t_loc = stage["eval"] * 1e-3
@@ -809,7 +820,13 @@ def main():
     ap.add_argument("--no-sharded", action="store_true", help="skip the sharded extras (config 4 / config 5 / 3-ext / training)")
     ap.add_argument("--config5-n", type=int, default=None, help="override N of the config-5 extra (default 65536 for 1-2 GPUs, 131072 for 4-8)")
     ap.add_argument("--config5-base", action="store_true", help="1 GPU only: also run config 5 at N = 131072 in place on one GPU (strong-scaling base, ~2.5 min)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write F and G of the last timed evaluation (rank 0) to DIR/F.npy and DIR/G.npy, float64")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the GPU path (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

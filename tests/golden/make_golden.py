@@ -9,6 +9,7 @@ compares the CUDA path with committed numbers, not only with an oracle evaluated
 """
 import os
 import sys
+import zipfile
 
 import numpy as np
 
@@ -69,8 +70,16 @@ def make(name):
     return out
 
 
+def save(path, arrays):
+    """np.savez_compressed with LZMA in place of deflate (np.load reads both): se_se_noise_d8 stays under 1 MB."""
+    with zipfile.ZipFile(path, "w", compression=zipfile.ZIP_LZMA) as z:
+        for key, val in arrays.items():
+            with z.open(key + ".npy", "w") as f:
+                np.lib.format.write_array(f, np.asanyarray(val), allow_pickle=False)
+
+
 if __name__ == "__main__":
     for name in CASES:
         d = make(name)
-        np.savez_compressed(os.path.join(HERE, name + ".npz"), **d)
+        save(os.path.join(HERE, name + ".npz"), d)
         print(name, "cond(K) = %.2e" % d["cond"], "F =", d["F"])
