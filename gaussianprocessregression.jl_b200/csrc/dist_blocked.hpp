@@ -282,4 +282,97 @@ struct DistBlocked {
   }
 };
 
+// Posterior prediction (predict_mean! / predict!, src/predict.jl:36-102) from the K^-1 that lauum leaves block-cyclic in L.
+// A distributed triangular solve with U^T would be sequential over the ranks; the explicit inverse needs no solve.
+// Uu = upper triangle of K^-1 including its diagonal (L of every rank, zeros below), d = diag(K^-1), so
+// K^-1 = Uu + Uu^T - diag(d).  For one tile of mtp test points with Kt = K(x, xp) (Np x mtp, training index fastest,
+// padded rows zero) held by every rank, and g(b) = global row of local column b:
+//   T(i, b)  = sum_a Kt(a, i) Uu(a, b)                one T,N product per rank (column tile n contracts up to its global tile)
+//   T~(i, b) = T(i, b) - 1/2 d_b Kt(g(b), i)
+//   quad_i   = 2 sum_r sum_{b in r} T~(i, b) Kt(g(b), i)       = (Kt^T K^-1 Kt)(i, i)
+//   X        = sum_r T~_r Kt(g(local columns of r), :)      Kt^T K^-1 Kt = X + X^T   (dense covariance only)
+//   mean     = -Kt^T (y columns of the y owner, which hold -K^-1 Y after trtri)
+// Every rank writes its share into `red` = [quad partial (mtp) | mean (mtp x ny) | X (mtp x mtp, dense only)] (ranks
+// without the y columns or without blocks contribute zeros) and one sum over the ranks completes the tile.  Cost per
+// rank ~ mtp Np^2 / G flop, the single-device solve split G ways; communication is the one sum of `red`.
+//   BE (in addition to gemm / gemm_map / activate):
+//     be.pred_fixup(T, ldt, ncols, Kt, ldk, L, ld, lay, r, mtp, part, out, write_back)
+//                         out[i] = sum_b T~(i, b) Kt(g(b), i) over the ncols local columns (fixed order), T <- T~ if write_back
+//     be.copy2d(dst, ldd, src, lds, rows, cols)   be.zero(p, n)
+//   COMM:
+//     comm.sum_vec(count)  red of the FIRST local rank <- sum over all G ranks of red[0 .. count), in a fixed order
+template <class BE>
+struct DistPredRank {
+  int r = 0;
+  BE* be = nullptr;
+  const double* L = nullptr;   // Np x lcols(r), ld
+  int64_t ld = 0;
+  const int* gtile = nullptr;
+  const double* Kt = nullptr;  // Np x mtp, ld Np
+  double* T = nullptr;         // mtp x nloc(r) * nb
+  double* Ktl = nullptr;       // nloc(r) * nb x mtp: the rows of Kt at the rank's global blocks (dense only)
+  double* mscr = nullptr;      // mtp x nyp (y owner)
+  double* part = nullptr;      // per-CTA partial sums of the fix-up (backend-defined size)
+  double* red = nullptr;
+};
+
+template <class BE, class COMM>
+struct DistPredict {
+  DistLayout lay;
+  std::vector<DistPredRank<BE>>& ranks;
+  COMM& comm;
+  int64_t mtp = 0;
+  int ny = 1;
+  bool want_quad = true, dense = false;
+
+  DistPredict(const DistLayout& l, std::vector<DistPredRank<BE>>& rk, COMM& c, int64_t mtp_, int ny_, bool quad, bool dense_)
+      : lay(l), ranks(rk), comm(c), mtp(mtp_), ny(ny_), want_quad(quad || dense_), dense(dense_) {}
+
+  int64_t count() const { return mtp * (1 + ny) + (dense ? mtp * mtp : 0); }
+  int64_t ncols(int r) const { return lay.nloc(r) * lay.nb; }
+
+  void product() {
+    if (!want_quad) return;
+    for (auto& R : ranks) {
+      const int64_t n = ncols(R.r);
+      if (n <= 0) continue;
+      R.be->activate();
+      TileMap map{R.gtile, 0, 0};
+      R.be->gemm_map('T', 'N', mtp, n, lay.Np, 1.0, R.Kt, lay.Np, R.L, R.ld, 0.0, R.T, mtp, BLK_MAP_KUPTO, map);
+    }
+  }
+  void fixup() {
+    for (auto& R : ranks) {
+      R.be->activate();
+      const int64_t n = ncols(R.r);
+      if (!want_quad || n <= 0) R.be->zero(R.red, mtp);
+      else R.be->pred_fixup(R.T, mtp, n, R.Kt, lay.Np, R.L, R.ld, lay, R.r, mtp, R.part, R.red, dense);
+    }
+  }
+  void mean() {
+    for (auto& R : ranks) {
+      R.be->activate();
+      if (R.r == lay.y_owner()) {
+        R.be->gemm('T', 'N', mtp, lay.nyp, lay.Np, -1.0, R.Kt, lay.Np, R.L + lay.ycol0(R.r) * R.ld, R.ld, 0.0, R.mscr, mtp, 0);
+        R.be->copy2d(R.red + mtp, mtp, R.mscr, mtp, mtp, ny);
+      } else {
+        R.be->zero(R.red + mtp, mtp * ny);
+      }
+    }
+  }
+  void dense_product() {
+    if (!dense) return;
+    for (auto& R : ranks) {
+      R.be->activate();
+      const int64_t n = ncols(R.r);
+      double* X = R.red + mtp * (1 + ny);
+      if (n <= 0) { R.be->zero(X, mtp * mtp); continue; }
+      for (int64_t lb = 0; lb < lay.nloc(R.r); ++lb)
+        R.be->copy2d(R.Ktl + lb * lay.nb, n, R.Kt + lay.gblock(R.r, lb) * lay.nb, lay.Np, lay.nb, mtp);
+      R.be->gemm('N', 'N', mtp, mtp, n, 1.0, R.T, mtp, R.Ktl, n, 0.0, X, mtp, 0);
+    }
+  }
+  void reduce() { comm.sum_vec(count()); }
+};
+
 }  // namespace gpr

@@ -5,7 +5,7 @@ from . import _ffi  # noqa: F401
 from ._ffi import Context, GPRError, ModelHandle, MultiContext, MultiModelHandle, DistContext, PosDefException, get_context  # noqa: F401
 from .api import *  # noqa: F401,F403
 from .api import (Cmap, ComposedKernel, Diagonal, Euclidean, GPRModel, GPRPredictCache, GPRSplitPredictCache,  # noqa: F401
-                  LogScale, MarginalLikelihood, Matern52, MllGradCache, MllLossCache, MultiGPUGradCache, NoLogScale, SplitKernel,
+                  LogScale, MarginalLikelihood, Matern52, MllGradCache, MllLossCache, MultiGPUGradCache, MultiGPUPredictCache, NoLogScale, SplitKernel,
                   SquaredExp, UniformScaling, WhiteNoise, add_noise_, alloc_kernels, dim_hp, find_idx, get_sample,
                   grad, grad_, grad_cache, init_params, islog, kernel, kernel_, kernels, log_loss_grad_, loss,
                   loss_cache, loss_grad_, loss_grad_cache, predict, predict_, predict_cache, predict_mean,

@@ -73,6 +73,8 @@ _SIGS = {
     "gpr_mgpu_model_create": (C.c_int, [_vp, _ip, C.c_int, C.c_int, _i64, _dp, _dp, C.c_int, C.c_int, C.POINTER(_vp)]),
     "gpr_mgpu_model_destroy": (C.c_int, [_vp]),
     "gpr_mgpu_nlml_grad": (C.c_int, [_vp, _dp, C.c_int, C.c_int, C.c_double, _dp, _dp, C.POINTER(_i64)]),
+    "gpr_mgpu_update_cache": (C.c_int, [_vp, _dp, C.c_int, C.c_double, C.POINTER(_i64)]),
+    "gpr_mgpu_predict": (C.c_int, [_vp, _dp, _i64, C.c_int, _dp, _dp, _dp]),
     "gpr_mgpu_fetch": (C.c_int, [_vp, C.c_int, _dp]),
     "gpr_mgpu_timings": (C.c_int, [_vp, _dp, C.c_int]),
     "gpr_mgpu_dbg_factor": (C.c_int, [_vp, _dp, _i64, _dp, C.c_int, C.c_int, C.POINTER(_i64), _dp]),
@@ -528,6 +530,21 @@ class MultiModelHandle:
                                       C.byref(F) if want_f else None, dptr(G), C.byref(info))
         self.mctx.check(rc, info)
         return (F.value if want_f else None), G
+
+    def update_cache(self, hp, eps=1e-8, want_inverse=True):
+        """gpr_mgpu_update_cache: the prediction needs K^-1, so want_inverse (the single-device signature) is always true here."""
+        hp = f64(np.asarray(hp, dtype=np.float64).ravel())
+        info = _i64(0)
+        self.mctx.check(lib().gpr_mgpu_update_cache(self.handle, dptr(hp), hp.size, float(eps), C.byref(info)), info)
+
+    def predict(self, xp, same_x=False, want_var=False, want_cov=False):
+        xp = f64(xp)
+        M = int(xp.shape[1])
+        mean = np.empty((M, self.ny), order="F")
+        var = np.empty(M) if want_var else None
+        cov = np.empty((M, M), order="F") if want_cov else None
+        self.mctx.check(lib().gpr_mgpu_predict(self.handle, dptr(xp), M, int(bool(same_x)), dptr(mean), dptr(var), dptr(cov)))
+        return mean, var, cov
 
     def fetch(self, which):
         out = np.empty((self.N, self.N), order="F") if which == FETCH_KINV else np.empty(self.N)

@@ -297,7 +297,8 @@ class MllGradCache(_DeviceCache):
 class MultiGPUGradCache:
     """Gradient cache whose K / U / K^-1 are block-cyclic over several ranks (one per entry of `devices`;
     default: every visible GPU once): BASELINE.json config 5, SURVEY.md 8e.  Drop-in for MllGradCache in
-    loss_grad! / log_loss_grad! (src/cost.jl:50-70) and therefore in `train`."""
+    loss_grad! / log_loss_grad! (src/cost.jl:50-70) and therefore in `train`.  After an evaluation with a gradient it
+    also predicts (predict_mean_ / predict_) at that evaluation's hyper-parameters."""
     want_inverse = True
 
     def __init__(self, md, devices=None, nb=None):
@@ -332,6 +333,11 @@ class MultiGPUGradCache:
     def close(self):
         self.handle.close()
         self.mctx.close()
+
+
+class MultiGPUPredictCache(MultiGPUGradCache):
+    """Predict cache on the block-cyclic multi-GPU model (src/caches/predict.jl:3-31): update_cache_(pc, md) forms K^-1
+    over the ranks (no gradient), predict_mean_ / predict_ (Diagonal and dense) evaluate the posterior from it."""
 
 
 def loss_cache(cost):

@@ -227,7 +227,8 @@ int gpr_dist_create(int device, int rank, int world, const void* id128, int64_t 
  * in-process copies (test of that path on one GPU); set before creating a model.
  * "prefetch_trtri" / "prefetch_lauum": how the panels of the next step travel while the current step computes:
  * 0 = on the main queue before the step (no overlap), 1 = side queue with SM-driven peer reads, 2 = side queue through
- * the copy engines.  Default 2 for both (measured on 8 x B200, profiles/README.md). */
+ * the copy engines.  Default 2 for both (measured on 8 x B200, profiles/README.md).
+ * "predict_tile" and the "ozaki*" options are forwarded to every rank's context (meaning as in gpr_ctx_set_option). */
 int gpr_mgpu_set_option(gpr_mgpu* mg, const char* name, int64_t value);
 const char* gpr_mgpu_last_error(gpr_mgpu* mg);     /* mg may be NULL: last error of a failed gpr_mgpu_create */
 int64_t gpr_mgpu_launch_count(gpr_mgpu* mg);
@@ -238,6 +239,22 @@ int gpr_mgpu_model_destroy(gpr_mgpu_model* model);
 /* loss_grad! / log_loss_grad!: src/cost.jl:50-70 (same contract as gpr_nlml_grad) */
 int gpr_mgpu_nlml_grad(gpr_mgpu_model* model, const double* hp_in, int P, int log_scale, double eps, double* F,
                        double* G, int64_t* info);
+/* update_cache!(pc, md) of a predict cache on the multi-GPU model (src/predict.jl:29-34): covariance, potrf, trtri, lauum
+ * (K^-1 block-cyclic), K^-1 Y for all ny columns; no gradient reduction.  Collective; same contract and info as gpr_update_cache. */
+int gpr_mgpu_update_cache(gpr_mgpu_model* model, const double* hp, int P, double eps, int64_t* info);
+/* predict_mean! / predict! (src/predict.jl:36-102) from the K^-1 left by the last gpr_mgpu_update_cache, or by a
+ * gpr_mgpu_nlml_grad call with G != NULL, at that call's hp and eps.  GPR_ERR_STATE if there is none (no evaluation yet,
+ * loss-only evaluation, failed factorization).  Arguments and outputs exactly as gpr_predict (mean M x ny, var_diag and
+ * cov_full nullable, same_x = the reference's xp === md.x).  Collective: under gpr_dist_create every process passes the
+ * same xp and receives the same outputs.
+ * No triangular solve: with Uu the upper triangle of K^-1 (diagonal included) every rank forms T = K(x, xp)^T Uu for its
+ * own block columns, the variance is the quadratic form of K^-1 = Uu + Uu^T - diag(K^-1), and one sum of
+ * M (ny + 1) doubles (+ M^2 for cov_full) over the ranks finishes a tile.  Test points go in tiles of "predict_tile"
+ * (gpr_mgpu_set_option, default 16384), halved while a tile does not fit (GPR_ERR_MEMORY below 128 points); cov_full
+ * takes all M points in one tile.  Timings (gpr_mgpu_timings): PRED_KSTAR = K(x, xp) build on every rank, PRED_TRSM =
+ * the products, PRED_ROWNORM = the fix-up / row-dot kernel, PRED_MEAN = the sum over the ranks and the download. */
+int gpr_mgpu_predict(gpr_mgpu_model* model, const double* xp, int64_t M, int same_x, double* mean, double* var_diag,
+                     double* cov_full);
 /* GPR_FETCH_ALPHA (N) or GPR_FETCH_KINV (N x N full symmetric; after an evaluation with G != NULL) */
 int gpr_mgpu_fetch(gpr_mgpu_model* model, int which, double* out);
 int gpr_mgpu_timings(gpr_mgpu_model* model, double* ms, int n);   /* GPR_T_* slots; POTRS = alpha extraction + broadcast */

@@ -212,7 +212,8 @@ function mcheck(h::MultiHandle, rc::Cint, info::Int64 = 0)
 end
 default_nb(md) = size(md.x, 2) >= 65536 ? 2048 : 1024      # block-column width (DESIGN.md 7: 2048 feeds the INT8 route at large N)
 all_devices() = 0:(ccall((:gpr_device_count, LIB), Cint, ()) - 1)
-function SM100MultiGradCache(md::GPRModel; devices = all_devices(), nb::Integer = default_nb(md))
+"distributed model of `md` over `devices`: (handle, x snapshot, y snapshot)"
+function _multi_model(md::GPRModel, devices, nb::Integer)
     devs = Cint.(collect(devices))
     mg = Ref{Ptr{Cvoid}}(C_NULL)
     rc = ccall((:gpr_mgpu_create, LIB), Cint, (Cint, Ptr{Cint}, Int64, Ref{Ptr{Cvoid}}), length(devs), devs, nb, mg)
@@ -231,8 +232,10 @@ function SM100MultiGradCache(md::GPRModel; devices = all_devices(), nb::Integer 
         mg[], t, length(t), size(x, 1), size(x, 2), x, y, size(y, 2), md.train_axis, h)
     mcheck(mh, rc)
     mh.h = h[]
-    SM100MultiGradCache(Vector{Float64}(md.params), mh, x, y)
+    mh, x, y
 end
+SM100MultiGradCache(md::GPRModel; devices = all_devices(), nb::Integer = default_nb(md)) =
+    SM100MultiGradCache(Vector{Float64}(md.params), _multi_model(md, devices, nb)...)
 function _fg!(F, G, v, md, tc::SM100MultiGradCache, logscale::Bool)
     (md.x == tc.x && _ymat(md.y) == tc.y) || error("SM100MultiGradCache: x / y changed; build a new cache")
     f = Ref{Float64}(0.0); info = Ref{Int64}(0)
@@ -249,7 +252,8 @@ log_loss_grad!(::MarginalLikelihood, F, G, log_hp, md, tc::SM100MultiGradCache) 
 Wrapper that makes `train(SM100Multi(md; devices = 0:7), MarginalLikelihood(); method = LBFGS())` build the multi-GPU gradient
 cache: `loss_grad_cache(cost)(md)` (src/train.jl:38,49) is `MllGradCache(md)`, overloaded below.  Same supertype parameters as
 `SM100`, so `islog` (src/cost.jl:4-8) dispatches on the wrapped kernel.  First-order methods only (the distributed handle has no
-loss-only / predict path; use `SM100` for those).
+loss-only path; use `SM100` for that).  `predict(SM100Multi(md; devices = 0:7), xp)` predicts on the same devices
+(SM100MultiPredictCache below).
 """
 struct SM100Multi{K<:AbstractKernel,T,P<:AbstractArray{T},X<:AbstractArray{T,2},M<:GPRModel{K,T,P,X}} <: AbstractGPRModel{K,T,P,X}
     md::M
@@ -263,6 +267,36 @@ Base.propertynames(s::SM100Multi) = (:md, :devices, :nb, propertynames(getfield(
 Base.show(io::IO, m::MIME"text/plain", s::SM100Multi) = (println(io, "SM100Multi wrapper (devices ", Int.(s.devices), ") of"); show(io, m, s.md))
 GaussianProcessRegression.get_sample(s::SM100Multi) = get_sample(s.md)
 GaussianProcessRegression.MllGradCache(s::SM100Multi) = SM100MultiGradCache(s.md; devices = s.devices, nb = s.nb)
+
+# Prediction on the distributed model (src/predict.jl:14-102): update_cache! forms K^-1 block-cyclic over the devices,
+# gpr_mgpu_predict evaluates mean, Diagonal variance or dense covariance from it without a triangular solve.
+struct SM100MultiPredictCache <: AbstractPredictCache
+    h::MultiHandle
+    x::Matrix{Float64}
+    y::Matrix{Float64}
+end
+predict_cache(s::SM100Multi, ::AbstractArray) = (md, xp) -> SM100MultiPredictCache(_multi_model(s.md, s.devices, s.nb)...)
+function update_cache!(pc::SM100MultiPredictCache, md::AbstractGPRModel)
+    (md.x == pc.x && _ymat(md.y) == pc.y) || error("SM100MultiPredictCache: x / y changed; build a new cache")
+    hp = Vector{Float64}(md.params); info = Ref{Int64}(0)
+    rc = ccall((:gpr_mgpu_update_cache, LIB), Cint, (Ptr{Cvoid}, Ptr{Float64}, Cint, Cdouble, Ref{Int64}),
+        pc.h.h, hp, length(hp), 1e-8, info)
+    mcheck(pc.h, rc, info[])
+end
+function _mpredict!(pc::SM100MultiPredictCache, md, xp, μₚ, var, Σ)
+    rc = ccall((:gpr_mgpu_predict, LIB), Cint, (Ptr{Cvoid}, Ptr{Float64}, Int64, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+        pc.h.h, xp, size(xp, 2), xp === md.x, μₚ, var, Σ)
+    mcheck(pc.h, rc)
+end
+function predict_mean!(μₚ, md::SM100Multi, xp::AbstractMatrix, pc::SM100MultiPredictCache)
+    _mpredict!(pc, md, xp, μₚ, C_NULL, C_NULL)
+end
+function predict!(μₚ, Σₚ::Diagonal, md::SM100Multi, xp::AbstractMatrix, pc::SM100MultiPredictCache)
+    _mpredict!(pc, md, xp, μₚ, Σₚ.diag, C_NULL)
+end
+function predict!(μₚ, Σₚ::AbstractMatrix, md::SM100Multi, xp::AbstractMatrix, pc::SM100MultiPredictCache)
+    _mpredict!(pc, md, xp, μₚ, C_NULL, Σₚ)
+end
 
 # ---------------------------------------------------------------------------------------------------------
 # sample(N::NormalDistribution) on the device (src/distributions.jl:30-35): the draws stay on the Julia side (rng),
