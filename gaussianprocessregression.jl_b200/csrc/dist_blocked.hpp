@@ -324,11 +324,12 @@ struct DistPredict {
   int64_t mtp = 0;
   int ny = 1;
   bool want_quad = true, dense = false;
+  bool quad_only = false;   // red = [quad partial (mtp)] only, mean() is not called (split-predict variance rows)
 
   DistPredict(const DistLayout& l, std::vector<DistPredRank<BE>>& rk, COMM& c, int64_t mtp_, int ny_, bool quad, bool dense_)
       : lay(l), ranks(rk), comm(c), mtp(mtp_), ny(ny_), want_quad(quad || dense_), dense(dense_) {}
 
-  int64_t count() const { return mtp * (1 + ny) + (dense ? mtp * mtp : 0); }
+  int64_t count() const { return quad_only ? mtp : mtp * (1 + ny) + (dense ? mtp * mtp : 0); }
   int64_t ncols(int r) const { return lay.nloc(r) * lay.nb; }
 
   void product() {
@@ -373,6 +374,82 @@ struct DistPredict {
     }
   }
   void reduce() { comm.sum_vec(count()); }
+};
+
+// Split prediction (predict_mean! / predict!(mu, Sigma::Diagonal, md, Cmap(+, xe, xq), pc), src/split_predict.jl:5-53).
+// The mean mu = sum_k A_k .* (B_k diag(alpha) C_k) never touches K^-1, and every rank holds x and alpha: the q columns are
+// SHARDED.  A chunk of `cols` padded q columns (a multiple of 128) is cut into contiguous slabs of whole 128-column tiles, one
+// per rank (split_slab; with fewer tiles than ranks the last ranks get none).  Rank r builds A and Cw = diag(alpha) C for its
+// slab only and runs per component the T,N product with the Hadamard epilogue against its Bt (all e rows) -- the call the
+// single-device path makes for the same columns.  It writes its slab into `red` (nep x cols, zeros elsewhere) and one sum over
+// the ranks assembles the chunk: adding zeros is exact, so the chunk is what one rank computing it alone would give.
+// The var_range rows are ordinary test points: DistPredict with quad_only, in tiles of ec rows x w q columns (split_var_tile).
+//   BE (in addition to zero / activate):
+//     be.split_slab(q0, qn, A, Cw)   A (nep x qn x nk, ld nep) and Cw (Np x qn x nk, ld Np) of the padded q columns q0 .. q0+qn-1
+//     be.gemm_hadamard(M, N, K, A, lda, B, ldb, E, lde, beta, C, ldc)    C = (A^T B) .* E + beta C
+//   COMM: comm.sum_vec(count) as for DistPredict (`red` of the first local rank)
+inline void split_slab(int64_t cols, int G, int r, int64_t& q0, int64_t& qn) {
+  const int64_t tiles = cols / LEAF, base = tiles / G, extra = tiles % G;
+  q0 = (r * base + std::min<int64_t>(r, extra)) * LEAF;
+  qn = (base + (r < extra ? 1 : 0)) * LEAF;
+}
+
+// variance tile of at most mt points (mt: a multiple of 128): w q columns (every one when a whole row fits, else a multiple of
+// 128 of them) of up to eb of the erows variance rows
+inline void split_var_tile(int64_t mt, int64_t nqp, int64_t erows, int64_t& w, int64_t& eb) {
+  w = std::min<int64_t>(nqp, mt);
+  eb = std::min<int64_t>(erows, std::max<int64_t>(1, mt / w));
+}
+
+template <class BE>
+struct DistSplitRank {
+  int r = 0;
+  BE* be = nullptr;
+  const double* Bt = nullptr;   // Np x nep x nk: B^T of every e row (training index fastest)
+  double* A = nullptr;          // nep x (slab width) x nk
+  double* Cw = nullptr;         // Np x (slab width) x nk
+  double* red = nullptr;        // nep x cols
+};
+
+template <class BE, class COMM>
+struct DistSplitMean {
+  int G = 1, nk = 1;
+  int64_t Np = 0, nep = 0, nqp = 0;
+  std::vector<DistSplitRank<BE>>& ranks;
+  COMM& comm;
+
+  DistSplitMean(int G_, int nk_, int64_t Np_, int64_t nep_, int64_t nqp_, std::vector<DistSplitRank<BE>>& rk, COMM& c)
+      : G(G_), nk(nk_), Np(Np_), nep(nep_), nqp(nqp_), ranks(rk), comm(c) {}
+
+  // chunk width for slabs of at most `slab` columns per rank (slab: a multiple of 128)
+  int64_t chunk_cols(int64_t slab) const { return std::min<int64_t>(nqp, slab * G); }
+  // widest slab of a chunk of `cols` columns: what A and Cw must hold
+  int64_t max_slab(int64_t cols) const { return (cols / LEAF + G - 1) / G * LEAF; }
+
+  // chunk = padded q columns c0 .. c0 + cols - 1
+  void build(int64_t c0, int64_t cols) {
+    for (auto& R : ranks) {
+      int64_t q0, qn;
+      split_slab(cols, G, R.r, q0, qn);
+      if (qn <= 0) continue;
+      R.be->activate();
+      R.be->split_slab(c0 + q0, qn, R.A, R.Cw);
+    }
+  }
+  void product(int64_t cols) {
+    for (auto& R : ranks) {
+      int64_t q0, qn;
+      split_slab(cols, G, R.r, q0, qn);
+      R.be->activate();
+      if (q0 > 0) R.be->zero(R.red, q0 * nep);
+      for (int k = 0; k < nk; ++k)
+        if (qn > 0)
+          R.be->gemm_hadamard(nep, qn, Np, R.Bt + (int64_t)k * Np * nep, Np, R.Cw + (int64_t)k * Np * qn, Np, R.A + (int64_t)k * nep * qn,
+                              nep, k == 0 ? 0.0 : 1.0, R.red + q0 * nep, nep);
+      if (q0 + qn < cols) R.be->zero(R.red + (q0 + qn) * nep, (cols - q0 - qn) * nep);
+    }
+  }
+  void reduce(int64_t cols) { comm.sum_vec(nep * cols); }
 };
 
 }  // namespace gpr

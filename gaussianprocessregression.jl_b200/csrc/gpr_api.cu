@@ -1284,10 +1284,13 @@ int split_build(gpr_ctx* ctx, const KSpec& spec, int D, const double* d_hp, cons
     one.ncomp = 1; one.type[0] = spec.type[c]; one.hp_off[0] = spec.hp_off[c];
     KBuildArgs a{};
     a.D = D; a.hp = d_hp; a.spec = one; a.eps = 0.0; a.same = 0; a.add_noise = 0; a.pad_identity = 0; a.diag_shift = 0;
-    // A[:, :, k] = exp(-sum (l xq)^2 - 2 sum l^2 xe xq), sigma := 1   (split_kernel.jl:152-155)
-    a.out = sb.A + (int64_t)k * nep * nqp; a.ldo = nep; a.R = ne; a.C = nq; a.Rp = nep; a.Cp = nqp;
-    a.x1 = d_xe; a.x2 = d_xq; a.sigma_one = 1; a.row_scale = nullptr;
-    int rc = launch_kbuild(ctx, DM_SPLIT_A, a); if (rc) return rc;
+    // A[:, :, k] = exp(-sum (l xq)^2 - 2 sum l^2 xe xq), sigma := 1   (split_kernel.jl:152-155); skipped when sb.A is NULL
+    int rc = GPR_OK;
+    if (sb.A) {
+      a.out = sb.A + (int64_t)k * nep * nqp; a.ldo = nep; a.R = ne; a.C = nq; a.Rp = nep; a.Cp = nqp;
+      a.x1 = d_xe; a.x2 = d_xq; a.sigma_one = 1; a.row_scale = nullptr;
+      rc = launch_kbuild(ctx, DM_SPLIT_A, a); if (rc) return rc;
+    }
     // B[:, :, k] = exp(-|l (xe - xs)|^2), sigma := 1                    (split_kernel.jl:156)
     if (want_B) {
       a.out = sb.B + (int64_t)k * nep * Np; a.ldo = nep; a.R = ne; a.C = N; a.Rp = nep; a.Cp = Np;

@@ -75,6 +75,7 @@ _SIGS = {
     "gpr_mgpu_nlml_grad": (C.c_int, [_vp, _dp, C.c_int, C.c_int, C.c_double, _dp, _dp, C.POINTER(_i64)]),
     "gpr_mgpu_update_cache": (C.c_int, [_vp, _dp, C.c_int, C.c_double, C.POINTER(_i64)]),
     "gpr_mgpu_predict": (C.c_int, [_vp, _dp, _i64, C.c_int, _dp, _dp, _dp]),
+    "gpr_mgpu_split_predict": (C.c_int, [_vp, _dp, _i64, _dp, _i64, _i64, _i64, _dp, _dp]),
     "gpr_mgpu_fetch": (C.c_int, [_vp, C.c_int, _dp]),
     "gpr_mgpu_timings": (C.c_int, [_vp, _dp, C.c_int]),
     "gpr_mgpu_dbg_factor": (C.c_int, [_vp, _dp, _i64, _dp, C.c_int, C.c_int, C.POINTER(_i64), _dp]),
@@ -283,15 +284,7 @@ class ModelHandle:
     def split_predict(self, xe, xq, var_range=None, want_var=True, mean_out=None, var_out=None):
         """mean_out / var_out: caller-owned result arrays (the reference's predict!(mu, Sigma, ...) writes in place too); a fresh
         134 MB array per call costs more in first-touch page faults under the device-to-host copy than the whole computation."""
-        xe, xq = f64(xe), f64(xq)
-        ne, nq = int(xe.shape[1]), int(xq.shape[1])
-        if mean_out is not None and (mean_out.shape != (ne, nq) or mean_out.dtype != np.float64 or not mean_out.flags.f_contiguous):
-            raise GPRError("mean_out must be a Fortran-ordered float64 array of shape (ne, nq)")
-        if var_out is not None and (var_out.shape != (ne * nq,) or var_out.dtype != np.float64 or not var_out.flags.c_contiguous):
-            raise GPRError("var_out must be a contiguous float64 vector of length ne * nq")
-        mean = mean_out if mean_out is not None else np.empty((ne, nq), order="F")
-        var = (var_out if var_out is not None else np.empty(ne * nq)) if want_var else None
-        lo, hi = (1, 0) if var_range is None else (int(var_range[0]), int(var_range[1]))
+        xe, ne, xq, nq, lo, hi, mean, var = _split_args(xe, xq, var_range, want_var, mean_out, var_out)
         self.ctx.check(lib().gpr_split_predict(self.handle, dptr(xe), ne, dptr(xq), nq, lo, hi, dptr(mean), dptr(var)))
         return mean, var
 
@@ -325,6 +318,21 @@ class ModelHandle:
             self.close()
         except Exception:
             pass
+
+
+def _split_args(xe, xq, var_range, want_var, mean_out, var_out):
+    """(xe, ne, xq, nq, e_lo, e_hi, mean, var) of gpr_split_predict / gpr_mgpu_split_predict; mean and var are the caller's
+    arrays when given (checked), fresh ones otherwise (var None unless want_var)."""
+    xe, xq = f64(xe), f64(xq)
+    ne, nq = int(xe.shape[1]), int(xq.shape[1])
+    if mean_out is not None and (mean_out.shape != (ne, nq) or mean_out.dtype != np.float64 or not mean_out.flags.f_contiguous):
+        raise GPRError("mean_out must be a Fortran-ordered float64 array of shape (ne, nq)")
+    if var_out is not None and (var_out.shape != (ne * nq,) or var_out.dtype != np.float64 or not var_out.flags.c_contiguous):
+        raise GPRError("var_out must be a contiguous float64 vector of length ne * nq")
+    mean = mean_out if mean_out is not None else np.empty((ne, nq), order="F")
+    var = (var_out if var_out is not None else np.empty(ne * nq)) if want_var else None
+    lo, hi = (1, 0) if var_range is None else (int(var_range[0]), int(var_range[1]))
+    return xe, ne, xq, nq, lo, hi, mean, var
 
 
 def kernel_matrix(ctx, types, D, hp, x, xp, same_x, eps, add_noise):
@@ -545,6 +553,12 @@ class MultiModelHandle:
         cov = np.empty((M, M), order="F") if want_cov else None
         self.mctx.check(lib().gpr_mgpu_predict(self.handle, dptr(xp), M, int(bool(same_x)), dptr(mean), dptr(var), dptr(cov)))
         return mean, var, cov
+
+    def split_predict(self, xe, xq, var_range=None, want_var=True, mean_out=None, var_out=None):
+        """gpr_mgpu_split_predict; arguments, results and in-place semantics as ModelHandle.split_predict"""
+        xe, ne, xq, nq, lo, hi, mean, var = _split_args(xe, xq, var_range, want_var, mean_out, var_out)
+        self.mctx.check(lib().gpr_mgpu_split_predict(self.handle, dptr(xe), ne, dptr(xq), nq, lo, hi, dptr(mean), dptr(var)))
+        return mean, var
 
     def fetch(self, which):
         out = np.empty((self.N, self.N), order="F") if which == FETCH_KINV else np.empty(self.N)

@@ -298,10 +298,12 @@ class MultiGPUGradCache:
     """Gradient cache whose K / U / K^-1 are block-cyclic over several ranks (one per entry of `devices`;
     default: every visible GPU once): BASELINE.json config 5, SURVEY.md 8e.  Drop-in for MllGradCache in
     loss_grad! / log_loss_grad! (src/cost.jl:50-70) and therefore in `train`.  After an evaluation with a gradient it
-    also predicts (predict_mean_ / predict_) at that evaluation's hyper-parameters."""
+    also predicts (predict_mean_ / predict_, general test points or Cmap grids) at that evaluation's hyper-parameters;
+    var_range: the rows e of a Cmap grid that get the posterior variance (1-based inclusive, as GPRSplitPredictCache)."""
     want_inverse = True
 
-    def __init__(self, md, devices=None, nb=None):
+    def __init__(self, md, devices=None, nb=None, var_range=(1, 3)):
+        self.var_range = var_range
         if devices is None:
             devices = list(range(max(1, _ffi.device_count())))
         if nb is None:
@@ -337,7 +339,8 @@ class MultiGPUGradCache:
 
 class MultiGPUPredictCache(MultiGPUGradCache):
     """Predict cache on the block-cyclic multi-GPU model (src/caches/predict.jl:3-31): update_cache_(pc, md) forms K^-1
-    over the ranks (no gradient), predict_mean_ / predict_ (Diagonal and dense) evaluate the posterior from it."""
+    over the ranks (no gradient), predict_mean_ / predict_ (Diagonal and dense; Cmap grids with Diagonal) evaluate the
+    posterior from it."""
 
 
 def loss_cache(cost):

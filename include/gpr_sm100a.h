@@ -228,7 +228,8 @@ int gpr_dist_create(int device, int rank, int world, const void* id128, int64_t 
  * "prefetch_trtri" / "prefetch_lauum": how the panels of the next step travel while the current step computes:
  * 0 = on the main queue before the step (no overlap), 1 = side queue with SM-driven peer reads, 2 = side queue through
  * the copy engines.  Default 2 for both (measured on 8 x B200, profiles/README.md).
- * "predict_tile" and the "ozaki*" options are forwarded to every rank's context (meaning as in gpr_ctx_set_option). */
+ * "predict_tile" and the "ozaki*" options (incl. "ozaki_split") are forwarded to every rank's context (meaning as in
+ * gpr_ctx_set_option). */
 int gpr_mgpu_set_option(gpr_mgpu* mg, const char* name, int64_t value);
 const char* gpr_mgpu_last_error(gpr_mgpu* mg);     /* mg may be NULL: last error of a failed gpr_mgpu_create */
 int64_t gpr_mgpu_launch_count(gpr_mgpu* mg);
@@ -255,6 +256,22 @@ int gpr_mgpu_update_cache(gpr_mgpu_model* model, const double* hp, int P, double
  * the products, PRED_ROWNORM = the fix-up / row-dot kernel, PRED_MEAN = the sum over the ranks and the download. */
 int gpr_mgpu_predict(gpr_mgpu_model* model, const double* xp, int64_t M, int same_x, double* mean, double* var_diag,
                      double* cov_full);
+/* predict_mean! / predict!(mu, Sigma::Diagonal, md, Cmap(+, xe, xq), pc) (src/split_predict.jl:5-53) on the multi-GPU model.
+ * Arguments and outputs exactly as gpr_split_predict (mean ne x nq, e fastest; var nullable, ne*nq entries, q fastest within e;
+ * rows e in [e_lo, e_hi] get the posterior variance, all others keep the prior; e_lo = e_hi + 1: no variance rows); the
+ * preconditions of gpr_mgpu_predict (GPR_ERR_STATE unless predict-ready, at that factorization's hp and eps), GPR_ERR_UNSUPPORTED
+ * for ny != 1.  Collective like gpr_mgpu_predict.
+ * Mean: nothing in mu = sum_k A_k .* (B_k diag(alpha) C_k) touches K^-1 and every rank holds x and alpha, so the q columns are
+ * sharded: a chunk of q columns is cut into one slab of whole 128-column tiles per rank, every rank builds B^T for all e rows
+ * and A, diag(alpha) C for its slab and runs the Hadamard-epilogue products of gpr_split_predict, and one sum over the ranks
+ * (zeros outside each slab) assembles the chunk.  Slabs hold at most "predict_tile" columns and are halved while they do not
+ * fit (GPR_ERR_MEMORY below 128).  With "ozaki" = 0 the mean does not depend on the number of ranks, the transport or the slab
+ * width.  Variance rows: ordinary test points through the quadratic form of gpr_mgpu_predict, in tiles of at most
+ * "predict_tile" points (whole rows e when one fits, else a slab of a row's q columns), halved while they do not fit.
+ * Timings: SPLIT_BUILD / SPLIT_GEMM / SPLIT_D2H (incl. the sum over the ranks) for the mean, PRED_KSTAR / PRED_TRSM /
+ * PRED_ROWNORM / PRED_MEAN for the variance rows as in gpr_mgpu_predict. */
+int gpr_mgpu_split_predict(gpr_mgpu_model* model, const double* xe, int64_t ne, const double* xq, int64_t nq, int64_t e_lo,
+                           int64_t e_hi, double* mean, double* var);
 /* GPR_FETCH_ALPHA (N) or GPR_FETCH_KINV (N x N full symmetric; after an evaluation with G != NULL) */
 int gpr_mgpu_fetch(gpr_mgpu_model* model, int which, double* out);
 int gpr_mgpu_timings(gpr_mgpu_model* model, double* ms, int n);   /* GPR_T_* slots; POTRS = alpha extraction + broadcast */

@@ -253,7 +253,7 @@ Wrapper that makes `train(SM100Multi(md; devices = 0:7), MarginalLikelihood(); m
 cache: `loss_grad_cache(cost)(md)` (src/train.jl:38,49) is `MllGradCache(md)`, overloaded below.  Same supertype parameters as
 `SM100`, so `islog` (src/cost.jl:4-8) dispatches on the wrapped kernel.  First-order methods only (the distributed handle has no
 loss-only path; use `SM100` for that).  `predict(SM100Multi(md; devices = 0:7), xp)` predicts on the same devices
-(SM100MultiPredictCache below).
+(SM100MultiPredictCache below; SM100MultiSplitPredictCache for `xp::Cmap`).
 """
 struct SM100Multi{K<:AbstractKernel,T,P<:AbstractArray{T},X<:AbstractArray{T,2},M<:GPRModel{K,T,P,X}} <: AbstractGPRModel{K,T,P,X}
     md::M
@@ -276,7 +276,15 @@ struct SM100MultiPredictCache <: AbstractPredictCache
     y::Matrix{Float64}
 end
 predict_cache(s::SM100Multi, ::AbstractArray) = (md, xp) -> SM100MultiPredictCache(_multi_model(s.md, s.devices, s.nb)...)
-function update_cache!(pc::SM100MultiPredictCache, md::AbstractGPRModel)
+# split prediction on Cmap(+, xe, xq) grids (src/split_predict.jl:5-53): gpr_mgpu_split_predict shards the q columns over the devices
+struct SM100MultiSplitPredictCache <: AbstractPredictCache
+    h::MultiHandle
+    x::Matrix{Float64}
+    y::Matrix{Float64}
+    var_range::UnitRange{Int64}
+end
+predict_cache(s::SM100Multi, ::Cmap) = (md, xp) -> SM100MultiSplitPredictCache(_multi_model(s.md, s.devices, s.nb)..., 1:3)
+function update_cache!(pc::Union{SM100MultiPredictCache,SM100MultiSplitPredictCache}, md::AbstractGPRModel)
     (md.x == pc.x && _ymat(md.y) == pc.y) || error("SM100MultiPredictCache: x / y changed; build a new cache")
     hp = Vector{Float64}(md.params); info = Ref{Int64}(0)
     rc = ccall((:gpr_mgpu_update_cache, LIB), Cint, (Ptr{Cvoid}, Ptr{Float64}, Cint, Cdouble, Ref{Int64}),
@@ -296,6 +304,18 @@ function predict!(μₚ, Σₚ::Diagonal, md::SM100Multi, xp::AbstractMatrix, pc
 end
 function predict!(μₚ, Σₚ::AbstractMatrix, md::SM100Multi, xp::AbstractMatrix, pc::SM100MultiPredictCache)
     _mpredict!(pc, md, xp, μₚ, C_NULL, Σₚ)
+end
+function _msplit!(pc::SM100MultiSplitPredictCache, xeq::Cmap, e_lo, e_hi, μₚ, var)
+    rc = ccall((:gpr_mgpu_split_predict, LIB), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Ptr{Float64}, Int64, Int64, Int64, Ptr{Float64}, Ptr{Float64}),
+        pc.h.h, xeq.xe, size(xeq.xe, 2), xeq.xq, size(xeq.xq, 2), e_lo, e_hi, μₚ, var)
+    mcheck(pc.h, rc)
+end
+function predict_mean!(μₚ, md::SM100Multi, xeq::Cmap, pc::SM100MultiSplitPredictCache)
+    _msplit!(pc, xeq, 1, 0, μₚ, C_NULL)
+end
+function predict!(μₚ, Σₚ::Diagonal, md::SM100Multi, xeq::Cmap, pc::SM100MultiSplitPredictCache)
+    _msplit!(pc, xeq, first(pc.var_range), last(pc.var_range), μₚ, Σₚ.diag)
 end
 
 # ---------------------------------------------------------------------------------------------------------
