@@ -104,6 +104,15 @@ struct gpr_ctx {
   cudaEvent_t ev_chunk[4] = {nullptr, nullptr, nullptr, nullptr};   // split predict: chunk-ready events for the overlapped download
   cudaEvent_t ev_d2h[4] = {nullptr, nullptr, nullptr, nullptr};     // ... and chunk-downloaded events (pinned staging buffer)
   double* h_stage = nullptr; size_t h_stage_elems = 0;              // pinned staging buffer of the split-predict mean
+  // h_stage grown to `elems` doubles if that is at most 1 GB; nullptr when the buffer is smaller and cannot be grown
+  double* host_stage(size_t elems) {
+    if (elems > h_stage_elems && elems * sizeof(double) <= ((size_t)1 << 30)) {
+      if (h_stage) { cudaFreeHost(h_stage); h_stage = nullptr; h_stage_elems = 0; }
+      if (cudaMallocHost(&h_stage, elems * sizeof(double)) == cudaSuccess) h_stage_elems = elems;
+      else { cudaGetLastError(); h_stage = nullptr; }
+    }
+    return h_stage_elems >= elems ? h_stage : nullptr;
+  }
 };
 
 namespace {
@@ -388,6 +397,14 @@ int kbuild_rows_per_cta(gpr_ctx* ctx, const KBuildArgs& a) {
 struct DevBuf {
   double* p = nullptr;
   size_t n = 0;   // elements
+  // grow to hold `need` doubles (no-op when it already does); false on an allocation failure, whose CUDA error is cleared
+  bool grow(size_t need) {
+    if (need <= n) return true;
+    cudaFree(p); p = nullptr; n = 0;
+    if (cudaMalloc(&p, need * sizeof(double)) != cudaSuccess) { cudaGetLastError(); return false; }
+    n = need;
+    return true;
+  }
 };
 
 }  // namespace
@@ -478,21 +495,29 @@ int check_pending(gpr_ctx* ctx, const char* where) {
 // predictive mean 4e-3 against 6e-6 on the DMMA pipe, tests/test_extended_precision.py with GPR_OZAKI_MIN=128).
 // Automatic mode therefore bounds the condition number from the hyper-parameters,
 //   cond(K) <= (N * sum_c sigma_c^2 + sigma_n^2 + nk * eps) / (sigma_n^2 + nk * eps),
-// and takes the INT8 route only below 1e8 (the benchmark model: 4e6).
-int ozaki_digits_for(const gpr_model* m, const double* hp, double eps) {
-  const gpr_ctx* ctx = m->ctx;
-  if (ctx->ozaki >= 0) return ctx->ozaki;
+// and takes the INT8 route only below 1e8 (the benchmark model: 4e6).  Shared with the multi-GPU model (mgpu_factor).
+int ozaki_auto_digits(const KSpec& spec, int nk, int64_t N, const double* hp, double eps) {
   double sig2 = 0.0, noise2 = 0.0;
   bool have_noise = false;
-  for (int c = 0; c < m->ncomp; ++c) {
-    const double v = hp[m->spec.hp_off[c]];
-    if (m->spec.type[c] == KT_NOISE) { if (!have_noise) { noise2 = v * v; have_noise = true; } }
+  for (int c = 0; c < spec.ncomp; ++c) {
+    const double v = hp[spec.hp_off[c]];
+    if (spec.type[c] == KT_NOISE) { if (!have_noise) { noise2 = v * v; have_noise = true; } }
     else sig2 += v * v;
   }
-  const double floor_ = noise2 + m->nk * eps;
+  const double floor_ = noise2 + nk * eps;
   if (!(floor_ > 0.0)) return 0;
-  const double bound = ((double)m->N * sig2 + floor_) / floor_;
+  const double bound = ((double)N * sig2 + floor_) / floor_;
   return bound <= 1e8 ? 8 : 0;
+}
+int ozaki_digits_for(const gpr_model* m, const double* hp, double eps) {
+  return m->ctx->ozaki >= 0 ? m->ctx->ozaki : ozaki_auto_digits(m->spec, m->nk, m->N, hp, eps);
+}
+
+// prior variance of a test point: sum over ALL components (noise included) of hp_c[1]^2, no jitter (src/predict.jl:55-58,67)
+double prior_var(const KSpec& spec, const double* hp) {
+  double s = 0.0;
+  for (int c = 0; c < spec.ncomp; ++c) { const double v = hp[spec.hp_off[c]]; s += v * v; }
+  return s;
 }
 
 // K (+ noise, + jitter, identity padding) into m->d_U, then blocked potrf; solves for all y columns.
@@ -1089,13 +1114,6 @@ int gpr_timings(gpr_model* m, double* ms, int n) {
 // ---------------------------------------------------------------------------
 namespace {
 
-double prior_diag(const gpr_model* m) {
-  // sum over ALL components (noise included) of hp_c[1]^2, no jitter (src/predict.jl:55-58,67)
-  double s = 0.0;
-  for (int c = 0; c < m->ncomp; ++c) { const double v = m->hp_host[m->spec.hp_off[c]]; s += v * v; }
-  return s;
-}
-
 // One tile of test points resident on the device: d_xp is D x mt (mt valid points, global index m0..m0+mt).
 // Writes mean (mt x ny, column stride ldmean) and var (mt) to device memory.
 int predict_tile(gpr_model* m, const double* d_xp, int64_t mt, int64_t m0, int same_x, double* d_mean, int64_t ldmean,
@@ -1158,7 +1176,7 @@ int predict_tile(gpr_model* m, const double* d_xp, int64_t mt, int64_t m0, int s
     }
     {
       Scope s(m->tm, GPR_T_PRED_ROWNORM, ctx->stream);
-      colsumsq_kernel<<<(unsigned)mt, 256, 0, ctx->stream>>>(Kt, Np, Np, mt, prior_diag(m), d_var);   // predict.jl:91-93
+      colsumsq_kernel<<<(unsigned)mt, 256, 0, ctx->stream>>>(Kt, Np, Np, mt, prior_var(m->spec, m->hp_host.data()), d_var);   // predict.jl:91-93
       ctx->launches++;
       CK(cudaGetLastError());
     }
@@ -1261,6 +1279,7 @@ namespace {
 struct SplitBufs {
   double *A = nullptr, *B = nullptr, *C = nullptr;   // per non-noise component slices
   double *Bt = nullptr, *Cu = nullptr;               // variance path: B transposed (Np x nep x k), C unscaled (Np x nqp x k)
+  const double* C_row_scale = nullptr;               // rows of C scaled by it (device, Np; nullptr: unscaled)
   double *d_xe = nullptr, *d_xq = nullptr;
   int64_t nep = 0, nqp = 0;
   void release() {
@@ -1269,13 +1288,11 @@ struct SplitBufs {
   }
 };
 
-// Builds A (nep x nqp x k), B (nep x Np x k) and, per request, C (Np x nqp x k; optionally row-scaled by wt)
-// and, for the variance, Bt (Np x nep x k) and the unscaled Cu (Np x nqp x k): the training index fastest, the layout the
-// transposed tile assembly reads coalesced.  d_hp: device global hp.  x: D x N device.
+// Builds each of A (nep x nqp x k), B (nep x Np x k), C (Np x nqp x k; rows scaled by sb.C_row_scale if set) and, for the
+// variance, Bt (Np x nep x k) and the unscaled Cu (Np x nqp x k) whose buffer in sb is not NULL: Bt and Cu with the training
+// index fastest, the layout the transposed tile assembly reads coalesced.  d_hp: device global hp.  x: D x N device.
 int split_build(gpr_ctx* ctx, const KSpec& spec, int D, const double* d_hp, const double* d_xe, int64_t ne,
-                const double* d_xq, int64_t nq, const double* d_x, int64_t N, int64_t Np, double eps, SplitBufs& sb,
-                bool want_B, bool want_C, const double* c_row_scale, bool want_Cu, bool want_Bt) {
-  (void)eps;
+                const double* d_xq, int64_t nq, const double* d_x, int64_t N, int64_t Np, const SplitBufs& sb) {
   const int64_t nep = sb.nep, nqp = sb.nqp;
   int k = 0;
   for (int c = 0; c < spec.ncomp; ++c) {
@@ -1284,7 +1301,7 @@ int split_build(gpr_ctx* ctx, const KSpec& spec, int D, const double* d_hp, cons
     one.ncomp = 1; one.type[0] = spec.type[c]; one.hp_off[0] = spec.hp_off[c];
     KBuildArgs a{};
     a.D = D; a.hp = d_hp; a.spec = one; a.eps = 0.0; a.same = 0; a.add_noise = 0; a.pad_identity = 0; a.diag_shift = 0;
-    // A[:, :, k] = exp(-sum (l xq)^2 - 2 sum l^2 xe xq), sigma := 1   (split_kernel.jl:152-155); skipped when sb.A is NULL
+    // A[:, :, k] = exp(-sum (l xq)^2 - 2 sum l^2 xe xq), sigma := 1   (split_kernel.jl:152-155)
     int rc = GPR_OK;
     if (sb.A) {
       a.out = sb.A + (int64_t)k * nep * nqp; a.ldo = nep; a.R = ne; a.C = nq; a.Rp = nep; a.Cp = nqp;
@@ -1292,23 +1309,23 @@ int split_build(gpr_ctx* ctx, const KSpec& spec, int D, const double* d_hp, cons
       rc = launch_kbuild(ctx, DM_SPLIT_A, a); if (rc) return rc;
     }
     // B[:, :, k] = exp(-|l (xe - xs)|^2), sigma := 1                    (split_kernel.jl:156)
-    if (want_B) {
+    if (sb.B) {
       a.out = sb.B + (int64_t)k * nep * Np; a.ldo = nep; a.R = ne; a.C = N; a.Rp = nep; a.Cp = Np;
       a.x1 = d_xe; a.x2 = d_x; a.sigma_one = 1;
       rc = launch_kbuild(ctx, DM_EUCLID, a, d_x); if (rc) return rc;
     }
     // C[:, :, k] = sigma^2 exp(+2 sum l^2 xs xq)                         (split_kernel.jl:157)
-    if (want_C) {
+    if (sb.C) {
       a.out = sb.C + (int64_t)k * Np * nqp; a.ldo = Np; a.R = N; a.C = nq; a.Rp = Np; a.Cp = nqp;
-      a.x1 = d_x; a.x2 = d_xq; a.sigma_one = 0; a.row_scale = c_row_scale;
+      a.x1 = d_x; a.x2 = d_xq; a.sigma_one = 0; a.row_scale = sb.C_row_scale;
       rc = launch_kbuild(ctx, DM_SPLIT_C, a); if (rc) return rc;
     }
-    if (want_Cu) {
+    if (sb.Cu) {
       a.out = sb.Cu + (int64_t)k * Np * nqp; a.ldo = Np; a.R = N; a.C = nq; a.Rp = Np; a.Cp = nqp;
       a.x1 = d_x; a.x2 = d_xq; a.sigma_one = 0; a.row_scale = nullptr;
       rc = launch_kbuild(ctx, DM_SPLIT_C, a); if (rc) return rc;
     }
-    if (want_Bt) {
+    if (sb.Bt) {
       a.out = sb.Bt + (int64_t)k * Np * nep; a.ldo = Np; a.R = N; a.C = ne; a.Rp = Np; a.Cp = nep;
       a.x1 = d_x; a.x2 = d_xe; a.sigma_one = 1; a.row_scale = nullptr;
       rc = launch_kbuild(ctx, DM_EUCLID, a, d_x); if (rc) return rc;   // B is symmetric in its two point sets: Bt[s, e] = B[e, s]
@@ -1346,7 +1363,7 @@ int gpr_split_kernel(gpr_ctx* ctx, const int* comp_types, int ncomp, int D, cons
   if (e == cudaSuccess) e = cudaMemcpyAsync(d_hp, hp, sizeof(double) * P, cudaMemcpyHostToDevice, ctx->stream);
   rc = GPR_OK;
   if (e == cudaSuccess) {
-    rc = split_build(ctx, spec, D, d_hp, sb.d_xe, ne, sb.d_xq, nq, d_x, N, N, 0.0, sb, true, true, nullptr, false, false);
+    rc = split_build(ctx, spec, D, d_hp, sb.d_xe, ne, sb.d_xq, nq, d_x, N, N, sb);
     if (!rc) e = cudaMemcpyAsync(A, sb.A, sizeof(double) * ne * nq * nk, cudaMemcpyDeviceToHost, ctx->stream);
     if (!rc && e == cudaSuccess) e = cudaMemcpyAsync(B, sb.B, sizeof(double) * ne * N * nk, cudaMemcpyDeviceToHost, ctx->stream);
     if (!rc && e == cudaSuccess) e = cudaMemcpyAsync(C, sb.C, sizeof(double) * N * nq * nk, cudaMemcpyDeviceToHost, ctx->stream);
@@ -1384,7 +1401,7 @@ int gpr_split_predict(gpr_model* m, const double* xe, int64_t ne, const double* 
   if (!rc) rc = ensure(ctx, m->w_sx, (size_t)D * (ne + nq));
   if (!rc) rc = ensure(ctx, m->w_smu, (size_t)nep * nqp);
   if (rc) return rc;
-  sb.A = m->w_sA.p; sb.Bt = m->w_sBt.p; sb.C = m->w_sC.p; sb.Cu = want_var ? m->w_sCu.p : nullptr;
+  sb.A = m->w_sA.p; sb.Bt = m->w_sBt.p; sb.C = m->w_sC.p; sb.Cu = want_var ? m->w_sCu.p : nullptr; sb.C_row_scale = m->d_wt;
   sb.d_xe = m->w_sx.p; sb.d_xq = m->w_sx.p + (size_t)D * ne;
   double* d_mu = m->w_smu.p;
   CK(cudaMemcpyAsync(sb.d_xe, xe, sizeof(double) * D * ne, cudaMemcpyHostToDevice, ctx->stream));
@@ -1392,7 +1409,7 @@ int gpr_split_predict(gpr_model* m, const double* xe, int64_t ne, const double* 
   {
     // A, Bt = B^T (training index fastest), Cw = Diagonal(wt) * C[:, :, k] (split_predict.jl:13), and Cu for the variance
     Scope s(m->tm, GPR_T_SPLIT_BUILD, ctx->stream);
-    rc = split_build(ctx, m->spec, D, m->d_hp, sb.d_xe, ne, sb.d_xq, nq, m->d_x, N, Np, 0.0, sb, false, true, m->d_wt, want_var, true);
+    rc = split_build(ctx, m->spec, D, m->d_hp, sb.d_xe, ne, sb.d_xq, nq, m->d_x, N, Np, sb);
     if (rc) return rc;
   }
   CudaBE be{ctx};
@@ -1420,16 +1437,10 @@ int gpr_split_predict(gpr_model* m, const double* xe, int64_t ne, const double* 
   // products since they moved to the INT8 tensor cores), so the chunks land in a pinned staging buffer of the context at PCIe speed
   // and the host copies each finished chunk on while the GPU computes the next one.  Falls back to the direct copy if the pinned
   // allocation fails or would exceed 1 GB.
-  const size_t stage_elems = (size_t)ne * (size_t)nq;
-  if (stage_elems > ctx->h_stage_elems && stage_elems * sizeof(double) <= ((size_t)1 << 30)) {
-    if (ctx->h_stage) { cudaFreeHost(ctx->h_stage); ctx->h_stage = nullptr; ctx->h_stage_elems = 0; }
-    if (cudaMallocHost(&ctx->h_stage, stage_elems * sizeof(double)) == cudaSuccess) ctx->h_stage_elems = stage_elems;
-    else { cudaGetLastError(); ctx->h_stage = nullptr; }
-  }
-  const bool staged = ctx->h_stage_elems >= stage_elems;
-  if (staged && !ctx->ev_d2h[0])
+  double* stage = ctx->host_stage((size_t)ne * (size_t)nq);
+  if (stage && !ctx->ev_d2h[0])
     for (int i = 0; i < 4; ++i) CK(cudaEventCreateWithFlags(&ctx->ev_d2h[i], cudaEventDisableTiming));
-  double* dst = staged ? ctx->h_stage : mean;
+  double* dst = stage ? stage : mean;
   int nsent = 0;
   {
     Scope s(m->tm, GPR_T_SPLIT_D2H, ctx->side_stream);
@@ -1439,24 +1450,21 @@ int gpr_split_predict(gpr_model* m, const double* xe, int64_t ne, const double* 
       CK(cudaStreamWaitEvent(ctx->side_stream, ctx->ev_chunk[ch], 0));
       CK(cudaMemcpy2DAsync(dst + q0 * ne, sizeof(double) * ne, d_mu + q0 * nep, sizeof(double) * nep, sizeof(double) * ne, qn,
                            cudaMemcpyDeviceToHost, ctx->side_stream));
-      if (staged) CK(cudaEventRecord(ctx->ev_d2h[ch], ctx->side_stream));
+      if (stage) CK(cudaEventRecord(ctx->ev_d2h[ch], ctx->side_stream));
       ++nsent;
     }
   }
-  if (staged)
+  if (stage)
     for (int ch = 0; ch < nsent; ++ch) {
       const int64_t q0 = ch * cw, qn = std::min<int64_t>(cw, nq - q0);
       CK(cudaEventSynchronize(ctx->ev_d2h[ch]));
-      memcpy(mean + q0 * ne, ctx->h_stage + q0 * ne, sizeof(double) * (size_t)ne * (size_t)qn);
+      memcpy(mean + q0 * ne, stage + q0 * ne, sizeof(double) * (size_t)ne * (size_t)qn);
     }
   CK(cudaStreamSynchronize(ctx->side_stream));
   CK(cudaStreamSynchronize(ctx->stream));
-  if (var) {
-    const double prior = prior_diag(m);
-    for (int64_t i = 0; i < ne * nq; ++i) var[i] = prior;   // fill!(Sigma.diag, sum sigma^2)  (src/predict.jl:55-58)
-  }
+  const double prior = prior_var(m->spec, m->hp_host.data());
+  if (var) for (int64_t i = 0; i < ne * nq; ++i) var[i] = prior;   // fill!(Sigma.diag, sum sigma^2)  (src/predict.jl:55-58)
   if (want_var) {
-    const double prior = prior_diag(m);
     const int64_t EB = std::max<int64_t>(1, ctx->predict_tile / nqp);
     rc = ensure(ctx, m->w_kxp, (size_t)EB * nqp * Np);
     if (!rc) rc = ensure(ctx, m->w_var, (size_t)EB * nqp);
