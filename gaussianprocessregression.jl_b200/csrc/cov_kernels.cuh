@@ -556,20 +556,44 @@ __device__ __forceinline__ double erf_between(double x, double y) {
   return erf(y) - erf(x);
 }
 
-// hp: [sigma, l_1..l_D] (the first D + 1 hyper-parameters of the model, as the reference reads them); k1 has np
-// entries, those >= n are set to zero (padding of the factor).
-__global__ void antideriv_se_kernel(const double* __restrict__ x, int D, long long n, long long np, const double* __restrict__ hp,
-                                    const double* __restrict__ a, const double* __restrict__ b, double* __restrict__ k1) {
+// hp: [sigma, l_1..l_D] (the first D + 1 hyper-parameters of the model, as the reference reads them).
+// k1 tile (np x mtp, ld ldk, training index fastest): column c is k1 of box c, bounds a[i + c D], b[i + c D] (D x nbox);
+// rows >= n (padding of the factor) and columns >= nbox (padding of the tile) are zero.  Threads run along the training
+// index (coalesced stores); each CTA stages ANTIDERIV_BOXES boxes' bounds in shared memory (2 D ANTIDERIV_BOXES doubles of
+// dynamic shared memory) and walks the box chunks blockIdx.y, blockIdx.y + gridDim.y, ...
+constexpr int ANTIDERIV_BOXES = 8;
+__global__ void __launch_bounds__(256) antideriv_se_kernel(const double* __restrict__ x, int D, long long n, long long np,
+                                                           const double* __restrict__ hp, const double* __restrict__ a,
+                                                           const double* __restrict__ b, long long nbox, long long mtp,
+                                                           double* __restrict__ k1, long long ldk) {
+  extern __shared__ double sab[];   // [a | b] of the chunk, D x ANTIDERIV_BOXES each
   const long long j = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-  if (j >= np) return;
-  if (j >= n) { k1[j] = 0.0; return; }
-  double prefac = hp[0] * hp[0], v = 1.0;
-  for (int i = 0; i < D; ++i) {
-    const double l = hp[1 + i], xij = x[i + j * D];
-    prefac *= 0.88622692545275801365 / l;
-    v *= erf_between(l * (a[i] - xij), l * (b[i] - xij));
+  const int nab = D * ANTIDERIV_BOXES;
+  for (long long c0 = (long long)blockIdx.y * ANTIDERIV_BOXES; c0 < mtp; c0 += (long long)gridDim.y * ANTIDERIV_BOXES) {
+    __syncthreads();
+    for (int t = threadIdx.x; t < 2 * nab; t += blockDim.x) {
+      const long long o = c0 * D + (t % nab);
+      sab[t] = o < nbox * D ? (t < nab ? a[o] : b[o]) : 0.0;
+    }
+    __syncthreads();
+    if (j >= np) continue;
+    for (int cc = 0; cc < ANTIDERIV_BOXES && c0 + cc < mtp; ++cc) {
+      const long long c = c0 + cc;
+      double out = 0.0;
+      if (j < n && c < nbox) {
+        const double* ac = sab + cc * D;
+        const double* bc = sab + nab + cc * D;
+        double prefac = hp[0] * hp[0], v = 1.0;
+        for (int i = 0; i < D; ++i) {
+          const double l = hp[1 + i], xij = x[i + j * D];
+          prefac *= 0.88622692545275801365 / l;
+          v *= erf_between(l * (ac[i] - xij), l * (bc[i] - xij));
+        }
+        out = v * prefac;
+      }
+      k1[j + c * ldk] = out;
+    }
   }
-  k1[j] = v * prefac;
 }
 
 // out[0] = sum_i v[i]^2 over n entries; one CTA, fixed order

@@ -520,6 +520,29 @@ double prior_var(const KSpec& spec, const double* hp) {
   return s;
 }
 
+// antideriv2(SquaredExp(), hp, a, b) (src/integrate.jl:33-41): sigma^2 prod_i erf_integ(l_i, a_i, b_i), hp = [sigma, l_1..l_D]
+// of the first component whatever the others are, as the reference reads it
+double antideriv2_se(const double* hp, const double* a, const double* b, int D) {
+  double k2 = hp[0] * hp[0];
+  for (int i = 0; i < D; ++i) {
+    const double w = hp[1 + i], d = b[i] - a[i];
+    k2 *= 1.0 / (w * w) * (std::exp(-(w * d) * (w * d)) - 1.0) + 2.0 * (0.88622692545275801365 / w) * d * std::erf(w * d);
+  }
+  return k2;
+}
+
+// k1 tile of nbox boxes on ctx's queue (antideriv_se_kernel: np x mtp, ld ldk; a, b D x nbox on the device)
+int launch_antideriv(gpr_ctx* ctx, const double* x, int D, int64_t n, int64_t np, const double* hp, const double* a,
+                     const double* b, int64_t nbox, int64_t mtp, double* k1, int64_t ldk) {
+  const size_t smem = sizeof(double) * 2 * D * ANTIDERIV_BOXES;
+  if (smem > 48 * 1024) CK(cudaFuncSetAttribute(antideriv_se_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const dim3 grid((unsigned)((np + 255) / 256), (unsigned)std::min<int64_t>((mtp + ANTIDERIV_BOXES - 1) / ANTIDERIV_BOXES, 65535));
+  antideriv_se_kernel<<<grid, 256, smem, ctx->stream>>>(x, D, n, np, hp, a, b, nbox, mtp, k1, ldk);
+  ctx->launches++;
+  CK(cudaGetLastError());
+  return GPR_OK;
+}
+
 // K (+ noise, + jitter, identity padding) into m->d_U, then blocked potrf; solves for all y columns.
 // Reads the factorization status back (the only host <-> device round trip of the factor / inverse sequence) and fixes the cache
 // state accordingly.  LAPACK-style info: first failing pivot, 0 = ok (src/cost.jl:104 throws PosDefException the same way).
@@ -1521,9 +1544,8 @@ int gpr_integrate(gpr_model* m, const double* a, const double* b, double* Iout, 
   CK(cudaMemcpyAsync(d_ab, a, sizeof(double) * D, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(d_ab + D, b, sizeof(double) * D, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemsetAsync(d_I, 0, sizeof(double) * m->nyp, ctx->stream));
-  antideriv_se_kernel<<<(unsigned)((Np + 255) / 256), 256, 0, ctx->stream>>>(m->d_x, D, N, Np, m->d_hp, d_ab, d_ab + D, d_k1);
-  ctx->launches++;
-  CK(cudaGetLastError());
+  rc = launch_antideriv(ctx, m->d_x, D, N, Np, m->d_hp, d_ab, d_ab + D, 1, 1, d_k1, Np);
+  if (rc) return rc;
   CudaBE be{ctx};
   be.gemv('T', m->nyp, Np, 1.0, m->d_wt, Np, d_k1, d_I);          // Iout = wt' * k1   (mean_integ_impl!, :118-121)
   std::vector<double> hI((size_t)m->ny);
@@ -1541,15 +1563,7 @@ int gpr_integrate(gpr_model* m, const double* a, const double* b, double* Iout, 
   rc = check_pending(ctx, "gpr_integrate");
   if (rc) return rc;
   for (int e = 0; e < m->ny; ++e) Iout[e] = hI[e];
-  if (var_out) {
-    // antideriv2 (src/integrate.jl:33-41): sigma^2 prod_i erf_integ(l_i, a_i, b_i)
-    double k2 = m->hp_host[0] * m->hp_host[0];
-    for (int i = 0; i < D; ++i) {
-      const double w = m->hp_host[1 + i], d = b[i] - a[i];
-      k2 *= 1.0 / (w * w) * (std::exp(-(w * d) * (w * d)) - 1.0) + 2.0 * (0.88622692545275801365 / w) * d * std::erf(w * d);
-    }
-    var_out[0] = k2 - hsq;
-  }
+  if (var_out) var_out[0] = antideriv2_se(m->hp_host.data(), a, b, D) - hsq;
   return GPR_OK;
 }
 

@@ -76,6 +76,7 @@ _SIGS = {
     "gpr_mgpu_update_cache": (C.c_int, [_vp, _dp, C.c_int, C.c_double, C.POINTER(_i64)]),
     "gpr_mgpu_predict": (C.c_int, [_vp, _dp, _i64, C.c_int, _dp, _dp, _dp]),
     "gpr_mgpu_split_predict": (C.c_int, [_vp, _dp, _i64, _dp, _i64, _i64, _i64, _dp, _dp]),
+    "gpr_mgpu_integrate": (C.c_int, [_vp, _i64, _dp, _dp, _dp, _dp]),
     "gpr_mgpu_fetch": (C.c_int, [_vp, C.c_int, _dp]),
     "gpr_mgpu_timings": (C.c_int, [_vp, _dp, C.c_int]),
     "gpr_mgpu_dbg_factor": (C.c_int, [_vp, _dp, _i64, _dp, C.c_int, C.c_int, C.POINTER(_i64), _dp]),
@@ -559,6 +560,19 @@ class MultiModelHandle:
         xe, ne, xq, nq, lo, hi, mean, var = _split_args(xe, xq, var_range, want_var, mean_out, var_out)
         self.mctx.check(lib().gpr_mgpu_split_predict(self.handle, dptr(xe), ne, dptr(xq), nq, lo, hi, dptr(mean), dptr(var)))
         return mean, var
+
+    def integrate(self, a, b, want_var=True):
+        """gpr_mgpu_integrate.  a, b of shape (D,): (Iout (ny,), var (1,)) as ModelHandle.integrate; of shape (D, nbox):
+        (Iout (nbox, ny), var (nbox,)), one pass over K^-1 for all boxes."""
+        a, b = np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64)
+        if a.shape != b.shape or a.ndim not in (1, 2) or a.shape[0] != self.D or a.ndim == 2 and a.shape[1] < 1:
+            raise GPRError("integration bounds must be (D,) or (D, nbox) arrays of the same shape")
+        single, nbox = a.ndim == 1, 1 if a.ndim == 1 else int(a.shape[1])
+        a, b = f64(a.reshape(self.D, nbox)), f64(b.reshape(self.D, nbox))
+        Iout = np.empty((nbox, self.ny), order="F")
+        var = np.empty(nbox) if want_var else None
+        self.mctx.check(lib().gpr_mgpu_integrate(self.handle, nbox, dptr(a), dptr(b), dptr(Iout), dptr(var)))
+        return (Iout[0], var) if single else (Iout, var)
 
     def fetch(self, which):
         out = np.empty((self.N, self.N), order="F") if which == FETCH_KINV else np.empty(self.N)

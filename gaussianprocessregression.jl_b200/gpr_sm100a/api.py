@@ -935,7 +935,7 @@ def antideriv2(cov, hp, a, b):
     return float(np.prod(erf_integ(ls, np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64))) * hp[0] ** 2)
 
 
-def integrate(md, *args, sample_noise=None, ctx=None):
+def integrate(md, *args, sample_noise=None, ctx=None, cache=None):
     """integrate(md, a, b; sample_noise) | integrate(md, hp, a, b; sample_noise)  (src/integrate.jl:45-62):
     mean and variance of the integral of the posterior over the box [a, b].  Returns (Iout[ny], var_Iout).
 
@@ -944,34 +944,52 @@ def integrate(md, *args, sample_noise=None, ctx=None):
     syevr, :72-80) and applies (K + eps_i I)^-1 = P (lambda + eps_i)^-1 P' per column.  The device has no symmetric
     eigensolver; the SAME quantities -- mu_i = y_i' (K + eps_i I)^-1 k1 and var_i = k2 - k1' (K + eps_i I)^-1 k1 -- are
     obtained from one shifted Cholesky factorization per distinct noise level (the shift rides in the jitter argument of
-    update_cache!), i.e. N^3/3 flop per level instead of one ~9 N^3 eigendecomposition: cheaper up to ~27 levels."""
+    update_cache!), i.e. N^3/3 flop per level instead of one ~9 N^3 eigendecomposition: cheaper up to ~27 levels.
+
+    a, b may also be D x nbox arrays (box i = column i): Iout is then (nbox, ny) and var_Iout (nbox,) -- (nbox, ny) with
+    sample_noise, one row per box as the single-box call returns it.
+    cache: a MultiGPUGradCache / MultiGPUPredictCache of md; the factorizations then run block-cyclic on its devices
+    (update_cache_ on that cache) and all boxes go through gpr_mgpu_integrate in one pass over K^-1.  Without it, one
+    device: gpr_integrate once per box."""
     if len(args) == 2:
         hp, (a, b) = md.params, args
     else:
         hp, a, b = args
-    wc = MllLossCache(md, ctx)
+    multi = isinstance(cache, MultiGPUGradCache)
+    a2, b2 = np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64)
+    batched = a2.ndim == 2
+    wc = cache if multi else MllLossCache(md, ctx)
+
+    def once(eps):
+        update_cache_(wc, hp, md, ϵ=eps)
+        if multi or not batched:
+            return wc.handle.integrate(a2, b2, want_var=True)
+        if a2.shape != b2.shape or a2.shape[1] < 1:
+            raise GPRError("integration bounds must be (D,) or (D, nbox) arrays of the same shape")
+        res = [wc.handle.integrate(a2[:, i], b2[:, i], want_var=True) for i in range(a2.shape[1])]
+        return np.stack([r[0] for r in res]), np.concatenate([r[1] for r in res])
+
     try:
         if sample_noise is None:
-            update_cache_(wc, hp, md)
-            return wc.handle.integrate(a, b, want_var=True)
+            return once(1e-8)
         ny = 1 if md.y.ndim == 1 else md.y.shape[1]
         # the jitter is added once per non-noise component (src/compose_covar.jl:53-55), so eps_i is split among them
         nk = sum(1 for k in _components(md.covar) if not isinstance(k, WhiteNoise))
         if np.ndim(sample_noise) == 0:
-            update_cache_(wc, hp, md, ϵ=1e-8 + float(sample_noise) / nk)
-            Iout, var = wc.handle.integrate(a, b, want_var=True)
-            return Iout, np.full(ny, var[0])          # var_Iout .= k2 .- scalar  (:157-158)
+            Iout, var = once(1e-8 + float(sample_noise) / nk)
+            return Iout, np.repeat(var[:, None], ny, axis=1) if batched else np.full(ny, var[0])   # var_Iout .= k2 .- scalar  (:157-158)
         noise = np.asarray(sample_noise, dtype=np.float64).ravel()
         if noise.size != ny:
             raise GPRError("sample_noise needs one entry per column of y")
-        Iout, var = np.empty(ny), np.empty(ny)
+        nbox = a2.shape[1] if batched else 1
+        Iout, var = np.empty((nbox, ny)), np.empty((nbox, ny))
         done = {}
         for i, e in enumerate(noise):
             if e not in done:
-                update_cache_(wc, hp, md, ϵ=1e-8 + float(e) / nk)
-                done[e] = wc.handle.integrate(a, b, want_var=True)
+                done[e] = once(1e-8 + float(e) / nk)
             Ii, vi = done[e]
-            Iout[i], var[i] = Ii[i], vi[0]
-        return Iout, var
+            Iout[:, i], var[:, i] = Ii.reshape(nbox, ny)[:, i], vi
+        return (Iout, var) if batched else (Iout[0], var[0])
     finally:
-        wc.close()
+        if not multi:
+            wc.close()

@@ -256,6 +256,19 @@ int gpr_mgpu_update_cache(gpr_mgpu_model* model, const double* hp, int P, double
  * the products, PRED_ROWNORM = the fix-up / row-dot kernel, PRED_MEAN = the sum over the ranks and the download. */
 int gpr_mgpu_predict(gpr_mgpu_model* model, const double* xp, int64_t M, int same_x, double* mean, double* var_diag,
                      double* cov_full);
+/* integrate!(Iout, var_Iout, md, hp, a, b, nothing, wc, ac) (src/integrate.jl:56-62,103-143) for nbox boxes at once on the
+ * multi-GPU model, from the K^-1 of gpr_mgpu_predict (same preconditions: GPR_ERR_STATE unless predict-ready, at that
+ * factorization's hp and eps).  a, b: D x nbox (box i is column i).  Iout: nbox x ny, box index fastest (the layout of the
+ * gpr_mgpu_predict mean; for nbox = 1 gpr_integrate's Iout[ny]), Iout[i + e nbox] = Y[:, e]^T K^-1 k1_i.  var_out: NULL or
+ * nbox entries, var_i = k2_i - k1_i^T K^-1 k1_i, not clamped.  As gpr_integrate, k1 = antideriv!(SquaredExp(), x, hp, a, b)
+ * (:15-31) and k2 = antideriv2 (:33-41) read hp[1..D+1] of the first component whatever the others are;
+ * GPR_ERR_UNSUPPORTED unless that component is a SquaredExp.  GPR_ERR_ARG for NULL a, b, Iout or nbox < 1.
+ * Collective like gpr_mgpu_predict: under gpr_dist_create every process passes the same boxes and receives the same outputs.
+ * The boxes are the test points of gpr_mgpu_predict with k1 in place of K(x, xp): tiles of "predict_tile" boxes (halved while
+ * they do not fit, GPR_ERR_MEMORY below 128), each one pass over every rank's K^-1 columns, so many boxes per call cost
+ * about as much as one.  Timings: PRED_KSTAR = the k1 tile build, PRED_TRSM = the products, PRED_ROWNORM = the fix-up,
+ * PRED_MEAN = the sum over the ranks and the download. */
+int gpr_mgpu_integrate(gpr_mgpu_model* model, int64_t nbox, const double* a, const double* b, double* Iout, double* var_out);
 /* predict_mean! / predict!(mu, Sigma::Diagonal, md, Cmap(+, xe, xq), pc) (src/split_predict.jl:5-53) on the multi-GPU model.
  * Arguments and outputs exactly as gpr_split_predict (mean ne x nq, e fastest; var nullable, ne*nq entries, q fastest within e;
  * rows e in [e_lo, e_hi] get the posterior variance, all others keep the prior; e_lo = e_hi + 1: no variance rows); the

@@ -370,4 +370,42 @@ function integrate_sm100(md::GPRModel, hp, a, b; sample_noise = nothing)
     Iout, var
 end
 
+# The same on the distributed model of SM100Multi: one gpr_mgpu_update_cache per distinct noise level, then
+# gpr_mgpu_integrate for all boxes at once (a, b: vectors or D x nbox matrices, box i = column i) in one pass over K^-1.
+# Vectors give the results of the single-device method; matrices give Iout nbox x ny and var nbox (nbox x ny with sample_noise).
+function _mintegrate_once(h::MultiHandle, hp::Vector{Float64}, a::Matrix{Float64}, b::Matrix{Float64}, eps::Float64, ny::Int)
+    info = Ref{Int64}(0)
+    mcheck(h, ccall((:gpr_mgpu_update_cache, LIB), Cint, (Ptr{Cvoid}, Ptr{Float64}, Cint, Cdouble, Ref{Int64}),
+        h.h, hp, length(hp), eps, info), info[])
+    nbox = size(a, 2)
+    Iout = Matrix{Float64}(undef, nbox, ny); v = Vector{Float64}(undef, nbox)
+    mcheck(h, ccall((:gpr_mgpu_integrate, LIB), Cint, (Ptr{Cvoid}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+        h.h, nbox, a, b, Iout, v))
+    Iout, v
+end
+function integrate_sm100(s::SM100Multi, hp, a, b; sample_noise = nothing)
+    h, _, _ = _multi_model(s.md, s.devices, s.nb)
+    ny = size(s.md.y, 2)
+    nk = count(k -> !(k isa WhiteNoise), s.md.covar isa ComposedKernel ? s.md.covar.kernels : (s.md.covar,))
+    single = a isa AbstractVector
+    hpv = Vector{Float64}(hp)
+    am = Matrix{Float64}(reshape(a, size(a, 1), :)); bm = Matrix{Float64}(reshape(b, size(b, 1), :))
+    if sample_noise === nothing
+        I, v = _mintegrate_once(h, hpv, am, bm, 1e-8, ny)
+        return single ? (I[1, :], v) : (I, v)
+    end
+    if sample_noise isa Real
+        I, v = _mintegrate_once(h, hpv, am, bm, 1e-8 + sample_noise / nk, ny)
+        return single ? (I[1, :], fill(v[1], ny)) : (I, repeat(v, 1, ny))
+    end
+    Iout = Matrix{Float64}(undef, size(am, 2), ny); var = similar(Iout)
+    levels = Dict{Float64,Tuple{Matrix{Float64},Vector{Float64}}}()
+    for (i, e) in enumerate(sample_noise)
+        haskey(levels, e) || (levels[e] = _mintegrate_once(h, hpv, am, bm, 1e-8 + e / nk, ny))
+        I, v = levels[e]
+        Iout[:, i] = I[:, i]; var[:, i] = v
+    end
+    single ? (Iout[1, :], var[1, :]) : (Iout, var)
+end
+
 end # module
