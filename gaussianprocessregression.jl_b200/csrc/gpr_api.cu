@@ -48,13 +48,10 @@ struct Timer {
   double acc_ms[GPR_T_COUNT];
 };
 
-}  // namespace
+// phase of the factorization / inverse being run (gpr_ctx::oz_cur); the values are the bits of the public option "ozaki_phases"
+constexpr int OZ_PH_POTRF = 1, OZ_PH_TRTRI = 2, OZ_PH_LAUUM = 4, OZ_PH_OTHER = 8;
 
-// default of the "ozaki_mc" context option; GPR_OZ_MC=0 / 1 in the environment overrides it (A/B runs without touching the callers)
-static int oz_mc_default() {
-  const char* e = getenv("GPR_OZ_MC");
-  return (e && *e) ? (atoi(e) != 0) : 0;
-}
+}  // namespace
 
 struct gpr_ctx {
   int device = 0;
@@ -77,16 +74,10 @@ struct gpr_ctx {
                                    // K >= this (0 = never): the windows pay for their second pass over the digit planes only on the largest products --
                                    // N = 32768 evaluation 680 -> 667 ms at 8192, 670 at 4096, 680 at 2048 (profiles/ozaki_win_mink_r2an.log)
   int ozaki_split = 9;          // option "ozaki_split": digits of the INT8 route for the split-predict mean products (0 = DMMA, 8, 9)
-  int ozaki_lauum_map = 0;      // option "ozaki_lauum_map": nine-digit INT8 form also for the rank-nb W W^T products of the block-cyclic lauum (slower: off)
-  int ozaki_windows = 0;        // option "ozaki_windows" (A/B switches of csrc/ozaki_i8.cuh): bit 0 two-diagonal-window 128 x 128 kernel for the
-                                // 8-digit products; bit 2 the THREE-window form of the 9-digit product (d = 10 | 6..9 | 2..5) instead of the
-                                // default two windows (d = 6..10 with 128 x 96 tiles | 2..5), bit 1 with it: 128 x 256 tiles for d = 10
-  int ozaki_mc = oz_mc_default();   // option "ozaki_mc": the 128 x 128 window kernels of the INT8 route run as clusters of two CTAs that share one
-                                    // op(B) tile through a multicast TMA load (csrc/ozaki_i8.cuh, launch flag 8192); results are bit-identical,
-                                    // the whole GPU suite passes with it, and it is measured neutral (668 -> 667 ms per evaluation): off
   int64_t ozaki_kchunk = 32768; // option "ozaki_kchunk": k-chunk of the long-K tile-mapped products (tests lower it to exercise the chunk loop)
   int64_t ozaki_panel = 32768;  // option "ozaki_panel": k-panel of the W^T W product (own digit scales per panel)
-  int oz_mask = 11, oz_cur = 8;   // option "ozaki_phases": bit 0 potrf, 1 trtri, 3 everything else (prediction solves); the W^T W product of the
+  int oz_mask = OZ_PH_POTRF | OZ_PH_TRTRI | OZ_PH_OTHER, oz_cur = OZ_PH_OTHER;
+                                  // option "ozaki_phases": bit 0 potrf, 1 trtri, 3 everything else (prediction solves); the W^T W product of the
                                   // inverse (lauum) is governed by "ozaki_lauum": its operand columns span many orders of magnitude under ONE
                                   // power-of-two scale per column, and with 8 digits the gradient keeps only 7 digits (1.1e-7 vs the oracle);
                                   // NINE digits restore it (4.0e-11, DMMA: 6.1e-11 at N = 32768; profiles/ozaki_lauum9_r2s.log)
@@ -136,60 +127,79 @@ int fail_cuda(gpr_ctx* ctx, cudaError_t e, const char* what, int line) {
 struct CudaBE {
   gpr_ctx* ctx;
   void note(cudaError_t e) { if (e != cudaSuccess && ctx->pending == cudaSuccess) ctx->pending = e; }
-  // digit-plane workspace of the INT8 route: grown on demand (a failed allocation leaves the product on the DMMA pipe)
-  void oz_reserve(size_t need) {
-    if (need <= ctx->oz_ws_bytes) return;
-    cudaStreamSynchronize(ctx->main_stream);
-    cudaFree(ctx->oz_ws); ctx->oz_ws = nullptr; ctx->oz_ws_bytes = 0;
-    if (cudaMalloc(&ctx->oz_ws, need) == cudaSuccess) ctx->oz_ws_bytes = need; else cudaGetLastError();
+  // digit-plane workspace of the INT8 route: grown on demand; false if it cannot hold `need` bytes (the product then stays on the DMMA pipe)
+  bool oz_reserve(size_t need) {
+    if (need > ctx->oz_ws_bytes) {
+      cudaStreamSynchronize(ctx->main_stream);
+      cudaFree(ctx->oz_ws); ctx->oz_ws = nullptr; ctx->oz_ws_bytes = 0;
+      if (cudaMalloc(&ctx->oz_ws, need) == cudaSuccess) ctx->oz_ws_bytes = need; else cudaGetLastError();
+    }
+    return ctx->oz_ws_bytes >= need;
   }
-  bool ozaki_eligible(char tA, char tB, int64_t M, int64_t N, int64_t K, const double* A, const double* B, const double* C, int flags,
-                      int64_t batch) const {
-    if (ctx->oz_active <= 0 || ctx->stream != ctx->main_stream) return false;
-    if (ctx->oz_cur == 4 ? ctx->ozaki_lauum == 0 : !(ctx->oz_mask & ctx->oz_cur)) return false;
-    if (tA != 'T' || tB != 'N') return false;
-    if (flags & ~(BLK_UPPER_ONLY | BLK_K_FROM_N | BLK_SKIP_TILE00)) return false;
-    if ((const double*)C == A || (const double*)C == B) return false;
-    if (batch < 1 || batch > 16) return false;
+  // Route of one product: digits of the INT8 tensor cores (csrc/ozaki_i8.cuh), 0 = DMMA pipe; launch flags it adds; k-split
+  // (0 = none): ozaki_panel for the W^T W product of the inverse, ozaki_kchunk for the k-upto product.
+  enum OzKind { OZ_PLAIN, OZ_HADAMARD, OZ_MAP_UPPER, OZ_MAP_KUPTO };
+  struct OzRoute { int digits = 0, flags = 0; int64_t ksplit = 0; };
+  OzRoute ozaki_route(OzKind kind, char tA, char tB, int64_t M, int64_t N, int64_t K, const double* A, int64_t lda, const double* B,
+                      int64_t ldb, const double* C, int flags, int64_t batch = 1) const {
+    OzRoute r;
+    if (ctx->oz_active <= 0 || ctx->stream != ctx->main_stream || tA != 'T' || tB != 'N') return r;   // (the side queue stays on DMMA)
+    if ((const double*)C == A || (const double*)C == B) return r;
     const int64_t mn = ctx->ozaki_min;
-    return M >= mn && N >= mn && K >= mn && K <= 32768 && (M % 128) == 0 && (N % 128) == 0 && (K % 128) == 0;
+    if (M < mn || N < mn || K < mn || (M % 128) || (N % 128) || (K % 128)) return r;
+    int digits = ctx->oz_active;
+    if (ctx->oz_cur == OZ_PH_LAUUM && kind == OZ_PLAIN) digits = ctx->ozaki_lauum;     // W^T W of the inverse: "ozaki_lauum", not the phase mask
+    else if (ctx->oz_cur == OZ_PH_LAUUM && kind == OZ_HADAMARD) return r;
+    else if (!(ctx->oz_mask & ctx->oz_cur)) return r;
+    switch (kind) {
+      case OZ_PLAIN:
+      case OZ_HADAMARD:
+        if ((flags & ~(BLK_UPPER_ONLY | BLK_K_FROM_N | BLK_SKIP_TILE00)) || batch < 1 || batch > 16 || K > 32768) return r;
+        if (kind == OZ_HADAMARD) { r.digits = ctx->ozaki_split; return r; }
+        r.digits = digits;
+        if (batch == 1 && flags == (BLK_UPPER_ONLY | BLK_K_FROM_N) && A == B && lda == ldb && M == N && N == K && K > ctx->ozaki_panel)
+          r.ksplit = ctx->ozaki_panel;
+        else if (ctx->ozaki_win_mink > 0 && std::min(K, std::min(M, N)) >= ctx->ozaki_win_mink)
+          r.flags = 512;
+        return r;
+      case OZ_MAP_UPPER:
+        if (flags == BLK_MAP_UPPER && K <= 32768) r.digits = digits;
+        return r;
+      case OZ_MAP_KUPTO:
+        if (flags == BLK_MAP_KUPTO && A != B) { r.digits = digits; r.ksplit = std::min<int64_t>(ctx->ozaki_kchunk, 32768); }
+        return r;
+    }
+    return r;
   }
   void gemm(char tA, char tB, int64_t M, int64_t N, int64_t K, double alpha, const double* A, int64_t lda,
             const double* B, int64_t ldb, double beta, double* C, int64_t ldc, int flags, int64_t batch = 1,
             int64_t sA = 0, int64_t sB = 0, int64_t sC = 0) {
-    // grid.z is limited to 65535: split very large batches
-    if (ozaki_eligible(tA, tB, M, N, K, A, B, C, flags, batch)) {
-      // large T,N product: INT8 tensor cores (csrc/ozaki_i8.cuh), one launch per batch member
-      const int digits = ctx->oz_cur == 4 ? ctx->ozaki_lauum : ctx->oz_active;
-      const size_t need = oz_workspace_bytes((int)std::max(M, N), (int)N, (int)K, digits);
-      oz_reserve(need);
-      if (ctx->oz_ws_bytes >= need && batch == 1 && flags == (BLK_UPPER_ONLY | BLK_K_FROM_N) && A == B && lda == ldb && M == N && N == K &&
-          K > ctx->ozaki_panel) {
+    const OzRoute oz = ozaki_route(OZ_PLAIN, tA, tB, M, N, K, A, lda, B, ldb, C, flags, batch);
+    if (oz.digits && oz_reserve(oz_workspace_bytes((int)std::max(M, N), (int)N, (int)K, oz.digits))) {
+      if (oz.ksplit) {
         // W^T W of the inverse (lauum_oop_t): the columns of the triangular factor span many orders of magnitude (O(1/sigma_n)
         // next to the diagonal, tiny far from it), and the digit planes of a column share ONE power-of-two scale.  Summing the
         // product over k-panels, each with its own column scales, keeps the error relative to the panel-local magnitudes
         // (measured on the benchmark model: gradient error vs the oracle 1.1e-7 with one scale per column -> see profiles/).
         // The last panel touches every column and initialises C (beta), the earlier ones accumulate into their leading block.
-        const int64_t P = ctx->ozaki_panel;
-        for (int64_t p1 = K; p1 > 0; p1 -= P) {
-          const int64_t p0 = std::max<int64_t>(0, p1 - P);
+        for (int64_t p1 = K; p1 > 0; p1 -= oz.ksplit) {
+          const int64_t p0 = std::max<int64_t>(0, p1 - oz.ksplit);
           const int64_t cols = std::min<int64_t>(N, p1);
-          note(launch_ozaki_dgemm(ctx->stream, (int)cols, (int)cols, (int)(p1 - p0), digits, alpha, A + p0, lda, B + p0, ldb,
-                                  p1 == K ? beta : 1.0, C, ldc, flags | ((ctx->ozaki_windows & 2) ? 1024 : 0) | ((ctx->ozaki_windows & 4) ? 4096 : 0) | (ctx->ozaki_mc ? 8192 : 0), ctx->oz_ws, (int)p0));
+          note(launch_ozaki_dgemm(ctx->stream, (int)cols, (int)cols, (int)(p1 - p0), oz.digits, alpha, A + p0, lda, B + p0, ldb,
+                                  p1 == K ? beta : 1.0, C, ldc, flags | oz.flags, ctx->oz_ws, (int)p0));
           ctx->launches += 2;
         }
         return;
       }
-      if (ctx->oz_ws_bytes >= need) {
-        for (int64_t z = 0; z < batch; ++z) {
-          note(launch_ozaki_dgemm(ctx->stream, (int)M, (int)N, (int)K, digits, alpha, A + z * sA, lda, B + z * sB, ldb, beta, C + z * sC, ldc,
-                                  flags | (((ctx->ozaki_windows & 1) || (ctx->ozaki_win_mink > 0 && std::min(K, std::min(M, N)) >= ctx->ozaki_win_mink)) ? 512 : 0) |
-                                      ((ctx->ozaki_windows & 2) ? 1024 : 0) | ((ctx->ozaki_windows & 4) ? 4096 : 0) | (ctx->ozaki_mc ? 8192 : 0), ctx->oz_ws));
-          ctx->launches += 3;
-        }
-        return;
+      // large T,N product: one launch per batch member
+      for (int64_t z = 0; z < batch; ++z) {
+        note(launch_ozaki_dgemm(ctx->stream, (int)M, (int)N, (int)K, oz.digits, alpha, A + z * sA, lda, B + z * sB, ldb, beta, C + z * sC, ldc,
+                                flags | oz.flags, ctx->oz_ws));
+        ctx->launches += 3;
       }
+      return;
     }
+    // grid.z is limited to 65535: split very large batches
     for (int64_t z0 = 0; z0 < batch; z0 += 32768) {
       const int64_t nb = std::min<int64_t>(32768, batch - z0);
       if (ctx->gemm_tma && gemm_tma_supported(tA, tB, (int)M, (int)N, (int)K, A, B, C, flags, (int)nb, sA, sB)) {
@@ -207,19 +217,15 @@ struct CudaBE {
   // C = (A^T B) .* E + beta C, T,N form with the Hadamard epilogue (split-predict mean)
   void gemm_hadamard(int64_t M, int64_t N, int64_t K, const double* A, int64_t lda, const double* B, int64_t ldb,
                      const double* E, int64_t lde, double beta, double* C, int64_t ldc) {
-    if (ctx->ozaki_split && ozaki_eligible('T', 'N', M, N, K, A, B, C, 0, 1) && ctx->oz_cur != 4) {
-      // split-predict mean on the INT8 tensor cores; the Hadamard factor and beta ride in the epilogue.  NINE digits by default: the
-      // columns of Diagonal(wt) C carry the weights' dynamic range and the sum over the training points cancels heavily -- with eight
-      // digits the mean agrees with the dense path to 4e-10 instead of 8e-12 (N = 32768, profiles/README.md)
-      const int digits = ctx->ozaki_split;
-      const size_t need = oz_workspace_bytes((int)M, (int)N, (int)K, digits);
-      oz_reserve(need);
-      if (ctx->oz_ws_bytes >= need) {
-        note(launch_ozaki_dgemm(ctx->stream, (int)M, (int)N, (int)K, digits, 1.0, A, lda, B, ldb, beta, C, ldc, ctx->ozaki_mc ? 8192 : 0, ctx->oz_ws, 0,
-                                nullptr, 0, 0, E, lde));
-        ctx->launches += 3;
-        return;
-      }
+    // split-predict mean on the INT8 tensor cores; the Hadamard factor and beta ride in the epilogue.  NINE digits by default ("ozaki_split"):
+    // the columns of Diagonal(wt) C carry the weights' dynamic range and the sum over the training points cancels heavily -- with eight
+    // digits the mean agrees with the dense path to 4e-10 instead of 8e-12 (N = 32768, profiles/README.md)
+    const OzRoute oz = ozaki_route(OZ_HADAMARD, 'T', 'N', M, N, K, A, lda, B, ldb, C, 0);
+    if (oz.digits && oz_reserve(oz_workspace_bytes((int)M, (int)N, (int)K, oz.digits))) {
+      note(launch_ozaki_dgemm(ctx->stream, (int)M, (int)N, (int)K, oz.digits, 1.0, A, lda, B, ldb, beta, C, ldc, oz.flags, ctx->oz_ws, 0,
+                              nullptr, 0, 0, E, lde));
+      ctx->launches += 3;
+      return;
     }
     if (ctx->gemm_tma && gemm_tma_supported('T', 'N', (int)M, (int)N, (int)K, A, B, C, 0, 1, 0, 0))
       note(launch_dgemm128_tma(ctx->stream, (int)M, (int)N, (int)K, 1.0, A, lda, B, ldb, beta, C, ldc, 0, 1, 0, 0, 0, nullptr, 0, 0, E, lde));
@@ -235,52 +241,19 @@ struct CudaBE {
   // tile-mapped GEMM of the block-cyclic multi-GPU drivers (csrc/dist_blocked.hpp)
   void gemm_map(char tA, char tB, int64_t M, int64_t N, int64_t K, double alpha, const double* A, int64_t lda,
                 const double* B, int64_t ldb, double beta, double* C, int64_t ldc, int flags, const TileMap& map) {
-    if (flags == BLK_MAP_UPPER && ctx->oz_active > 0 && ctx->stream == ctx->main_stream && (ctx->oz_mask & ctx->oz_cur) && tA == 'T' &&
-        tB == 'N' && (const double*)C != A && (const double*)C != B && M >= ctx->ozaki_min && N >= ctx->ozaki_min && K >= ctx->ozaki_min &&
-        K <= 32768 && !(M % 128) && !(N % 128) && !(K % 128)) {
-      // rank-nb trailing update of the block-cyclic potrf on the INT8 tensor cores (csrc/ozaki_i8.cuh)
-      const size_t need = oz_workspace_bytes((int)M, (int)N, (int)K, ctx->oz_active);
-      oz_reserve(need);
-      if (ctx->oz_ws_bytes >= need) {
-        note(launch_ozaki_dgemm(ctx->stream, (int)M, (int)N, (int)K, ctx->oz_active, alpha, A, lda, B, ldb, beta, C, ldc, flags, ctx->oz_ws, 0,
-                                map.col_gtile, map.row_gtile0));
+    // INT8 tensor cores: the rank-nb trailing update of the block-cyclic potrf (map-upper) and the row-panel recurrence of the
+    // block-cyclic trtri (k-upto: M = nb rows, per-column contraction limit, K up to N, in k-chunks of at most 32768 -- the int32
+    // accumulators are exact up to there -- each with its own digit scales, accumulated in C)
+    const OzRoute oz = ozaki_route(flags == BLK_MAP_KUPTO ? OZ_MAP_KUPTO : OZ_MAP_UPPER, tA, tB, M, N, K, A, lda, B, ldb, C, flags);
+    const int64_t KC = oz.ksplit ? oz.ksplit : K;
+    if (oz.digits && oz_reserve(oz_workspace_bytes((int)M, (int)N, (int)std::min(K, KC), oz.digits))) {
+      for (int64_t k0 = 0; k0 < K; k0 += KC) {
+        const int64_t kc = std::min(KC, K - k0);
+        note(launch_ozaki_dgemm(ctx->stream, (int)M, (int)N, (int)kc, oz.digits, alpha, A + k0, lda, B + k0, ldb, k0 == 0 ? beta : 1.0, C, ldc,
+                                flags | oz.flags, ctx->oz_ws, (int)k0, map.col_gtile, map.row_gtile0, map.k_gtile0));
         ctx->launches += 3;
-        return;
       }
-    }
-    if (flags == (BLK_MAP_UPPER | BLK_MAP_BROWS) && ctx->oz_active > 0 && ctx->ozaki_lauum_map && ctx->oz_cur == 4 && ctx->stream == ctx->main_stream &&
-        tA == 'T' && tB == 'N' && A == B && lda == ldb && (const double*)C != A && M >= ctx->ozaki_min && N >= ctx->ozaki_min &&
-        K >= ctx->ozaki_min && K <= 32768 && N <= M && !(M % 128) && !(N % 128) && !(K % 128)) {
-      // W W^T accumulation of the block-cyclic lauum (one column panel of W against itself, rank-nb) with NINE digits: the panel is
-      // cut into digit planes once (shared operand), the tile column reads its op(B) rows by global position.  OFF by default
-      // (option "ozaki_lauum_map"): at K = nb the three diagonal windows are dominated by their epilogues -- one rank, N = 32768:
-      // lauum 386 -> 501 ms at nb = 2048, 374 -> 723 ms at nb = 1024 (profiles/mgpu_int8_lauum_r2aa.log); parity is unchanged
-      const size_t need = oz_workspace_bytes((int)M, (int)N, (int)K, 9);
-      oz_reserve(need);
-      if (ctx->oz_ws_bytes >= need) {
-        note(launch_ozaki_dgemm(ctx->stream, (int)M, (int)N, (int)K, 9, alpha, A, lda, B, ldb, beta, C, ldc, flags, ctx->oz_ws, 0,
-                                map.col_gtile, map.row_gtile0));
-        ctx->launches += 4;
-        return;
-      }
-    }
-    if (flags == BLK_MAP_KUPTO && ctx->oz_active > 0 && ctx->stream == ctx->main_stream && (ctx->oz_mask & ctx->oz_cur) && tA == 'T' &&
-        tB == 'N' && (const double*)C != A && (const double*)C != B && M >= ctx->ozaki_min && N >= ctx->ozaki_min && K >= ctx->ozaki_min &&
-        !(M % 128) && !(N % 128) && !(K % 128) && A != B) {
-      // row-panel recurrence of the block-cyclic trtri (M = nb rows, per-column contraction limit, K up to N) on the INT8 tensor
-      // cores: k-chunks of at most 32768 (the int32 accumulators are exact up to there), each with its own digit scales, accumulated in C
-      const int64_t KC = std::min<int64_t>(ctx->ozaki_kchunk, 32768);
-      const size_t need = oz_workspace_bytes((int)M, (int)N, (int)std::min(K, KC), ctx->oz_active);
-      oz_reserve(need);
-      if (ctx->oz_ws_bytes >= need) {
-        for (int64_t k0 = 0; k0 < K; k0 += KC) {
-          const int64_t kc = std::min(KC, K - k0);
-          note(launch_ozaki_dgemm(ctx->stream, (int)M, (int)N, (int)kc, ctx->oz_active, alpha, A + k0, lda, B + k0, ldb, k0 == 0 ? beta : 1.0, C, ldc,
-                                  flags, ctx->oz_ws, (int)k0, map.col_gtile, map.row_gtile0, map.k_gtile0));
-          ctx->launches += 3;
-        }
-        return;
-      }
+      return;
     }
     if (ctx->gemm_tma && gemm_tma_supported(tA, tB, (int)M, (int)N, (int)K, A, B, C, flags, 1, 0, 0))
       note(launch_dgemm128_tma(ctx->stream, (int)M, (int)N, (int)K, alpha, A, lda, B, ldb, beta, C, ldc, flags, 1, 0, 0, 0, map.col_gtile,
@@ -593,9 +566,9 @@ int factor_and_solve(gpr_model* m, const double* hp, double eps, int64_t* info, 
   blk.leaf_lookahead = ctx->leaf_lookahead != 0;
   {
     Scope s(m->tm, GPR_T_POTRF, ctx->stream);
-    ctx->oz_cur = 1;
+    ctx->oz_cur = OZ_PH_POTRF;
     blk.potrf(m->d_U, Np, Np, 0);
-    ctx->oz_cur = 8;
+    ctx->oz_cur = OZ_PH_OTHER;
   }
   {
     Scope s(m->tm, GPR_T_POTRS, ctx->stream);
@@ -642,14 +615,14 @@ int form_inverse(gpr_model* m) {
   if (m->d_W) {
     {
       Scope s(m->tm, GPR_T_TRTRI, ctx->stream);
-      ctx->oz_cur = 2;
+      ctx->oz_cur = OZ_PH_TRTRI;
       blk.trtri_t(m->d_U, Np, m->d_W, Np, Np, 0);      // lower(W) = U^-T, all products in the T,N form
     }
     {
       Scope s(m->tm, GPR_T_LAUUM, ctx->stream);
-      ctx->oz_cur = 4;
+      ctx->oz_cur = OZ_PH_LAUUM;
       blk.lauum_oop_t(m->d_W, Np, Np, m->d_Kinv, Np);  // K^-1 = (U^-T)^T U^-T
-      ctx->oz_cur = 8;
+      ctx->oz_cur = OZ_PH_OTHER;
     }
   } else {
     {
@@ -831,14 +804,11 @@ int gpr_ctx_set_option(gpr_ctx* ctx, const char* name, int64_t value) {
     if (value != 0 && value != 8 && value != 9) return fail(ctx, GPR_ERR_ARG, "ozaki_lauum: 0 (DMMA), 8 or 9 digits");
     ctx->ozaki_lauum = (int)value; return GPR_OK;
   }
-  if (!strcmp(name, "ozaki_windows")) { ctx->ozaki_windows = (int)value & 7; return GPR_OK; }
-  if (!strcmp(name, "ozaki_mc")) { ctx->ozaki_mc = value != 0; return GPR_OK; }
   if (!strcmp(name, "ozaki_win_mink")) { ctx->ozaki_win_mink = std::max<int64_t>(0, value); return GPR_OK; }
   if (!strcmp(name, "ozaki_split")) {
     if (value != 0 && value != 8 && value != 9) return fail(ctx, GPR_ERR_ARG, "ozaki_split: 0 (DMMA), 8 or 9 digits");
     ctx->ozaki_split = (int)value; return GPR_OK;
   }
-  if (!strcmp(name, "ozaki_lauum_map")) { ctx->ozaki_lauum_map = value ? 1 : 0; return GPR_OK; }
   if (!strcmp(name, "ozaki_kchunk")) { ctx->ozaki_kchunk = std::min<int64_t>(32768, std::max<int64_t>(128, (value / 128) * 128)); return GPR_OK; }
   if (!strcmp(name, "ozaki_panel")) { ctx->ozaki_panel = std::max<int64_t>(128, (value / 128) * 128); return GPR_OK; }
   if (!strcmp(name, "ozaki_phases")) { ctx->oz_mask = (int)value & 15; return GPR_OK; }
@@ -1116,7 +1086,18 @@ int gpr_fetch(gpr_model* m, int which, double* out) {
 int gpr_model_route(gpr_model* m, int* digits, int* digits_inverse) {
   if (!m) return GPR_ERR_ARG;
   if (digits) *digits = m->oz > 0 ? m->oz : 0;
-  if (digits_inverse) *digits_inverse = (m->oz > 0 && m->d_W && m->Np >= m->ctx->ozaki_min && m->Np <= 32768) ? m->ctx->ozaki_lauum : 0;
+  if (digits_inverse) {
+    // the route form_inverse's lauum_oop_t takes: W^T W (Np^3, upper only, K-from-N) in the lauum phase with the model's digits
+    gpr_ctx* ctx = m->ctx;
+    const int active = ctx->oz_active, cur = ctx->oz_cur;
+    ctx->oz_active = m->oz > 0 ? m->oz : 0;
+    ctx->oz_cur = OZ_PH_LAUUM;
+    *digits_inverse = m->d_W ? CudaBE{ctx}.ozaki_route(CudaBE::OZ_PLAIN, 'T', 'N', m->Np, m->Np, m->Np, m->d_W, m->Np, m->d_W, m->Np,
+                                                       m->d_Kinv, BLK_UPPER_ONLY | BLK_K_FROM_N).digits
+                             : 0;
+    ctx->oz_active = active;
+    ctx->oz_cur = cur;
+  }
   return GPR_OK;
 }
 

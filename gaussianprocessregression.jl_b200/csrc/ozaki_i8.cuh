@@ -30,15 +30,14 @@
 // ncu (profiles/ozaki_ncu_full_r2t.md): tensor-core pipe 94 % busy -- every 128 x 64 x 32 product re-reads its 4 KB A operand from
 // shared memory, and eight accumulators cannot be wider than 64 of the 512 TMEM columns: the roof of this instruction shape.
 //
-// Kernel (oz_gemm_win_kernel): the same roles for ONE window of diagonals d = DLO..DHI with BN = 96 / 128 / 256 columns per
+// Kernel (oz_gemm_win_kernel): the same roles for ONE window of diagonals d = DLO..DHI with BN = 96 / 128 columns per
 // accumulator.  Used for NINE digits (45 products: the W^T W of the inverse, whose operand columns span many orders of magnitude
 // under one scale): d = 6..10 in five 96-column accumulators, then d = 2..5, each launch accumulating into C.
 //
-// Launch flags of launch_ozaki_dgemm only: 512 two-window form of the 8-digit product, 1024 / 4096 window layouts of the 9-digit
-// product, 8192 cluster pairs with a multicast op(B) tile for the 128 x 128 window kernels.
+// Launch flag of launch_ozaki_dgemm only: 512 two-window form of the 8-digit product.
 // Forms (flags, same meaning as dgemm_sm100.cuh): upper only (1), K-from-N (2: triangular operand, masked in the digit extraction),
-// skip tile (0,0) (64), and the tile-mapped forms of the block-cyclic multi-GPU drivers: MAP_UPPER (8), MAP_KUPTO (16: per-column
-// contraction limit, masked in the digit extraction; long K comes in k-chunks <= 32768 with their own scales), MAP_BROWS (32).
+// skip tile (0,0) (64), and, in the single-pass kernel only, the tile-mapped forms of the block-cyclic multi-GPU drivers: MAP_UPPER (8),
+// MAP_KUPTO (16: per-column contraction limit, masked in the digit extraction; long K comes in k-chunks <= 32768 with their own scales).
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -150,34 +149,6 @@ __device__ __forceinline__ void tc_mma_i8(unsigned tmem_d, uint64_t desc_a, uint
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate), "r"(0u), "r"(0u), "r"(0u), "r"(0u)
       : "memory");
 }
-// ---- thread-block-cluster primitives of the multicast variant of the window kernel (oz_gemm_win_mc_kernel) ----
-__device__ __forceinline__ unsigned oz_cluster_ctarank() {
-  unsigned r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;\n" : "=r"(r));
-  return r;
-}
-// every thread of every CTA of the cluster (release / acquire at cluster scope)
-__device__ __forceinline__ void oz_cluster_sync() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;\n" ::: "memory");
-}
-// one TMA load delivered to the SAME shared-memory offset of every CTA in `mask`, completing bytes on the mbarrier at the same
-// offset in each of them (L2 is read once for the whole cluster)
-__device__ __forceinline__ void tma_load_3d_mc(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, unsigned short mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%4, %5, %6}], [%2], %3;\n" ::"r"(
-          (unsigned)__cvta_generic_to_shared(smem_dst)),
-      "l"((uint64_t)map), "r"((unsigned)__cvta_generic_to_shared(bar)), "h"(mask), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-// completion of the MMAs issued so far arrives on the mbarrier at this offset in every CTA of `mask`
-__device__ __forceinline__ void tc_commit_mc(uint64_t* bar, unsigned short mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;\n" ::"r"(
-                   (unsigned)__cvta_generic_to_shared(bar)),
-               "h"(mask)
-               : "memory");
-}
-
 // K-major operand tile with 64-byte rows, SWIZZLE_64B: 8-row groups are 512 bytes apart
 __device__ __forceinline__ uint64_t oz_smem_desc(const void* p) {
   const unsigned a = (unsigned)__cvta_generic_to_shared(p);
@@ -376,8 +347,8 @@ oz_gemm_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const
 // needs four accumulators per launch, i.e. N = 128 per MMA: half as many tensor-pipe instructions for the same work.
 // The digit planes are streamed twice (once per window).  MEASURED (profiles/ozaki_probe_r2p.log): an N = 128 instruction takes
 // twice as long as an N = 64 one -- 73.5 against 69.1 TFLOP/s FP64-equivalent at 8192^3, nothing inside the factorization --
-// so the tensor pipe itself (~2.65 INT8 POPS in this access pattern), not the instruction shape, is the limit.  Kept as the
-// optional variant (launch flag 512, option "ozaki_windows").
+// so the tensor pipe itself (~2.65 INT8 POPS in this access pattern), not the instruction shape, is the limit.  Launch flag 512:
+// the largest products take it (context option "ozaki_win_mink").
 // ---------------------------------------------------------------------------------------------------------------
 template <int S, int BN, int BK, int DLO, int DHI> struct OzWin {
   static constexpr int NACC = DHI - DLO + 1;
@@ -401,22 +372,11 @@ template <int BK> __device__ __forceinline__ uint64_t oz_smem_desc_k(const void*
   return d;
 }
 
-// MC = 1 (oz_gemm_win_mc_kernel, launched as clusters of two CTAs along x): the pair works on the row tiles (2j, 2j + 1) of ONE
-// column tile, so both need the same op(B) tile.  Each CTA loads its own op(A) tile and HALF of the digit planes of the op(B) tile,
-// multicast into both CTAs' shared memory: 25 % fewer bytes read from L2 per product.  MEASURED NEUTRAL (profiles/
-// ozaki_multicast_ab_r2ap.log: 8192^3 14.76 -> 14.74 ms with 8 digits, 18.80 -> 18.23 ms with 9; N = 32768 evaluation 668 -> 667 ms,
-// results bit-identical), so it is off by default: what limits the windows is not the L2 read side of the fill but what each SM
-// takes in and reads back from shared memory -- a multicast still delivers every byte of the tile to both SMs; only
-// cta_group::2 (each SM keeps HALF of op(B)) lowers that.  Protocol: full[s] of a CTA receives its own A bytes + both halves of B; a stage may
-// only be refilled once BOTH CTAs' MMAs have read it, so empty[s] counts two arrivals and every tcgen05.commit of a stage arrives
-// on both CTAs' barriers; cluster barriers after the mbarrier initialisation and before exit keep either CTA from signalling a
-// peer that is not there.  A CTA whose tile is skipped (below the diagonal of an upper-only product, tile (0,0) of a skip-tile
-// product) while its partner's is not runs as a ghost: same loads, same MMAs, no stores.
-template <int S, int BN, int BK, int DLO, int DHI, int MC>
-__device__ __forceinline__ void oz_gemm_win_body(const OzParams& p, const CUtensorMap* pmapA, const CUtensorMap* pmapB) {
+template <int S, int BN, int BK, int DLO, int DHI>
+__global__ void __launch_bounds__(OZ_THREADS, 1)
+oz_gemm_win_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB) {
   using W = OzWin<S, BN, BK, DLO, DHI>;
   constexpr int NST = W::NST, PL = W::PL;
-  static_assert(!MC || (PL % 2 == 0), "the multicast variant splits the digit planes of op(B) in two halves");
   extern __shared__ unsigned char oz_smem_raw[];
   unsigned char* smem = reinterpret_cast<unsigned char*>(((uintptr_t)oz_smem_raw + 1023) & ~(uintptr_t)1023);
   uint64_t* full = reinterpret_cast<uint64_t*>(smem + NST * W::STAGE);
@@ -436,38 +396,16 @@ __device__ __forceinline__ void oz_gemm_win_body(const OzParams& p, const CUtens
     tile_m = first_m + rem % gsize;
     tile_n = rem / gsize;
   }
-  const int blk_n = (tile_n * BN) >> 7;                       // first 128-block of the tile's columns (BN = 256 spans two)
+  const int blk_n = (tile_n * BN) >> 7;                       // first 128-block of the tile's columns
   if (tile_n * BN >= p.N) return;
-  [[maybe_unused]] bool ghost = false;
-  [[maybe_unused]] unsigned crank = 0;
-  if constexpr (!MC) {
-    if ((p.flags & 1) && tile_m > ((tile_n * BN + BN - 1) >> 7)) return;
-    if ((p.flags & 64) && tile_m == 0 && blk_n == 0) return;
-  } else {
-    // the partner holds row tile tile_m ^ 1 of the same column tile (grid x even, GM even: consecutive CTAs of a pair are
-    // consecutive row tiles); the pair leaves only if BOTH tiles are skipped
-    crank = oz_cluster_ctarank();
-    const int last_blk = (tile_n * BN + BN - 1) >> 7;
-    const bool skip_me = ((p.flags & 1) && tile_m > last_blk) || ((p.flags & 64) && tile_m == 0 && blk_n == 0);
-    const int pm = tile_m ^ 1;
-    const bool skip_peer = ((p.flags & 1) && pm > last_blk) || ((p.flags & 64) && pm == 0 && blk_n == 0);
-    if (skip_me && skip_peer) return;
-    ghost = skip_me;
-  }
-  int gt = 0;
-  if (p.flags & 8) {
-    gt = p.col_gtile[blk_n];
-    if (p.row_gtile0 + tile_m > gt) return;
-  }
+  if ((p.flags & 1) && tile_m > ((tile_n * BN + BN - 1) >> 7)) return;
+  if ((p.flags & 64) && tile_m == 0 && blk_n == 0) return;
   const int kt0 = (p.flags & 2) ? max(0, blk_n * 128 - p.k_off) / BK : 0;
   const int KT = p.K / BK - kt0;
   const int m0 = tile_m * OZ_BM, n0 = tile_n * BN;
-  // GEMM_MAP_BROWS (flag 32, BN = 128 with flag 8): the op(B) columns of this tile column are the columns gt * 128 .. of the operand
-  // (the W W^T accumulation of the block-cyclic lauum reads its column panel by GLOBAL position), C stays local
-  const int nB = (p.flags & 32) ? gt * 128 + (n0 & 127) : n0;
 
   if (tid == 0) {
-    for (int s = 0; s < NST; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], MC ? 2 : 1); }
+    for (int s = 0; s < NST; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
     mbar_init(tfull, 1);
     mbar_fence_init();
   }
@@ -477,7 +415,6 @@ __device__ __forceinline__ void oz_gemm_win_body(const OzParams& p, const CUtens
   }
   tc_fence_before();
   __syncthreads();
-  if constexpr (MC) oz_cluster_sync();      // the peer's barriers exist before anything is multicast to them
   tc_fence_after();
   const unsigned tmem_base = *tmem_slot;
 
@@ -488,14 +425,8 @@ __device__ __forceinline__ void oz_gemm_win_body(const OzParams& p, const CUtens
         if (kt >= NST) oz_wait(&empty[s], (unsigned)((kt / NST - 1) & 1));
         unsigned char* st = smem + (size_t)s * W::STAGE;
         mbar_expect_tx(&full[s], (unsigned)W::STAGE);
-        tma_load_3d(st, pmapA, &full[s], (kt0 + kt) * BK, m0, 0);                               // PL x 128 x BK
-        if constexpr (!MC) {
-          tma_load_3d(st + (size_t)PL * OZ_BM * BK, pmapB, &full[s], (kt0 + kt) * BK, nB, 0);   // PL x BN  x BK
-        } else {
-          // planes crank * PL/2 .. of the op(B) tile into both CTAs (the map's box holds PL / 2 planes)
-          tma_load_3d_mc(st + (size_t)PL * OZ_BM * BK + (size_t)crank * (PL / 2) * BN * BK, pmapB, &full[s], (kt0 + kt) * BK, nB,
-                         (int)crank * (PL / 2), (unsigned short)0x3);
-        }
+        tma_load_3d(st, &mapA, &full[s], (kt0 + kt) * BK, m0, 0);                               // PL x 128 x BK
+        tma_load_3d(st + (size_t)PL * OZ_BM * BK, &mapB, &full[s], (kt0 + kt) * BK, n0, 0);     // PL x BN  x BK
       }
     }
   } else if (warp == 1) {
@@ -530,7 +461,7 @@ __device__ __forceinline__ void oz_gemm_win_body(const OzParams& p, const CUtens
             }
           }
         }
-        if constexpr (MC) tc_commit_mc(&empty[s], (unsigned short)0x3); else tc_commit(&empty[s]);
+        tc_commit(&empty[s]);
       }
       __syncwarp();
     }
@@ -541,16 +472,11 @@ __device__ __forceinline__ void oz_gemm_win_body(const OzParams& p, const CUtens
     const int q = warp & 3;
     const int row = 32 * q + lane;
     const unsigned lane_addr = tmem_base + ((unsigned)(32 * q) << 16);
-    // rows below the diagonal of a diagonal tile stay untouched: local product (flag 1) by global index, tile-mapped form
-    // (flag 8, BN <= 128 only) by the position inside the 128-block
-    const bool diag_local = (p.flags & 1) && !(p.flags & 8) && (tile_m >= blk_n);
-    const bool diag_map = (p.flags & 8) && (p.row_gtile0 + tile_m == gt);
-    const int coff = n0 & 127;
+    const bool diag_local = (p.flags & 1) && (tile_m >= blk_n);     // upper only: rows below the diagonal stay untouched
     const double sa = p.scaleA[m0 + row] * p.alpha;
     double* Crow = p.C + (long long)(m0 + row) + (long long)n0 * p.ldc;
     for (int c0 = 0; c0 < BN; c0 += 16) {
       if (n0 + c0 >= p.N) break;
-      if constexpr (MC) { if (ghost) break; }
       double acc[16];
 #pragma unroll
       for (int j = 0; j < 16; ++j) acc[j] = 0.0;
@@ -571,9 +497,8 @@ __device__ __forceinline__ void oz_gemm_win_body(const OzParams& p, const CUtens
       for (int j = 0; j < 16; ++j) {
         const int col = c0 + j;
         if (diag_local && m0 + row > n0 + col) continue;
-        if (diag_map && row > col + coff) continue;
         double* cp = Crow + (long long)col * p.ldc;
-        double r = acc[j] * sa * p.scaleB[nB + col];
+        double r = acc[j] * sa * p.scaleB[n0 + col];
         if (p.E) r *= p.E[(long long)(m0 + row) + (long long)(n0 + col) * p.lde];       // Hadamard epilogue: linear, so every window applies it
         *cp = (p.beta != 0.0) ? fma(p.beta, *cp, r) : r;
       }
@@ -581,23 +506,10 @@ __device__ __forceinline__ void oz_gemm_win_body(const OzParams& p, const CUtens
     tc_fence_before();
   }
   __syncthreads();
-  if constexpr (MC) oz_cluster_sync();      // no CTA leaves while its peer may still signal its barriers
   if (warp == 1) {
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;\n" ::"r"(tmem_base) : "memory");
   }
-}
-
-template <int S, int BN, int BK, int DLO, int DHI>
-__global__ void __launch_bounds__(OZ_THREADS, 1)
-oz_gemm_win_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB) {
-  oz_gemm_win_body<S, BN, BK, DLO, DHI, 0>(p, &mapA, &mapB);
-}
-// cluster pairs with a multicast op(B) tile; mapB's box holds PL / 2 digit planes
-template <int S, int BN, int BK, int DLO, int DHI>
-__global__ void __launch_bounds__(OZ_THREADS, 1)
-oz_gemm_win_mc_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB) {
-  oz_gemm_win_body<S, BN, BK, DLO, DHI, 1>(p, &mapA, &mapB);
 }
 
 // ---- host side ----
@@ -629,41 +541,17 @@ inline bool oz_make_map_k(CUtensorMap* map, const int8_t* base, uint64_t Kp, uin
 }
 using OzWinLo = OzWin<8, 128, 32, 6, 9>;
 using OzWinHi = OzWin<8, 128, 64, 2, 5>;      // (k-tiles of 32 with seven stages instead of 64 with three: measured slower, 20.1 vs 18.7 ms per 8192^3 nine-digit product)
-using OzWin9X = OzWin<9, 128, 32, 10, 10>;    // ninth digit: the extra diagonal d = 10 (pairs (1,9) .. (9,1))
 using OzWin9Z = OzWin<9, 96, 32, 6, 10>;      // nine digits in TWO windows: d = 6..10 in five 96-column accumulators (480 TMEM columns, 35 pairs)
-using OzWin9Y = OzWin<9, 256, 32, 10, 10>;    // the same with 128 x 256 tiles (one accumulator of 256 columns): 25% fewer operand bytes per product
 
 inline cudaError_t oz_set_attr() {
   cudaError_t e = cudaFuncSetAttribute(oz_gemm_win_kernel<8, 128, 32, 6, 9>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OzWinLo::SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(oz_gemm_win_kernel<8, 128, 64, 2, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OzWinHi::SMEM);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(oz_gemm_win_kernel<9, 128, 32, 10, 10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OzWin9X::SMEM);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(oz_gemm_win_kernel<9, 256, 32, 10, 10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OzWin9Y::SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(oz_gemm_win_kernel<9, 96, 32, 6, 10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OzWin9Z::SMEM);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(oz_gemm_win_mc_kernel<8, 128, 32, 6, 9>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OzWinLo::SMEM);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(oz_gemm_win_mc_kernel<8, 128, 64, 2, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OzWinHi::SMEM);
   if (e == cudaSuccess) e = oz_set_attr_s<8>();
   if (e == cudaSuccess) e = oz_set_attr_s<7>();
   if (e == cudaSuccess) e = oz_set_attr_s<6>();
   if (e == cudaSuccess) e = oz_set_attr_s<2>();
   return e;
-}
-
-// launch of a window kernel as clusters of two CTAs along x (grid.x even)
-template <typename Kern>
-inline cudaError_t oz_launch_pairs(Kern kern, dim3 grid, size_t smem, cudaStream_t st, const OzParams& p, const CUtensorMap& a, const CUtensorMap& b) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3(OZ_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = 2;
-  at[0].val.clusterDim.y = 1;
-  at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kern, p, a, b);
 }
 
 // workspace (bytes) for the digit planes and scales of one product
@@ -673,16 +561,18 @@ inline size_t oz_workspace_bytes(int M, int N, int K, int S) {
 }
 
 // C = alpha A^T B + beta C through the int8 tensor cores.  M % 128 == 0, N % 128 == 0, K % 128 == 0, K <= 32768.
-// flags: GEMM_UPPER_ONLY (1), GEMM_K_FROM_N (2), GEMM_SKIP_TILE00 (64).  When A and B are the same matrix (the symmetric
+// flags: GEMM_UPPER_ONLY (1), GEMM_K_FROM_N (2), GEMM_SKIP_TILE00 (64), 512 (above); the tile-mapped MAP_UPPER (8) and MAP_KUPTO (16)
+// and the timing probe (256) are forms of the single-pass kernel (S <= 8 without 512).  When A and B are the same matrix (the symmetric
 // updates of potrf and the W^T W product of the inverse) its digit planes are formed once and shared.
 inline cudaError_t launch_ozaki_dgemm(cudaStream_t st, int M, int N, int K, int S, double alpha, const double* A, long long lda, const double* B,
                                       long long ldb, double beta, double* C, long long ldc, int flags, void* workspace, int k_off = 0,
                                       const int* col_gtile = nullptr, int row_gtile0 = 0, int k_gtile0 = 0, const double* E = nullptr,
                                       long long lde = 0) {
-  if (E && (flags & (8 | 16 | 32))) return cudaErrorInvalidValue;                    // Hadamard epilogue: plain forms only
-  if ((flags & (8 | 16)) && !col_gtile) return cudaErrorInvalidValue;
-  if ((flags & 32) && (S != 9 || !(flags & 8))) return cudaErrorInvalidValue;      // mapped B rows: nine-digit window kernels, tile-mapped form only
-  if ((flags & 16) && (S == 9 || (flags & (1 | 2 | 8 | 64 | 512)) || (A == B && lda == ldb))) return cudaErrorInvalidValue;   // KUPTO: plain 8-digit kernel only
+  if (flags & ~(1 | 2 | 8 | 16 | 64 | 256 | 512)) return cudaErrorInvalidValue;
+  if (E && (flags & (8 | 16))) return cudaErrorInvalidValue;                         // Hadamard epilogue: plain forms only
+  if ((flags & (8 | 16)) && (!col_gtile || S == 9 || (flags & 512))) return cudaErrorInvalidValue;   // tile-mapped: single-pass kernel only
+  if ((flags & 16) && ((flags & (1 | 2 | 8 | 64)) || (A == B && lda == ldb))) return cudaErrorInvalidValue;   // KUPTO: plain form only
+  if (S == 9 && (flags & 64)) return cudaErrorInvalidValue;                           // a 96-wide tile straddles tile (0,0)'s columns
   if ((S != 9 && S != 8 && S != 7 && S != 6 && S != 2) || (M % OZ_BM) || (N % 128) || (K % 128) || K > 32768) return cudaErrorInvalidValue;
   const size_t Kp = (size_t)K;
   const bool shared = (A == B && lda == ldb);
@@ -700,77 +590,32 @@ inline cudaError_t launch_ozaki_dgemm(cudaStream_t st, int M, int N, int K, int 
     if (flags & 16) oz_slice_kernel<<<(N + 7) / 8, 256, 0, st>>>(B, ldb, K, N, S, pb, (long long)Kp, N, sb, 2, k_off, col_gtile, k_gtile0);
     else oz_slice_kernel<<<(N + 7) / 8, 256, 0, st>>>(B, ldb, K, N, S, pb, (long long)Kp, N, sb, kfrom, k_off);
   }
+  const OzParams p{M, N, K, S, alpha, beta, C, ldc, sa, sb, flags & ~512, k_off, col_gtile, row_gtile0, k_gtile0, E, lde};
+  if (S == 9 || (S == 8 && (flags & 512))) {
+    // Two windows of diagonals, lowest order first, the second accumulating into C.
+    // NINE digits (products whose operands span several orders of magnitude under one scale per column: the W^T W of the inverse):
+    // nine 64-column accumulators do not fit the 512 TMEM columns, so d = 6..10 runs in five 96-column accumulators (35 pairs,
+    // 128 x 96 tiles; the last column tile is partial: TMA zero fill, masked epilogue), then d = 2..5 (10 pairs, 128 x 128 tiles):
+    // 19.4 ms at 8192^3.
+    // EIGHT digits (flag 512): d = 6..9 then d = 2..5, 128 x 128 tiles; measured 73.5 against 69.1 TFLOP/s at 8192^3 and no gain inside
+    // the factorization below 8192, so the single-pass 128 x 64 kernel stays the default there.  ncu (profiles/ozaki_ncu_full_r2t.md):
+    // the single-pass kernel keeps the tensor-core pipe 94 % busy (sm__pipe_tc_cycles_active; every N = 64 product re-reads its 4 KB
+    // A operand from shared memory), the windows load the planes twice and sit at 81 % of the L2 -> SM fill rate instead.
+    const bool nine = (S == 9);
+    const int plLo = nine ? OzWin9Z::PL : OzWinLo::PL, bnLo = nine ? 96 : 128;
+    CUtensorMap aLo, bLo, aHi, bHi;
+    if (!oz_make_map_k(&aLo, pa, Kp, (uint64_t)Ra, S, plLo, OZ_BM, 32) || !oz_make_map_k(&bLo, pb, Kp, (uint64_t)Rb, S, plLo, bnLo, 32) ||
+        !oz_make_map_k(&aHi, pa, Kp, (uint64_t)Ra, S, OzWinHi::PL, OZ_BM, 64) || !oz_make_map_k(&bHi, pb, Kp, (uint64_t)Rb, S, OzWinHi::PL, 128, 64))
+      return cudaErrorInvalidValue;
+    if (nine) oz_gemm_win_kernel<9, 96, 32, 6, 10><<<dim3(M / OZ_BM, (N + 95) / 96), OZ_THREADS, OzWin9Z::SMEM, st>>>(p, aLo, bLo);
+    else oz_gemm_win_kernel<8, 128, 32, 6, 9><<<dim3(M / OZ_BM, N / 128), OZ_THREADS, OzWinLo::SMEM, st>>>(p, aLo, bLo);
+    OzParams p2 = p;
+    p2.beta = 1.0;
+    oz_gemm_win_kernel<8, 128, 64, 2, 5><<<dim3(M / OZ_BM, N / 128), OZ_THREADS, OzWinHi::SMEM, st>>>(p2, aHi, bHi);
+    return cudaGetLastError();
+  }
   CUtensorMap mA, mB;
   if (!oz_make_map(&mA, pa, Kp, (uint64_t)Ra, S, OZ_BM) || !oz_make_map(&mB, pb, Kp, (uint64_t)Rb, S, OZ_BN)) return cudaErrorInvalidValue;
-  OzParams p{M, N, K, S, alpha, beta, C, ldc, sa, sb, flags & ~(512 | 1024 | 4096 | 8192), k_off, col_gtile, row_gtile0, k_gtile0, E, lde};
-  // flag 8192: cluster pairs with a multicast op(B) tile for the 128 x 128 window kernels (plain forms with an even number of row tiles)
-  const bool mc = (flags & 8192) && !(flags & (8 | 16 | 32)) && (M % (2 * OZ_BM)) == 0;
-  if (S == 9) {
-    // nine digits (products whose operands span several orders of magnitude under one scale per column: the W^T W of the inverse).
-    // Nine 64-column accumulators do not fit the 512 TMEM columns, so the diagonals are summed in windows, lowest order first, each
-    // launch accumulating into C.  Default: TWO windows -- d = 6..10 in five 96-column accumulators (35 pairs, 128 x 96 tiles), then
-    // d = 2..5 (10 pairs, 128 x 128 tiles): 19.4 ms at 8192^3.  Flag 4096: three windows d = 10 | 6..9 | 2..5 (24.3 ms; ncu, profiles/
-    // ozaki_ncu_full_r2t.md: the d = 10 window moves all nine planes for nine products and sits at 93 % of the L2 -> SM fill rate)
-    CUtensorMap aX, bX, aLo, bLo, aHi, bHi;
-    if (!oz_make_map_k(&aX, pa, Kp, (uint64_t)Ra, S, OzWin9X::PL, OZ_BM, 32) || !oz_make_map_k(&bX, pb, Kp, (uint64_t)Rb, S, OzWin9X::PL, 128, 32) ||
-        !oz_make_map_k(&aLo, pa, Kp, (uint64_t)Ra, S, OzWinLo::PL, OZ_BM, 32) || !oz_make_map_k(&bLo, pb, Kp, (uint64_t)Rb, S, OzWinLo::PL, 128, 32) ||
-        !oz_make_map_k(&aHi, pa, Kp, (uint64_t)Ra, S, OzWinHi::PL, OZ_BM, 64) || !oz_make_map_k(&bHi, pb, Kp, (uint64_t)Rb, S, OzWinHi::PL, 128, 64))
-      return cudaErrorInvalidValue;
-    dim3 grid2(M / OZ_BM, N / 128);
-    if (!(flags & 4096) && !(flags & (8 | 64))) {
-      // two windows: d = 6..10 with 128 x 96 tiles (the last column tile is partial: TMA zero fill, masked epilogue), then d = 2..5
-      CUtensorMap aZ, bZ;
-      if (!oz_make_map_k(&aZ, pa, Kp, (uint64_t)Ra, S, OzWin9Z::PL, OZ_BM, 32) || !oz_make_map_k(&bZ, pb, Kp, (uint64_t)Rb, S, OzWin9Z::PL, 96, 32))
-        return cudaErrorInvalidValue;
-      oz_gemm_win_kernel<9, 96, 32, 6, 10><<<dim3(M / OZ_BM, (N + 95) / 96), OZ_THREADS, OzWin9Z::SMEM, st>>>(p, aZ, bZ);
-      OzParams pz = p;
-      pz.beta = 1.0;
-      if (mc) {
-        CUtensorMap bHiH;
-        if (!oz_make_map_k(&bHiH, pb, Kp, (uint64_t)Rb, S, OzWinHi::PL / 2, 128, 64)) return cudaErrorInvalidValue;
-        cudaError_t e = oz_launch_pairs(oz_gemm_win_mc_kernel<8, 128, 64, 2, 5>, grid2, OzWinHi::SMEM, st, pz, aHi, bHiH);
-        return e != cudaSuccess ? e : cudaGetLastError();
-      }
-      oz_gemm_win_kernel<8, 128, 64, 2, 5><<<grid2, OZ_THREADS, OzWinHi::SMEM, st>>>(pz, aHi, bHi);
-      return cudaGetLastError();
-    }
-    if ((flags & 1024) && !(flags & (8 | 64))) {
-      CUtensorMap bY;
-      if (!oz_make_map_k(&bY, pb, Kp, (uint64_t)Rb, S, OzWin9Y::PL, 256, 32)) return cudaErrorInvalidValue;
-      oz_gemm_win_kernel<9, 256, 32, 10, 10><<<dim3(M / OZ_BM, (N + 255) / 256), OZ_THREADS, OzWin9Y::SMEM, st>>>(p, aX, bY);
-    } else {
-      oz_gemm_win_kernel<9, 128, 32, 10, 10><<<grid2, OZ_THREADS, OzWin9X::SMEM, st>>>(p, aX, bX);
-    }
-    OzParams p2 = p;
-    p2.beta = 1.0;
-    oz_gemm_win_kernel<8, 128, 32, 6, 9><<<grid2, OZ_THREADS, OzWinLo::SMEM, st>>>(p2, aLo, bLo);
-    oz_gemm_win_kernel<8, 128, 64, 2, 5><<<grid2, OZ_THREADS, OzWinHi::SMEM, st>>>(p2, aHi, bHi);
-    return cudaGetLastError();
-  }
-  if (S == 8 && (flags & 512)) {
-    // two diagonal windows, 128 x 128 tiles (flag 512; measured 73.5 against 69.1 TFLOP/s at 8192^3 and no gain inside the
-    // factorization, so the single-pass 128 x 64 kernel stays the default).  ncu (profiles/ozaki_ncu_full_r2t.md): the single-pass
-    // kernel keeps the tensor-core pipe 94 % busy (sm__pipe_tc_cycles_active; every N = 64 product re-reads its 4 KB A operand from
-    // shared memory), the windows load the planes twice and sit at 81 % of the L2 -> SM fill rate instead)
-    CUtensorMap aLo, bLo, aHi, bHi;
-    if (!oz_make_map_k(&aLo, pa, Kp, (uint64_t)Ra, S, OzWinLo::PL, OZ_BM, 32) || !oz_make_map_k(&bLo, pb, Kp, (uint64_t)Rb, S, OzWinLo::PL, 128, 32) ||
-        !oz_make_map_k(&aHi, pa, Kp, (uint64_t)Ra, S, OzWinHi::PL, OZ_BM, 64) || !oz_make_map_k(&bHi, pb, Kp, (uint64_t)Rb, S, OzWinHi::PL, 128, 64))
-      return cudaErrorInvalidValue;
-    dim3 grid2(M / OZ_BM, N / 128);
-    OzParams p2 = p;
-    p2.beta = 1.0;
-    if (mc) {
-      CUtensorMap bLoH, bHiH;
-      if (!oz_make_map_k(&bLoH, pb, Kp, (uint64_t)Rb, S, OzWinLo::PL / 2, 128, 32) || !oz_make_map_k(&bHiH, pb, Kp, (uint64_t)Rb, S, OzWinHi::PL / 2, 128, 64))
-        return cudaErrorInvalidValue;
-      cudaError_t e = oz_launch_pairs(oz_gemm_win_mc_kernel<8, 128, 32, 6, 9>, grid2, OzWinLo::SMEM, st, p, aLo, bLoH);
-      if (e == cudaSuccess) e = oz_launch_pairs(oz_gemm_win_mc_kernel<8, 128, 64, 2, 5>, grid2, OzWinHi::SMEM, st, p2, aHi, bHiH);
-      return e != cudaSuccess ? e : cudaGetLastError();
-    }
-    oz_gemm_win_kernel<8, 128, 32, 6, 9><<<grid2, OZ_THREADS, OzWinLo::SMEM, st>>>(p, aLo, bLo);     // low-order diagonals first: C = ... + beta C
-    oz_gemm_win_kernel<8, 128, 64, 2, 5><<<grid2, OZ_THREADS, OzWinHi::SMEM, st>>>(p2, aHi, bHi);    // high-order diagonals accumulate
-    return cudaGetLastError();
-  }
   dim3 grid(M / OZ_BM, N / OZ_BN);
   if (S == 8) oz_gemm_kernel<8><<<grid, OZ_THREADS, oz_smem_bytes(8), st>>>(p, mA, mB);
   else if (S == 7) oz_gemm_kernel<7><<<grid, OZ_THREADS, oz_smem_bytes(7), st>>>(p, mA, mB);

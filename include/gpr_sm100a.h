@@ -98,10 +98,8 @@ const char* gpr_last_error(gpr_ctx* ctx);          /* ctx may be NULL: last erro
  *   "ozaki" FP64 products on the INT8 tensor cores: -1 automatic from a condition-number bound [default], 0 off, 6 / 7 / 8 digits forced;
  *   "ozaki_lauum" digits of the inverse's W^T W product on that route: 9 [default], 8, 0 = DMMA; "ozaki_split" the same for the
  *   split-predict mean products; "ozaki_min" smallest routed M, N, K [1024];
- *   "ozaki_phases" bit mask potrf 1 | trtri 2 | other solves 8 [11]; "ozaki_panel", "ozaki_kchunk" k-panels [32768]; "ozaki_windows" kernel variants [0];
- *   "ozaki_win_mink" smallest M, N, K for the two-window form of the 8-digit product [8192];
- *   "ozaki_mc" 0/1 [0; environment GPR_OZ_MC overrides the default]: the 128 x 128 window kernels of that route as clusters of two CTAs
- *   sharing one op(B) tile through a multicast TMA load (bit-identical results; measured neutral, profiles/ozaki_multicast_ab_r2ap.log). */
+ *   "ozaki_phases" bit mask potrf 1 | trtri 2 | other solves 8 [11]; "ozaki_panel", "ozaki_kchunk" k-panels [32768];
+ *   "ozaki_win_mink" smallest M, N, K for the two-window form of the 8-digit product [8192]. */
 int gpr_ctx_set_option(gpr_ctx* ctx, const char* name, int64_t value);
 int64_t gpr_ctx_launch_count(gpr_ctx* ctx);        /* kernels launched by this context so far */
 
@@ -192,7 +190,8 @@ int gpr_dbg_dgemm(gpr_ctx* ctx, char transA, char transB, int M, int N, int K, d
  * tensor cores (tcgen05.mma kind::i8 with TMEM accumulators): Ozaki-type splitting of every row of A^T and column of B
  * into S signed 7-bit digits, S (S + 1) / 2 exact integer products, FP64 recombination (csrc/ozaki_i8.cuh).
  * M % 128 == 0, N % 128 == 0, K % 128 == 0, K <= 32768, S in {2, 6, 7, 8, 9} (9: two diagonal windows, 45 products).
- * flags: 1 = upper only, 2 = K-from-N, 512 / 1024 / 4096 = kernel variants (csrc/ozaki_i8.cuh). */
+ * flags: 1 = upper only, 2 = K-from-N, 64 = skip tile (0,0) (not with S = 9), 512 = two-window form of the 8-digit product
+ * (csrc/ozaki_i8.cuh); any other flag returns an error. */
 int gpr_dbg_ozaki_dgemm(gpr_ctx* ctx, int M, int N, int K, int S, double alpha, const double* A, int64_t lda, const double* B,
                         int64_t ldb, double beta, double* C, int64_t ldc, int flags, int reps, double* ms);
 /* factor (and optionally invert) a host SPD matrix in place through the blocked path; A is N x N.

@@ -475,11 +475,11 @@ def test_ozaki_int8_gemm_is_an_fp64_product(gpr):
         ctx.close()
 
 
-def test_ozaki_nine_digit_product(gpr):
+def test_ozaki_nine_digit_two_window_product(gpr):
     """The W^T W product of the inverse takes NINE digits (csrc/ozaki_i8.cuh: 45 integer products in two diagonal windows,
-    d = 6..10 with 128 x 96 tiles | d = 2..5; a three-window form is kept behind a flag): on operands whose entries span many
-    orders of magnitude under one scale per column it must be at least 16x closer to the exact product than the 8-digit form,
-    and honour upper-only / K-from-N (lauum_oop_t's flags) on a size that is no multiple of the 96- and 256-wide tiles."""
+    d = 6..10 with 128 x 96 tiles | d = 2..5): on operands whose entries span many orders of magnitude under one scale per column
+    it must be at least 16x closer to the exact product than the 8-digit form, and honour upper-only / K-from-N (lauum_oop_t's
+    flags) on a size that is no multiple of the 96-wide tiles."""
     from gpr_sm100a import _ffi
     rng = np.random.default_rng(77)
     ctx = gpr.Context(0)
@@ -490,14 +490,12 @@ def test_ozaki_nine_digit_product(gpr):
         den = np.abs(A).T @ np.abs(A)
         err = {}
         out = {}
-        for S, fl in ((8, 0), (9, 0), (9, 4096), (9, 4096 | 1024)):       # 9 digits: two windows (default) | three | three with 128 x 256 tiles
-            out[(S, fl)], _ = _ffi.dbg_ozaki_dgemm(ctx, 1.0, A, A, 0.0, np.zeros((M, M)), S=S, flags=fl)
-            err[(S, fl)] = float(np.max(np.abs(out[(S, fl)] - ref) / den))
-        print(f"\nW^T W with 6 decades inside a column: err/(|A|^T|A|) 8 digits {err[(8, 0)]:.2e}, 9 digits {err[(9, 0)]:.2e} (two windows), "
-              f"{err[(9, 4096)]:.2e} (three), {err[(9, 4096 | 1024)]:.2e} (three, 128x256)")
-        assert max(err[(9, 0)], err[(9, 4096)], err[(9, 4096 | 1024)]) < 2e-15
-        assert err[(9, 0)] * 16 <= err[(8, 0)] or err[(8, 0)] < 1e-15
-        assert np.array_equal(out[(9, 4096)], out[(9, 4096 | 1024)])          # same windows, same order of summation
+        for S in (8, 9):
+            out[S], _ = _ffi.dbg_ozaki_dgemm(ctx, 1.0, A, A, 0.0, np.zeros((M, M)), S=S, flags=0)
+            err[S] = float(np.max(np.abs(out[S] - ref) / den))
+        print(f"\nW^T W with 6 decades inside a column: err/(|A|^T|A|) 8 digits {err[8]:.2e}, 9 digits {err[9]:.2e}")
+        assert err[9] < 2e-15
+        assert err[9] * 16 <= err[8] or err[8] < 1e-15
         # lauum_oop_t's form: lower-triangular operand (garbage above the diagonal blocks), upper triangle of C only
         Kt = 640
         L = np.tril(rng.standard_normal((Kt, Kt))) + 4 * np.eye(Kt)
@@ -508,48 +506,35 @@ def test_ozaki_nine_digit_product(gpr):
         reft = L.astype(np.longdouble).T @ L.astype(np.longdouble)
         dent = np.abs(L).T @ np.abs(L)
         C0 = np.asfortranarray(rng.standard_normal((Kt, Kt)))
-        for fl in (3, 3 | 4096, 3 | 4096 | 1024):
-            Cm, _ = _ffi.dbg_ozaki_dgemm(ctx, 1.0, np.asfortranarray(L), G, 0.0, C0, S=9, flags=fl)      # separate operands: only op(B) is masked
-            up = np.triu(np.ones((Kt, Kt), dtype=bool))
-            e = float(np.max((np.abs(Cm - reft) / dent)[up]))
-            print(f"L^T L, K-from-N + upper-only, flags {fl}: err {e:.2e}")
-            assert e < 2e-15
-            assert np.array_equal(Cm[~up], C0[~up])
+        Cm, _ = _ffi.dbg_ozaki_dgemm(ctx, 1.0, np.asfortranarray(L), G, 0.0, C0, S=9, flags=3)      # separate operands: only op(B) is masked
+        up = np.triu(np.ones((Kt, Kt), dtype=bool))
+        e = float(np.max((np.abs(Cm - reft) / dent)[up]))
+        print(f"L^T L, K-from-N + upper-only: err {e:.2e}")
+        assert e < 2e-15
+        assert np.array_equal(Cm[~up], C0[~up])
     finally:
         ctx.close()
 
 
-def test_ozaki_multicast_pairs_are_bit_identical(gpr):
-    """csrc/ozaki_i8.cuh, launch flag 8192 (ctx option "ozaki_mc"): the 128 x 128 window kernels launched as clusters of two CTAs that
-    share one op(B) tile through a multicast TMA load.  Integer products are exact and the epilogue is the same code, so the result
-    must equal the single-CTA windows BIT FOR BIT -- for the 8-digit two-window product (flag 512) and the second window of the
-    9-digit product, in the plain, upper-only (ghost CTAs below the diagonal), K-from-N and skip-tile(0,0) forms, with beta != 0,
-    on row counts that are multiples of 256 (pairs) and on one that is not (falls back to single CTAs)."""
+def test_ozaki_rejects_retired_forms(gpr):
+    """Forms of the INT8 product that no kernel serves fail cleanly: option names of retired variants are unknown to the
+    context, and launch_ozaki_dgemm refuses nine digits with the tile-mapped or skip-tile forms, the two-window 8-digit form
+    with the tile-mapped forms, and flags it does not know.  The context stays usable afterwards."""
     from gpr_sm100a import _ffi
-    rng = np.random.default_rng(2024)
+    rng = np.random.default_rng(5)
     ctx = gpr.Context(0)
     try:
-        for (M, N, K, S, base, beta) in ((512, 512, 1024, 8, 512, 0.0), (768, 512, 2048, 8, 512, 0.5), (512, 768, 512, 8, 512 | 1, 1.0),
-                                         (1024, 1024, 1024, 8, 512 | 1 | 2, 0.0), (512, 512, 640, 8, 512 | 64, 1.0), (512, 512, 640, 8, 512 | 1 | 64, 1.0),
-                                         (1024, 1024, 1024, 9, 0, 0.0), (768, 768, 768, 9, 1 | 2, 0.25), (384, 384, 512, 8, 512, 0.0),
-                                         (2304, 2304, 4096, 8, 512 | 1, 1.0)):
-            if base & 2:
-                A = np.tril(rng.standard_normal((K, M)))
-                for J in range(M // 128):
-                    A[:128 * J, 128 * J:128 * (J + 1)] = 1e30          # garbage above the diagonal blocks, masked by the digit extraction
-                B = A
-            elif S == 9:
-                A = rng.standard_normal((K, M)) * np.exp(rng.uniform(-8, 0, (K, M)))
-                B = A
-            else:
-                A, B = rng.standard_normal((K, M)), rng.standard_normal((K, N))
-            A, B = np.asfortranarray(A), np.asfortranarray(B)
-            C0 = np.asfortranarray(rng.standard_normal((M, N)))
-            C1, _ = _ffi.dbg_ozaki_dgemm(ctx, 1.0, A, B, beta, C0, S=S, flags=base)
-            C2, _ = _ffi.dbg_ozaki_dgemm(ctx, 1.0, A, B, beta, C0, S=S, flags=base | 8192)
-            assert np.array_equal(C1, C2), (M, N, K, S, base, float(np.abs(C1 - C2).max()))
-            if base & 64:
-                assert np.array_equal(C2[:128, :128], C0[:128, :128])      # tile (0,0) untouched by the ghost CTA
+        for name in ("ozaki_mc", "ozaki_windows", "ozaki_lauum_map"):
+            with pytest.raises(_ffi.GPRError, match="unknown option"):
+                ctx.set_option(name, 0)
+        A = np.asfortranarray(rng.standard_normal((256, 256)))
+        C0 = np.zeros((256, 256), order="F")
+        for S, fl in ((9, 8), (9, 16), (9, 32), (9, 64), (9, 1 | 64), (8, 512 | 8), (8, 512 | 16), (8, 1024), (8, 4096), (8, 8192),
+                      (9, 1024), (9, 4096), (8, 512 | 8192), (8, 32)):
+            with pytest.raises(_ffi.GPRError):
+                _ffi.dbg_ozaki_dgemm(ctx, 1.0, A, A, 0.0, C0, S=S, flags=fl)
+        C, _ = _ffi.dbg_ozaki_dgemm(ctx, 1.0, A, A, 0.0, C0, S=9, flags=3)
+        assert np.all(np.isfinite(C))
     finally:
         ctx.close()
 
@@ -860,36 +845,36 @@ def test_mgpu_rank_count_independence_n8192(gpr):
 
 
 @pytest.mark.parametrize("G", [1, 2, 3])
-def test_mgpu_potrf_on_int8_tensor_cores_vs_oracle(gpr, G):
+def test_mgpu_int8_routes_vs_oracle(gpr, G):
     """The tile-mapped products of the block-cyclic drivers (csrc/dist_blocked.hpp) through the INT8-tensor-core product
     (csrc/ozaki_i8.cuh; nb = 1024 so that they reach the route): the rank-nb trailing updates of potrf (GEMM_MAP_UPPER) and the
     row-panel recurrence of trtri (GEMM_MAP_KUPTO: per-column contraction limit, long K cut into k-chunks with their own digit
     scales -- ozaki_kchunk = 2048 exercises the chunk loop) against the committed oracle values of config 2 (N = 8192, D = 8,
-    SquaredExp()+WhiteNoise(), set A), and the W W^T accumulation of lauum with nine digits (GEMM_MAP_UPPER | GEMM_MAP_BROWS, shared
-    digit planes of the column panel): forced on, automatic, without lauum, potrf only, off."""
+    SquaredExp()+WhiteNoise(), set A): forced on with k-chunks, automatic, forced on, potrf only, off.  The automatic rule picks
+    8 digits for this model, so that leg takes the forced leg's route."""
     from gpr_sm100a import _ffi
     mg2 = _load_module("mg2", "make_golden_config2.py")
     x, y, sets = mg2.inputs()
     g = np.load(os.path.join(HERE, "golden", "config2_n8192.npz"))
     hp = sets["A"]
     launches = {}
-    for forced, phases, kchunk, lauum in ((8, 11, 2048, 9), (-1, 11, 32768, 9), (8, 11, 32768, 0), (8, 1, 32768, 0), (0, 11, 32768, 9)):
+    for forced, phases, kchunk in ((8, 11, 2048), (-1, 11, 32768), (8, 11, 32768), (8, 1, 32768), (0, 11, 32768)):
         mc = _ffi.MultiContext(_devices(G), nb=1024)
         mc.set_option("ozaki", forced)
         mc.set_option("ozaki_phases", phases)
         mc.set_option("ozaki_kchunk", kchunk)
-        mc.set_option("ozaki_lauum_map", 1 if lauum else 0)          # W W^T accumulation of lauum: nine-digit tile-mapped form with mapped
-        #                                                              B rows (off by default: slower at K = nb) / DMMA
         mm = _ffi.MultiModelHandle(mc, [1, 2], 8, x, y)
         l0 = mc.launch_count()
         F, Gd = mm.nlml_grad(hp)
         nl = mc.launch_count() - l0
-        launches[(forced, phases, kchunk, lauum)] = nl
+        launches[(forced, phases, kchunk)] = nl
         mm.close(); mc.close()
         relF, relG = abs(F - float(g["F_A"])) / abs(float(g["F_A"])), grad_err(Gd, g["G_A"])
-        print(f"\nmgpu INT8 routes, G={G}, ozaki={forced} phases={phases} kchunk={kchunk} lauum={lauum}: relF {relF:.2e} relG {relG:.2e} ({nl} launches)")
+        print(f"\nmgpu INT8 routes, G={G}, ozaki={forced} phases={phases} kchunk={kchunk}: relF {relF:.2e} relG {relG:.2e} ({nl} launches)")
         assert relF <= TOL_F and relG <= TOL_G
-    assert len(set(launches.values())) == 5          # five different routes were actually taken
+    assert launches[(-1, 11, 32768)] == launches[(8, 11, 32768)]          # automatic = 8 digits: the same route
+    distinct = [launches[k] for k in ((8, 11, 2048), (8, 11, 32768), (8, 1, 32768), (0, 11, 32768))]
+    assert len(set(distinct)) == 4          # four different routes were actually taken
 
 
 # ------------------------------------------------------------------ (6) SURVEY.md 8f "next" rows on the device

@@ -1,6 +1,6 @@
-"""[Historical A/B script: it produced profiles/ozaki_lauum9_r2s.log when the nine-digit product ran as three windows and launch flag 1024 /
-option ozaki_windows = 2 selected 128 x 256 tiles for the tenth diagonal; the default is now two windows, see csrc/ozaki_i8.cuh.]
-The W^T W product of the inverse (lauum) on the INT8 tensor cores with NINE 7-bit digits (three diagonal windows):
+"""[profiles/ozaki_lauum9_r2s.log is the record of this script when the nine-digit product ran as three diagonal windows, with a
+128 x 256-tile variant for the tenth diagonal; both are retired, the product now runs as two windows, see csrc/ozaki_i8.cuh.]
+The W^T W product of the inverse (lauum) on the INT8 tensor cores with NINE 7-bit digits:
 accuracy of NLML + gradient vs the committed N = 32768 oracle golden and stage times.   python tools/ozaki_lauum9.py"""
 import os
 import sys
@@ -26,37 +26,23 @@ for n in (2048,):
             print(f"raw A^T A ({name}) n={n} S={S}: max err / max|C| {np.abs(Cm - ref).max() / np.abs(ref).max():.2e}  ({ms:.3f} ms)", flush=True)
 n = 8192
 A = rng.standard_normal((n, n))
-ref = None
-for S, fl in ((8, 0), (9, 0), (9, 1024), (9, 1024 | 3)):
+for S, fl in ((8, 0), (9, 0), (9, 3)):
     Cm, ms = _ffi.dbg_ozaki_dgemm(ctx, 1.0, A, A, 0.0, np.zeros((n, n)), S=S, flags=fl, reps=5)
-    if fl == 0 and S == 9:
-        ref = Cm
-    extra = ""
-    if fl == 1024:
-        extra = f", 128x256 tenth-diagonal tiles vs 128x128: max|diff| {np.abs(Cm - ref).max():.2e}"
-    print(f"timing 8192^3 S={S} flags={fl}: {ms:.3f} ms -> {2 * n ** 3 / ms / 1e9:.1f} TFLOP/s FP64-equivalent (full product count){extra}", flush=True)
-for nn in (2048 + 128,):      # odd multiple of 128: the last 256-wide tile is half outside
-    B = rng.standard_normal((1024, nn))
-    r0, _ = _ffi.dbg_ozaki_dgemm(ctx, 1.0, B, B, 0.0, np.zeros((nn, nn)), S=9, flags=0)
-    r1, _ = _ffi.dbg_ozaki_dgemm(ctx, 1.0, B, B, 0.0, np.zeros((nn, nn)), S=9, flags=1024)
-    r2, _ = _ffi.dbg_ozaki_dgemm(ctx, 1.0, B, B, 0.0, np.full((nn, nn), 7.0), S=9, flags=1024 | 1)
-    print(f"n={nn}: 256-wide vs 128-wide max|diff| {np.abs(r1 - r0).max():.2e}; upper-only: upper diff {np.abs(np.triu(r2) - np.triu(r0)).max():.2e}, "
-          f"strict lower untouched {bool(np.all(np.tril(r2, -1) == np.tril(np.full((nn, nn), 7.0), -1)))}", flush=True)
+    print(f"timing 8192^3 S={S} flags={fl}: {ms:.3f} ms -> {2 * n ** 3 / ms / 1e9:.1f} TFLOP/s FP64-equivalent (full product count)", flush=True)
 g = np.load(os.path.join(ROOT, "tests", "golden", "config3_n32768.npz"))
 x, y, hp = m3.inputs()
 mh = _ffi.ModelHandle(ctx, [1, 1, 2], 8, x, y)
-for lau, pan, win in ((0, 32768, 0), (9, 32768, 0), (9, 32768, 2), (9, 8192, 2)):
+for lau, pan in ((0, 32768), (9, 32768), (9, 8192)):
     ctx.set_option("ozaki", -1)
     ctx.set_option("ozaki_lauum", lau)
     ctx.set_option("ozaki_panel", pan)
-    ctx.set_option("ozaki_windows", win)
     mh.nlml_grad(hp * 1.001)
     F, G = mh.nlml_grad(hp)
     t = mh.timings()
     relF = abs(F - float(g["F"])) / abs(float(g["F"]))
     relG = float((np.abs(G - g["G"]) / np.maximum(np.abs(g["G"]), 1e-8 * np.linalg.norm(g["G"]))).max())
-    print(f"ozaki_lauum={lau} panel={pan} windows={win}: eval {t['eval']:.1f} ms (potrf {t['potrf']:.1f}, trtri {t['trtri']:.1f}, lauum {t['lauum']:.1f}); "
+    print(f"ozaki_lauum={lau} panel={pan}: eval {t['eval']:.1f} ms (potrf {t['potrf']:.1f}, trtri {t['trtri']:.1f}, lauum {t['lauum']:.1f}); "
           f"vs oracle: relF {relF:.2e} relG {relG:.2e}", flush=True)
-ctx.set_option("ozaki_windows", 0)
 ctx.set_option("ozaki_lauum", 9)
+ctx.set_option("ozaki_panel", 32768)
 mh.close()
