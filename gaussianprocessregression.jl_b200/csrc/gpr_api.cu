@@ -73,6 +73,8 @@ struct gpr_ctx {
   int64_t ozaki_win_mink = 8192;   // option "ozaki_win_mink": two-diagonal-window form (128 x 128 tiles) of the 8-digit product for products with M, N,
                                    // K >= this (0 = never): the windows pay for their second pass over the digit planes only on the largest products --
                                    // N = 32768 evaluation 680 -> 667 ms at 8192, 670 at 4096, 680 at 2048 (profiles/ozaki_win_mink_r2an.log)
+  int ozaki_pair = 1;           // option "ozaki_pair": the plain INT8 products run as CTA pairs (tcgen05 cta_group::2, launch flag 2048): each SM
+                                // reads half of the op(B) tile from shared memory per MMA; bit-identical to the single-CTA kernels
   int ozaki_split = 9;          // option "ozaki_split": digits of the INT8 route for the split-predict mean products (0 = DMMA, 8, 9)
   int64_t ozaki_kchunk = 32768; // option "ozaki_kchunk": k-chunk of the long-K tile-mapped products (tests lower it to exercise the chunk loop)
   int64_t ozaki_panel = 32768;  // option "ozaki_panel": k-panel of the W^T W product (own digit scales per panel)
@@ -157,10 +159,11 @@ struct CudaBE {
         if ((flags & ~(BLK_UPPER_ONLY | BLK_K_FROM_N | BLK_SKIP_TILE00)) || batch < 1 || batch > 16 || K > 32768) return r;
         if (kind == OZ_HADAMARD) { r.digits = ctx->ozaki_split; return r; }
         r.digits = digits;
+        if (ctx->ozaki_pair) r.flags |= 2048;
         if (batch == 1 && flags == (BLK_UPPER_ONLY | BLK_K_FROM_N) && A == B && lda == ldb && M == N && N == K && K > ctx->ozaki_panel)
           r.ksplit = ctx->ozaki_panel;
         else if (ctx->ozaki_win_mink > 0 && std::min(K, std::min(M, N)) >= ctx->ozaki_win_mink)
-          r.flags = 512;
+          r.flags |= 512;
         return r;
       case OZ_MAP_UPPER:
         if (flags == BLK_MAP_UPPER && K <= 32768) r.digits = digits;
@@ -804,6 +807,7 @@ int gpr_ctx_set_option(gpr_ctx* ctx, const char* name, int64_t value) {
     if (value != 0 && value != 8 && value != 9) return fail(ctx, GPR_ERR_ARG, "ozaki_lauum: 0 (DMMA), 8 or 9 digits");
     ctx->ozaki_lauum = (int)value; return GPR_OK;
   }
+  if (!strcmp(name, "ozaki_pair")) { ctx->ozaki_pair = value ? 1 : 0; return GPR_OK; }
   if (!strcmp(name, "ozaki_win_mink")) { ctx->ozaki_win_mink = std::max<int64_t>(0, value); return GPR_OK; }
   if (!strcmp(name, "ozaki_split")) {
     if (value != 0 && value != 8 && value != 9) return fail(ctx, GPR_ERR_ARG, "ozaki_split: 0 (DMMA), 8 or 9 digits");

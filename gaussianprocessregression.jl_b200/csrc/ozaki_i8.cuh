@@ -53,8 +53,9 @@ constexpr int OZ_SMAX = 8;
 constexpr int OZ_THREADS = 192;
 constexpr int OZ_STAGES = 2;
 
-__host__ __device__ inline size_t oz_stage_bytes(int S) { return (size_t)S * (OZ_BM + OZ_BN) * OZ_BK; }
-__host__ __device__ inline size_t oz_smem_bytes(int S) { return OZ_STAGES * oz_stage_bytes(S) + 1024 + 128; }
+// pair: a CTA of a cta_group::2 pair holds half of the op(B) tile
+__host__ __device__ inline size_t oz_stage_bytes(int S, bool pair = false) { return (size_t)S * (OZ_BM + (pair ? OZ_BN / 2 : OZ_BN)) * OZ_BK; }
+__host__ __device__ inline size_t oz_smem_bytes(int S, bool pair = false) { return OZ_STAGES * oz_stage_bytes(S, pair) + 1024 + 128; }
 
 // ---------------------------------------------------------------------------------------------------------------
 // digit planes: X is K x R column major (column r = the vector over k of row / column r of the product operand).
@@ -149,6 +150,66 @@ __device__ __forceinline__ void tc_mma_i8(unsigned tmem_d, uint64_t desc_a, uint
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate), "r"(0u), "r"(0u), "r"(0u), "r"(0u)
       : "memory");
 }
+// ---- CTA pairs (tcgen05 cta_group::2): one MMA of M = 256 reads 128 rows of op(A) and half of op(B) from each CTA's shared memory
+// at the same offset and accumulates into both CTAs' TMEM (128 lanes each) ----
+__device__ __forceinline__ unsigned oz_cluster_ctarank() {
+  unsigned r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;\n" : "=r"(r));
+  return r;
+}
+// every thread of both CTAs (release / acquire at cluster scope)
+__device__ __forceinline__ void oz_cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\n" ::: "memory");
+  asm volatile("barrier.cluster.wait.acquire.aligned;\n" ::: "memory");
+}
+// shared::cluster address of the object at the same offset in CTA `rank` of the cluster
+__device__ __forceinline__ unsigned oz_mapa(const void* p, unsigned rank) {
+  unsigned r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;\n" : "=r"(r) : "r"((unsigned)__cvta_generic_to_shared(p)), "r"(rank));
+  return r;
+}
+// TMA load into this CTA's shared memory whose bytes complete on the mbarrier at cluster address `bar` (the leader's)
+__device__ __forceinline__ void tma_load_3d_pair(void* smem_dst, const CUtensorMap* map, unsigned bar, int c0, int c1, int c2) {
+  asm volatile("cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];\n" ::"r"(
+                   (unsigned)__cvta_generic_to_shared(smem_dst)),
+               "l"((uint64_t)map), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
+               : "memory");
+}
+// completion of the pair's MMAs issued so far arrives on the mbarrier at this offset in both CTAs
+__device__ __forceinline__ void tc_commit_pair(uint64_t* bar) {
+  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;\n" ::"r"(
+                   (unsigned)__cvta_generic_to_shared(bar)),
+               "h"((unsigned short)0x3)
+               : "memory");
+}
+__device__ __forceinline__ void tc_mma_i8_pair(unsigned tmem_d, uint64_t desc_a, uint64_t desc_b, unsigned idesc, unsigned accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(tmem_d),
+      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// TMEM: all 512 columns; with cta_group::2 one warp of EACH CTA of the pair takes part
+template <bool PAIR> __device__ __forceinline__ void oz_tmem_alloc(unsigned* slot) {
+  if constexpr (PAIR) {
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], 512;\n" ::"r"((unsigned)__cvta_generic_to_shared(slot)) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;\n" ::: "memory");
+  } else {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;\n" ::"r"((unsigned)__cvta_generic_to_shared(slot)) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
+  }
+}
+template <bool PAIR> __device__ __forceinline__ void oz_tmem_dealloc(unsigned base) {
+  if constexpr (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, 512;\n" ::"r"(base) : "memory");
+  else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;\n" ::"r"(base) : "memory");
+}
+// A pair works on row tiles 2j (leader, cluster rank 0) and 2j + 1 of one column tile.  It leaves only when both tiles are skipped;
+// otherwise a CTA whose own tile is skipped (below the diagonal of an upper-only product, tile (0,0) of a skip-tile product, the row
+// tile past M of an odd row-tile count: TMA zero fill) runs as a ghost: same loads, its half of the MMAs, no stores.
+
 // K-major operand tile with 64-byte rows, SWIZZLE_64B: 8-row groups are 512 bytes apart
 __device__ __forceinline__ uint64_t oz_smem_desc(const void* p) {
   const unsigned a = (unsigned)__cvta_generic_to_shared(p);
@@ -162,6 +223,7 @@ __device__ __forceinline__ uint64_t oz_smem_desc(const void* p) {
 }
 // instruction descriptor: D = S32, A = B = signed int8, both K-major, N = 64, M = 128
 constexpr unsigned OZ_IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(OZ_BN >> 3) << 17) | ((unsigned)(OZ_BM >> 4) << 24);
+constexpr unsigned OZ_IDESC_PAIR = (2u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(OZ_BN >> 3) << 17) | ((unsigned)((2 * OZ_BM) >> 4) << 24);   // M = 256
 
 struct OzParams {
   int M, N, K, S;
@@ -175,12 +237,14 @@ struct OzParams {
   const double* E; long long lde;                // Hadamard epilogue: C = alpha (A^T B) .* E + beta C  (split-predict mean)
 };
 
-template <int S>
+// PAIR: clusters of two CTAs issuing tcgen05.mma.cta_group::2 of M = 256 (256 x 64 tile per pair; mapB's box holds 32 rows)
+template <int S, bool PAIR = false>
 __global__ void __launch_bounds__(OZ_THREADS, 1)
 oz_gemm_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB) {
+  constexpr int BNC = PAIR ? OZ_BN / 2 : OZ_BN;      // op(B) rows in this CTA's shared memory
   extern __shared__ unsigned char oz_smem_raw[];
   unsigned char* smem = reinterpret_cast<unsigned char*>(((uintptr_t)oz_smem_raw + 1023) & ~(uintptr_t)1023);
-  const size_t stage_bytes = oz_stage_bytes(S);
+  const size_t stage_bytes = oz_stage_bytes(S, PAIR);
   uint64_t* full = reinterpret_cast<uint64_t*>(smem + OZ_STAGES * stage_bytes);
   uint64_t* empty = full + OZ_STAGES;
   uint64_t* tfull = empty + OZ_STAGES;
@@ -190,11 +254,13 @@ oz_gemm_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const
   // CTA rasterisation as in dgemm128_kernel: consecutive CTAs walk 16 row tiles x all column tiles, so one wave of 148 CTAs
   // touches ~16 x 9 tiles of C and re-reads few digit planes (issued x-fastest, a wave would stream every plane of op(A)
   // from DRAM once per column tile: 467 GB for a 16384^3 product against 4.3 GB of planes).
+  // (a pair is one unit of the rasterisation: x counts pairs of row tiles, 8 pairs = 16 row tiles per group)
+  constexpr int NC = PAIR ? 2 : 1;
   int tile_m, tile_n;
   {
-    constexpr int GM = 16;
-    const int Mx = gridDim.x, Ny = gridDim.y;
-    const int pid = blockIdx.x + blockIdx.y * Mx;
+    constexpr int GM = 16 / NC;
+    const int Mx = gridDim.x / NC, Ny = gridDim.y;
+    const int pid = blockIdx.x / NC + blockIdx.y * Mx;
     const int group = pid / (GM * Ny), first_m = group * GM;
     const int gsize = min(Mx - first_m, GM);
     const int rem = pid - group * GM * Ny;
@@ -202,8 +268,20 @@ oz_gemm_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const
     tile_n = rem / gsize;
   }
   const int blk_n = (tile_n * OZ_BN) >> 7;
-  if ((p.flags & 1) && tile_m > blk_n) return;                       // GEMM_UPPER_ONLY: whole CTA leaves before any allocation
-  if ((p.flags & 64) && tile_m == 0 && blk_n == 0) return;           // GEMM_SKIP_TILE00
+  [[maybe_unused]] unsigned crank = 0;
+  [[maybe_unused]] bool ghost = false;
+  if constexpr (!PAIR) {
+    if ((p.flags & 1) && tile_m > blk_n) return;                       // GEMM_UPPER_ONLY: whole CTA leaves before any allocation
+    if ((p.flags & 64) && tile_m == 0 && blk_n == 0) return;           // GEMM_SKIP_TILE00
+  } else {
+    crank = oz_cluster_ctarank();
+    const int m_lead = 2 * tile_m;
+    tile_m = m_lead + (int)crank;
+    const bool skip_lead = ((p.flags & 1) && m_lead > blk_n) || ((p.flags & 64) && m_lead == 0 && blk_n == 0);
+    const bool skip_peer = ((p.flags & 1) && m_lead + 1 > blk_n) || (m_lead + 1) * OZ_BM >= p.M;
+    if (skip_lead && skip_peer) return;
+    ghost = crank ? skip_peer : skip_lead;
+  }
   int gt = 0;
   if (p.flags & 8) {                                                  // GEMM_MAP_UPPER: tile-mapped trailing update of the block-cyclic potrf
     gt = p.col_gtile[blk_n];
@@ -222,12 +300,10 @@ oz_gemm_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const
     mbar_init(tfull, 1);
     mbar_fence_init();
   }
-  if (warp == 1) {   // TMEM: all 512 columns (8 diagonals x 64)
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;\n" ::"r"((unsigned)__cvta_generic_to_shared(tmem_slot)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
-  }
+  if (warp == 1) oz_tmem_alloc<PAIR>(tmem_slot);   // TMEM: all 512 columns (8 diagonals x 64)
   tc_fence_before();
   __syncthreads();
+  if constexpr (PAIR) oz_cluster_sync();         // the peer's barriers exist before anything signals them
   tc_fence_after();
   const unsigned tmem_base = *tmem_slot;
 
@@ -238,10 +314,19 @@ oz_gemm_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const
         const int s = kt & 1;
         if (kt >= OZ_STAGES) oz_wait(&empty[s], (unsigned)(((kt >> 1) - 1) & 1));
         unsigned char* st = smem + (size_t)s * stage_bytes;
-        if ((p.flags & 256) && kt >= OZ_STAGES) { mbar_arrive(&full[s]); continue; }   // timing probe: no reload (results are garbage)
-        mbar_expect_tx(&full[s], (unsigned)stage_bytes);
-        tma_load_3d(st, &mapA, &full[s], (kt0 + kt) * OZ_BK, m0, 0);                               // S x 128 x 64 B
-        tma_load_3d(st + (size_t)S * OZ_BM * OZ_BK, &mapB, &full[s], (kt0 + kt) * OZ_BK, n0, 0);   // S x  64 x 64 B
+        if constexpr (!PAIR) {
+          if ((p.flags & 256) && kt >= OZ_STAGES) { mbar_arrive(&full[s]); continue; }   // timing probe: no reload (results are garbage)
+          mbar_expect_tx(&full[s], (unsigned)stage_bytes);
+          tma_load_3d(st, &mapA, &full[s], (kt0 + kt) * OZ_BK, m0, 0);                               // S x 128 x 64 B
+          tma_load_3d(st + (size_t)S * OZ_BM * OZ_BK, &mapB, &full[s], (kt0 + kt) * OZ_BK, n0, 0);   // S x  64 x 64 B
+        } else {
+          // both CTAs' bytes complete on the leader's full[s]; the leader's MMA thread is the only one waiting on it
+          if ((p.flags & 256) && kt >= OZ_STAGES) { if (crank == 0) mbar_arrive(&full[s]); continue; }
+          if (crank == 0) mbar_expect_tx(&full[s], (unsigned)(2 * stage_bytes));
+          const unsigned bar = oz_mapa(&full[s], 0);
+          tma_load_3d_pair(st, &mapA, bar, (kt0 + kt) * OZ_BK, m0, 0);                                            // S x 128 x 64 B
+          tma_load_3d_pair(st + (size_t)S * OZ_BM * OZ_BK, &mapB, bar, (kt0 + kt) * OZ_BK, n0 + (int)crank * BNC, 0);   // S x 32 x 64 B
+        }
       }
     }
   } else if (warp == 1) {
@@ -266,6 +351,7 @@ oz_gemm_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const
         baseA[s] = oz_smem_desc(smem + (size_t)s * stage_bytes);
         baseB[s] = oz_smem_desc(smem + (size_t)s * stage_bytes + (size_t)S * OZ_BM * OZ_BK);
       }
+      if (PAIR && crank != 0) KT = 0;        // the leader issues the pair's MMAs
       for (int kt = 0; kt < KT; ++kt) {
         const int s = kt & 1;
         oz_wait(&full[s], (unsigned)((kt >> 1) & 1));
@@ -280,16 +366,18 @@ oz_gemm_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const
 #pragma unroll
               for (int kk = 0; kk < OZ_BK / 32; ++kk) {   // 32-byte k-steps inside the 64-byte swizzle atom: +2 in the 16-byte address field
                 const uint64_t da = dA + (uint64_t)(((sa - 1) * OZ_BM * OZ_BK + 32 * kk) >> 4);
-                const uint64_t db = dB + (uint64_t)(((t - 1) * OZ_BN * OZ_BK + 32 * kk) >> 4);
-                tc_mma_i8(tmem_base + (unsigned)((sa + t - 2) * OZ_BN), da, db, OZ_IDESC, (kk > 0 || t > 1) ? 1u : acc_first);
+                const uint64_t db = dB + (uint64_t)(((t - 1) * BNC * OZ_BK + 32 * kk) >> 4);
+                if constexpr (PAIR) tc_mma_i8_pair(tmem_base + (unsigned)((sa + t - 2) * OZ_BN), da, db, OZ_IDESC_PAIR, (kk > 0 || t > 1) ? 1u : acc_first);
+                else tc_mma_i8(tmem_base + (unsigned)((sa + t - 2) * OZ_BN), da, db, OZ_IDESC, (kk > 0 || t > 1) ? 1u : acc_first);
               }
             }
           }
-          tc_commit(&empty[s]);              // the stage may be refilled once these MMAs have read it
+          if constexpr (PAIR) tc_commit_pair(&empty[s]); else tc_commit(&empty[s]);   // the stage may be refilled once these MMAs have read it
         }
         __syncwarp();
       }
-      if (elected) tc_commit(tfull);       // all accumulators complete
+      if constexpr (PAIR) { if (elected && crank == 0) tc_commit_pair(tfull); }
+      else if (elected) tc_commit(tfull);       // all accumulators complete
     }
   } else {
     // ===== epilogue: warps 2..5 own TMEM lanes 32 (warp % 4) .. +31 = rows of the tile =====
@@ -303,6 +391,7 @@ oz_gemm_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const
     const double sa = p.scaleA[m0 + row] * p.alpha;
     double* Crow = p.C + (long long)(m0 + row) + (long long)n0 * p.ldc;
     for (int c0 = 0; c0 < OZ_BN; c0 += 16) {
+      if constexpr (PAIR) { if (ghost) break; }
       double acc[16];
 #pragma unroll
       for (int j = 0; j < 16; ++j) acc[j] = 0.0;
@@ -331,9 +420,10 @@ oz_gemm_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const
     tc_fence_before();
   }
   __syncthreads();
+  if constexpr (PAIR) oz_cluster_sync();      // no CTA leaves (or frees TMEM) while its peer may still signal or use it
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;\n" ::"r"(tmem_base) : "memory");
+    oz_tmem_dealloc<PAIR>(tmem_base);
   }
 }
 
@@ -350,13 +440,16 @@ oz_gemm_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const
 // so the tensor pipe itself (~2.65 INT8 POPS in this access pattern), not the instruction shape, is the limit.  Launch flag 512:
 // the largest products take it (context option "ozaki_win_mink").
 // ---------------------------------------------------------------------------------------------------------------
-template <int S, int BN, int BK, int DLO, int DHI> struct OzWin {
+// PAIR: clusters of two CTAs issuing tcgen05.mma.cta_group::2 of M = 256; a CTA holds BN / 2 rows of op(B) per plane, so a stage is
+// smaller and more of them fit (three -> four for every window below).
+template <int S, int BN, int BK, int DLO, int DHI, bool PAIR = false> struct OzWin {
   static constexpr int NACC = DHI - DLO + 1;
   static constexpr int PL = (DHI - 1 < S) ? DHI - 1 : S;                  // digit planes needed
-  static constexpr size_t STAGE = (size_t)PL * (OZ_BM + BN) * BK;
+  static constexpr int BNC = PAIR ? BN / 2 : BN;                          // op(B) rows in this CTA's shared memory
+  static constexpr size_t STAGE = (size_t)PL * (OZ_BM + BNC) * BK;
   static constexpr int NST = (int)(231000 / STAGE) > 4 ? 4 : (int)(231000 / STAGE);      // 227 KB of shared memory per CTA
   static constexpr size_t SMEM = NST * STAGE + 1024 + 256;
-  static constexpr unsigned IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(BN >> 3) << 17) | ((unsigned)(OZ_BM >> 4) << 24);
+  static constexpr unsigned IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(BN >> 3) << 17) | ((unsigned)(((PAIR ? 2 : 1) * OZ_BM) >> 4) << 24);
   static_assert(NACC * BN <= 512, "accumulators exceed TMEM");
   static_assert(NST >= 2, "need two stages");
 };
@@ -372,11 +465,11 @@ template <int BK> __device__ __forceinline__ uint64_t oz_smem_desc_k(const void*
   return d;
 }
 
-template <int S, int BN, int BK, int DLO, int DHI>
+template <int S, int BN, int BK, int DLO, int DHI, bool PAIR = false>
 __global__ void __launch_bounds__(OZ_THREADS, 1)
 oz_gemm_win_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB) {
-  using W = OzWin<S, BN, BK, DLO, DHI>;
-  constexpr int NST = W::NST, PL = W::PL;
+  using W = OzWin<S, BN, BK, DLO, DHI, PAIR>;
+  constexpr int NST = W::NST, PL = W::PL, BNC = W::BNC;
   extern __shared__ unsigned char oz_smem_raw[];
   unsigned char* smem = reinterpret_cast<unsigned char*>(((uintptr_t)oz_smem_raw + 1023) & ~(uintptr_t)1023);
   uint64_t* full = reinterpret_cast<uint64_t*>(smem + NST * W::STAGE);
@@ -385,11 +478,12 @@ oz_gemm_win_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, c
   unsigned* tmem_slot = reinterpret_cast<unsigned*>(tfull + 1);
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  constexpr int NC = PAIR ? 2 : 1;
   int tile_m, tile_n;
   {
-    constexpr int GM = 8;      // 8 row tiles x all column tiles per pass (tiles are 128 x 128 here)
-    const int Mx = gridDim.x, Ny = gridDim.y;
-    const int pid = blockIdx.x + blockIdx.y * Mx;
+    constexpr int GM = 8 / NC;      // 8 row tiles x all column tiles per pass (tiles are 128 x 128 here); x counts pairs of row tiles
+    const int Mx = gridDim.x / NC, Ny = gridDim.y;
+    const int pid = blockIdx.x / NC + blockIdx.y * Mx;
     const int group = pid / (GM * Ny), first_m = group * GM;
     const int gsize = min(Mx - first_m, GM);
     const int rem = pid - group * GM * Ny;
@@ -398,10 +492,22 @@ oz_gemm_win_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, c
   }
   const int blk_n = (tile_n * BN) >> 7;                       // first 128-block of the tile's columns
   if (tile_n * BN >= p.N) return;
-  if ((p.flags & 1) && tile_m > ((tile_n * BN + BN - 1) >> 7)) return;
-  if ((p.flags & 64) && tile_m == 0 && blk_n == 0) return;
+  [[maybe_unused]] unsigned crank = 0;
+  [[maybe_unused]] bool ghost = false;
+  if constexpr (!PAIR) {
+    if ((p.flags & 1) && tile_m > ((tile_n * BN + BN - 1) >> 7)) return;
+    if ((p.flags & 64) && tile_m == 0 && blk_n == 0) return;
+  } else {
+    crank = oz_cluster_ctarank();
+    const int m_lead = 2 * tile_m, last_blk = (tile_n * BN + BN - 1) >> 7;
+    tile_m = m_lead + (int)crank;
+    const bool skip_lead = ((p.flags & 1) && m_lead > last_blk) || ((p.flags & 64) && m_lead == 0 && blk_n == 0);
+    const bool skip_peer = ((p.flags & 1) && m_lead + 1 > last_blk) || (m_lead + 1) * OZ_BM >= p.M;
+    if (skip_lead && skip_peer) return;
+    ghost = crank ? skip_peer : skip_lead;
+  }
   const int kt0 = (p.flags & 2) ? max(0, blk_n * 128 - p.k_off) / BK : 0;
-  const int KT = p.K / BK - kt0;
+  int KT = p.K / BK - kt0;
   const int m0 = tile_m * OZ_BM, n0 = tile_n * BN;
 
   if (tid == 0) {
@@ -409,12 +515,10 @@ oz_gemm_win_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, c
     mbar_init(tfull, 1);
     mbar_fence_init();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;\n" ::"r"((unsigned)__cvta_generic_to_shared(tmem_slot)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
-  }
+  if (warp == 1) oz_tmem_alloc<PAIR>(tmem_slot);
   tc_fence_before();
   __syncthreads();
+  if constexpr (PAIR) oz_cluster_sync();      // the peer's barriers exist before anything signals them
   tc_fence_after();
   const unsigned tmem_base = *tmem_slot;
 
@@ -424,9 +528,17 @@ oz_gemm_win_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, c
         const int s = kt % NST;
         if (kt >= NST) oz_wait(&empty[s], (unsigned)((kt / NST - 1) & 1));
         unsigned char* st = smem + (size_t)s * W::STAGE;
-        mbar_expect_tx(&full[s], (unsigned)W::STAGE);
-        tma_load_3d(st, &mapA, &full[s], (kt0 + kt) * BK, m0, 0);                               // PL x 128 x BK
-        tma_load_3d(st + (size_t)PL * OZ_BM * BK, &mapB, &full[s], (kt0 + kt) * BK, n0, 0);     // PL x BN  x BK
+        if constexpr (!PAIR) {
+          mbar_expect_tx(&full[s], (unsigned)W::STAGE);
+          tma_load_3d(st, &mapA, &full[s], (kt0 + kt) * BK, m0, 0);                               // PL x 128 x BK
+          tma_load_3d(st + (size_t)PL * OZ_BM * BK, &mapB, &full[s], (kt0 + kt) * BK, n0, 0);     // PL x BN  x BK
+        } else {
+          // both CTAs' bytes complete on the leader's full[s]
+          if (crank == 0) mbar_expect_tx(&full[s], (unsigned)(2 * W::STAGE));
+          const unsigned bar = oz_mapa(&full[s], 0);
+          tma_load_3d_pair(st, &mapA, bar, (kt0 + kt) * BK, m0, 0);                                            // PL x 128 x BK
+          tma_load_3d_pair(st + (size_t)PL * OZ_BM * BK, &mapB, bar, (kt0 + kt) * BK, n0 + (int)crank * BNC, 0);   // PL x BN / 2 x BK
+        }
       }
     }
   } else if (warp == 1) {
@@ -439,6 +551,7 @@ oz_gemm_win_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, c
         "}\n"
         : "=r"(elected));
     const uint64_t baseA0 = oz_smem_desc_k<BK>(smem), baseB0 = oz_smem_desc_k<BK>(smem + (size_t)PL * OZ_BM * BK);
+    if (PAIR && crank != 0) KT = 0;          // the leader issues the pair's MMAs
     for (int kt = 0; kt < KT; ++kt) {
       const int s = kt % NST;
       oz_wait(&full[s], (unsigned)((kt / NST) & 1));
@@ -456,16 +569,18 @@ oz_gemm_win_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, c
 #pragma unroll
             for (int kk = 0; kk < BK / 32; ++kk) {
               const uint64_t da = dA + (uint64_t)(((sa - 1) * OZ_BM * BK + 32 * kk) >> 4);
-              const uint64_t db = dB + (uint64_t)(((t - 1) * BN * BK + 32 * kk) >> 4);
-              tc_mma_i8(tmem_base + (unsigned)((sa + t - DLO) * BN), da, db, W::IDESC, (kk > 0 || !first_pair) ? 1u : acc_first);
+              const uint64_t db = dB + (uint64_t)(((t - 1) * BNC * BK + 32 * kk) >> 4);
+              if constexpr (PAIR) tc_mma_i8_pair(tmem_base + (unsigned)((sa + t - DLO) * BN), da, db, W::IDESC, (kk > 0 || !first_pair) ? 1u : acc_first);
+              else tc_mma_i8(tmem_base + (unsigned)((sa + t - DLO) * BN), da, db, W::IDESC, (kk > 0 || !first_pair) ? 1u : acc_first);
             }
           }
         }
-        tc_commit(&empty[s]);
+        if constexpr (PAIR) tc_commit_pair(&empty[s]); else tc_commit(&empty[s]);
       }
       __syncwarp();
     }
-    if (elected) tc_commit(tfull);
+    if constexpr (PAIR) { if (elected && crank == 0) tc_commit_pair(tfull); }
+    else if (elected) tc_commit(tfull);
   } else {
     oz_wait(tfull, 0);
     tc_fence_after();
@@ -477,6 +592,7 @@ oz_gemm_win_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, c
     double* Crow = p.C + (long long)(m0 + row) + (long long)n0 * p.ldc;
     for (int c0 = 0; c0 < BN; c0 += 16) {
       if (n0 + c0 >= p.N) break;
+      if constexpr (PAIR) { if (ghost) break; }
       double acc[16];
 #pragma unroll
       for (int j = 0; j < 16; ++j) acc[j] = 0.0;
@@ -506,9 +622,10 @@ oz_gemm_win_kernel(const OzParams p, const __grid_constant__ CUtensorMap mapA, c
     tc_fence_before();
   }
   __syncthreads();
+  if constexpr (PAIR) oz_cluster_sync();      // no CTA leaves (or frees TMEM) while its peer may still signal or use it
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;\n" ::"r"(tmem_base) : "memory");
+    oz_tmem_dealloc<PAIR>(tmem_base);
   }
 }
 
@@ -525,8 +642,8 @@ inline bool oz_make_map(CUtensorMap* map, const int8_t* base, uint64_t Kp, uint6
             CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <int S> inline cudaError_t oz_set_attr_s() {
-  return cudaFuncSetAttribute(oz_gemm_kernel<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)oz_smem_bytes(S));
+template <int S, bool PAIR = false> inline cudaError_t oz_set_attr_s() {
+  return cudaFuncSetAttribute(oz_gemm_kernel<S, PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)oz_smem_bytes(S, PAIR));
 }
 inline bool oz_make_map_k(CUtensorMap* map, const int8_t* base, uint64_t Kp, uint64_t Rp, int planes_total, int box_planes, uint32_t box_rows, int BK) {
   PFN_encodeTiled fn = tma_encode_fn();
@@ -542,6 +659,9 @@ inline bool oz_make_map_k(CUtensorMap* map, const int8_t* base, uint64_t Kp, uin
 using OzWinLo = OzWin<8, 128, 32, 6, 9>;
 using OzWinHi = OzWin<8, 128, 64, 2, 5>;      // (k-tiles of 32 with seven stages instead of 64 with three: measured slower, 20.1 vs 18.7 ms per 8192^3 nine-digit product)
 using OzWin9Z = OzWin<9, 96, 32, 6, 10>;      // nine digits in TWO windows: d = 6..10 in five 96-column accumulators (480 TMEM columns, 35 pairs)
+using OzWinLoP = OzWin<8, 128, 32, 6, 9, true>;
+using OzWinHiP = OzWin<8, 128, 64, 2, 5, true>;
+using OzWin9ZP = OzWin<9, 96, 32, 6, 10, true>;
 
 inline cudaError_t oz_set_attr() {
   cudaError_t e = cudaFuncSetAttribute(oz_gemm_win_kernel<8, 128, 32, 6, 9>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OzWinLo::SMEM);
@@ -551,7 +671,32 @@ inline cudaError_t oz_set_attr() {
   if (e == cudaSuccess) e = oz_set_attr_s<7>();
   if (e == cudaSuccess) e = oz_set_attr_s<6>();
   if (e == cudaSuccess) e = oz_set_attr_s<2>();
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(oz_gemm_win_kernel<8, 128, 32, 6, 9, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OzWinLoP::SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(oz_gemm_win_kernel<8, 128, 64, 2, 5, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OzWinHiP::SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(oz_gemm_win_kernel<9, 96, 32, 6, 10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)OzWin9ZP::SMEM);
+  if (e == cudaSuccess) e = oz_set_attr_s<8, true>();
+  if (e == cudaSuccess) e = oz_set_attr_s<7, true>();
+  if (e == cudaSuccess) e = oz_set_attr_s<6, true>();
   return e;
+}
+
+// launch as clusters of two CTAs along x (the cta_group::2 pairs): grid.x = row tiles rounded up to even
+template <typename Kern>
+inline cudaError_t oz_launch_pairs(Kern kern, int row_tiles, int col_tiles, size_t smem, cudaStream_t st, const OzParams& p, const CUtensorMap& a,
+                                   const CUtensorMap& b) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)(row_tiles + (row_tiles & 1)), (unsigned)col_tiles, 1);
+  cfg.blockDim = dim3(OZ_THREADS, 1, 1);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeClusterDimension;
+  at[0].val.clusterDim.x = 2;
+  at[0].val.clusterDim.y = 1;
+  at[0].val.clusterDim.z = 1;
+  cfg.attrs = at;
+  cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kern, p, a, b);
 }
 
 // workspace (bytes) for the digit planes and scales of one product
@@ -562,13 +707,15 @@ inline size_t oz_workspace_bytes(int M, int N, int K, int S) {
 
 // C = alpha A^T B + beta C through the int8 tensor cores.  M % 128 == 0, N % 128 == 0, K % 128 == 0, K <= 32768.
 // flags: GEMM_UPPER_ONLY (1), GEMM_K_FROM_N (2), GEMM_SKIP_TILE00 (64), 512 (above); the tile-mapped MAP_UPPER (8) and MAP_KUPTO (16)
-// and the timing probe (256) are forms of the single-pass kernel (S <= 8 without 512).  When A and B are the same matrix (the symmetric
+// and the timing probe (256) are forms of the single-pass kernel (S <= 8 without 512).  2048: CTA pairs (tcgen05 cta_group::2) for
+// S = 6..9 in every form but the tile-mapped and Hadamard ones, bit-identical to the single-CTA kernels (exact integer accumulation,
+// same epilogue).  When A and B are the same matrix (the symmetric
 // updates of potrf and the W^T W product of the inverse) its digit planes are formed once and shared.
 inline cudaError_t launch_ozaki_dgemm(cudaStream_t st, int M, int N, int K, int S, double alpha, const double* A, long long lda, const double* B,
                                       long long ldb, double beta, double* C, long long ldc, int flags, void* workspace, int k_off = 0,
                                       const int* col_gtile = nullptr, int row_gtile0 = 0, int k_gtile0 = 0, const double* E = nullptr,
                                       long long lde = 0) {
-  if (flags & ~(1 | 2 | 8 | 16 | 64 | 256 | 512)) return cudaErrorInvalidValue;
+  if (flags & ~(1 | 2 | 8 | 16 | 64 | 256 | 512 | 2048)) return cudaErrorInvalidValue;
   if (E && (flags & (8 | 16))) return cudaErrorInvalidValue;                         // Hadamard epilogue: plain forms only
   if ((flags & (8 | 16)) && (!col_gtile || S == 9 || (flags & 512))) return cudaErrorInvalidValue;   // tile-mapped: single-pass kernel only
   if ((flags & 16) && ((flags & (1 | 2 | 8 | 64)) || (A == B && lda == ldb))) return cudaErrorInvalidValue;   // KUPTO: plain form only
@@ -590,7 +737,10 @@ inline cudaError_t launch_ozaki_dgemm(cudaStream_t st, int M, int N, int K, int 
     if (flags & 16) oz_slice_kernel<<<(N + 7) / 8, 256, 0, st>>>(B, ldb, K, N, S, pb, (long long)Kp, N, sb, 2, k_off, col_gtile, k_gtile0);
     else oz_slice_kernel<<<(N + 7) / 8, 256, 0, st>>>(B, ldb, K, N, S, pb, (long long)Kp, N, sb, kfrom, k_off);
   }
-  const OzParams p{M, N, K, S, alpha, beta, C, ldc, sa, sb, flags & ~512, k_off, col_gtile, row_gtile0, k_gtile0, E, lde};
+  const OzParams p{M, N, K, S, alpha, beta, C, ldc, sa, sb, flags & ~(512 | 2048), k_off, col_gtile, row_gtile0, k_gtile0, E, lde};
+  // CTA pairs: each SM reads its own 128 rows of op(A) and half of the op(B) tile from shared memory per MMA
+  const bool pair = (flags & 2048) && !(flags & (8 | 16)) && !E && S != 2;
+  const int mt = M / OZ_BM;
   if (S == 9 || (S == 8 && (flags & 512))) {
     // Two windows of diagonals, lowest order first, the second accumulating into C.
     // NINE digits (products whose operands span several orders of magnitude under one scale per column: the W^T W of the inverse):
@@ -603,10 +753,19 @@ inline cudaError_t launch_ozaki_dgemm(cudaStream_t st, int M, int N, int K, int 
     // A operand from shared memory), the windows load the planes twice and sit at 81 % of the L2 -> SM fill rate instead.
     const bool nine = (S == 9);
     const int plLo = nine ? OzWin9Z::PL : OzWinLo::PL, bnLo = nine ? 96 : 128;
+    const int bdiv = pair ? 2 : 1;       // a CTA of a pair loads half of the op(B) tile
     CUtensorMap aLo, bLo, aHi, bHi;
-    if (!oz_make_map_k(&aLo, pa, Kp, (uint64_t)Ra, S, plLo, OZ_BM, 32) || !oz_make_map_k(&bLo, pb, Kp, (uint64_t)Rb, S, plLo, bnLo, 32) ||
-        !oz_make_map_k(&aHi, pa, Kp, (uint64_t)Ra, S, OzWinHi::PL, OZ_BM, 64) || !oz_make_map_k(&bHi, pb, Kp, (uint64_t)Rb, S, OzWinHi::PL, 128, 64))
+    if (!oz_make_map_k(&aLo, pa, Kp, (uint64_t)Ra, S, plLo, OZ_BM, 32) || !oz_make_map_k(&bLo, pb, Kp, (uint64_t)Rb, S, plLo, bnLo / bdiv, 32) ||
+        !oz_make_map_k(&aHi, pa, Kp, (uint64_t)Ra, S, OzWinHi::PL, OZ_BM, 64) || !oz_make_map_k(&bHi, pb, Kp, (uint64_t)Rb, S, OzWinHi::PL, 128 / bdiv, 64))
       return cudaErrorInvalidValue;
+    if (pair) {
+      OzParams p2 = p;
+      p2.beta = 1.0;
+      cudaError_t e = nine ? oz_launch_pairs(oz_gemm_win_kernel<9, 96, 32, 6, 10, true>, mt, (N + 95) / 96, OzWin9ZP::SMEM, st, p, aLo, bLo)
+                           : oz_launch_pairs(oz_gemm_win_kernel<8, 128, 32, 6, 9, true>, mt, N / 128, OzWinLoP::SMEM, st, p, aLo, bLo);
+      if (e == cudaSuccess) e = oz_launch_pairs(oz_gemm_win_kernel<8, 128, 64, 2, 5, true>, mt, N / 128, OzWinHiP::SMEM, st, p2, aHi, bHi);
+      return e != cudaSuccess ? e : cudaGetLastError();
+    }
     if (nine) oz_gemm_win_kernel<9, 96, 32, 6, 10><<<dim3(M / OZ_BM, (N + 95) / 96), OZ_THREADS, OzWin9Z::SMEM, st>>>(p, aLo, bLo);
     else oz_gemm_win_kernel<8, 128, 32, 6, 9><<<dim3(M / OZ_BM, N / 128), OZ_THREADS, OzWinLo::SMEM, st>>>(p, aLo, bLo);
     OzParams p2 = p;
@@ -615,7 +774,13 @@ inline cudaError_t launch_ozaki_dgemm(cudaStream_t st, int M, int N, int K, int 
     return cudaGetLastError();
   }
   CUtensorMap mA, mB;
-  if (!oz_make_map(&mA, pa, Kp, (uint64_t)Ra, S, OZ_BM) || !oz_make_map(&mB, pb, Kp, (uint64_t)Rb, S, OZ_BN)) return cudaErrorInvalidValue;
+  if (!oz_make_map(&mA, pa, Kp, (uint64_t)Ra, S, OZ_BM) || !oz_make_map(&mB, pb, Kp, (uint64_t)Rb, S, pair ? OZ_BN / 2 : OZ_BN)) return cudaErrorInvalidValue;
+  if (pair) {
+    cudaError_t e = (S == 8)   ? oz_launch_pairs(oz_gemm_kernel<8, true>, mt, N / OZ_BN, oz_smem_bytes(8, true), st, p, mA, mB)
+                    : (S == 7) ? oz_launch_pairs(oz_gemm_kernel<7, true>, mt, N / OZ_BN, oz_smem_bytes(7, true), st, p, mA, mB)
+                               : oz_launch_pairs(oz_gemm_kernel<6, true>, mt, N / OZ_BN, oz_smem_bytes(6, true), st, p, mA, mB);
+    return e != cudaSuccess ? e : cudaGetLastError();
+  }
   dim3 grid(M / OZ_BM, N / OZ_BN);
   if (S == 8) oz_gemm_kernel<8><<<grid, OZ_THREADS, oz_smem_bytes(8), st>>>(p, mA, mB);
   else if (S == 7) oz_gemm_kernel<7><<<grid, OZ_THREADS, oz_smem_bytes(7), st>>>(p, mA, mB);

@@ -99,7 +99,8 @@ const char* gpr_last_error(gpr_ctx* ctx);          /* ctx may be NULL: last erro
  *   "ozaki_lauum" digits of the inverse's W^T W product on that route: 9 [default], 8, 0 = DMMA; "ozaki_split" the same for the
  *   split-predict mean products; "ozaki_min" smallest routed M, N, K [1024];
  *   "ozaki_phases" bit mask potrf 1 | trtri 2 | other solves 8 [11]; "ozaki_panel", "ozaki_kchunk" k-panels [32768];
- *   "ozaki_win_mink" smallest M, N, K for the two-window form of the 8-digit product [8192]. */
+ *   "ozaki_win_mink" smallest M, N, K for the two-window form of the 8-digit product [8192];
+ *   "ozaki_pair" 1 = the INT8 product kernels run as CTA pairs (tcgen05 cta_group::2), 0 = single CTAs [1]; same bits either way. */
 int gpr_ctx_set_option(gpr_ctx* ctx, const char* name, int64_t value);
 int64_t gpr_ctx_launch_count(gpr_ctx* ctx);        /* kernels launched by this context so far */
 
@@ -190,8 +191,9 @@ int gpr_dbg_dgemm(gpr_ctx* ctx, char transA, char transB, int M, int N, int K, d
  * tensor cores (tcgen05.mma kind::i8 with TMEM accumulators): Ozaki-type splitting of every row of A^T and column of B
  * into S signed 7-bit digits, S (S + 1) / 2 exact integer products, FP64 recombination (csrc/ozaki_i8.cuh).
  * M % 128 == 0, N % 128 == 0, K % 128 == 0, K <= 32768, S in {2, 6, 7, 8, 9} (9: two diagonal windows, 45 products).
- * flags: 1 = upper only, 2 = K-from-N, 64 = skip tile (0,0) (not with S = 9), 512 = two-window form of the 8-digit product
- * (csrc/ozaki_i8.cuh); any other flag returns an error. */
+ * flags: 1 = upper only, 2 = K-from-N, 64 = skip tile (0,0) (not with S = 9), 512 = two-window form of the 8-digit product,
+ * 2048 = CTA pairs (tcgen05 cta_group::2; S = 6..9, bit-identical to the single-CTA kernels) (csrc/ozaki_i8.cuh); any other flag
+ * returns an error. */
 int gpr_dbg_ozaki_dgemm(gpr_ctx* ctx, int M, int N, int K, int S, double alpha, const double* A, int64_t lda, const double* B,
                         int64_t ldb, double beta, double* C, int64_t ldc, int flags, int reps, double* ms);
 /* factor (and optionally invert) a host SPD matrix in place through the blocked path; A is N x N.
