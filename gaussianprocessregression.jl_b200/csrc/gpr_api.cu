@@ -1192,6 +1192,55 @@ int predict_tile(gpr_model* m, const double* d_xp, int64_t mt, int64_t m0, int s
   return check_pending(ctx, "predict_tile");
 }
 
+// One tile of boxes resident on the device: d_a, d_b are D x mt (mt boxes).  k1 of every box is a column of the transposed
+// tile, as Kt in predict_tile, but there is no covariance build to fuse the mean into.  Writes Iout = k1^T wt to the host
+// (mt x ny, column stride ldI) and, when h_sq is given, h_sq[i] = -|U^-T k1_i|^2 (mt entries, host).
+int integrate_tile(gpr_model* m, const double* d_a, const double* d_b, int64_t mt, double* Iout, int64_t ldI, double* h_sq) {
+  gpr_ctx* ctx = m->ctx;
+  const int64_t Np = m->Np;
+  const int64_t mtp = round_up(mt, 128);
+  ctx->oz_active = m->oz;
+  int rc = ensure(ctx, m->w_kxp, (size_t)mtp * Np);
+  if (!rc) rc = ensure(ctx, m->w_part, (size_t)mtp * m->nyp);
+  if (!rc && h_sq) rc = ensure(ctx, m->w_var, (size_t)mtp);
+  if (rc) return rc;
+  double* k1 = m->w_kxp.p;
+  double* d_I = m->w_part.p;     // mtp x ny
+  CudaBE be{ctx};
+  {
+    Scope s(m->tm, GPR_T_PRED_KSTAR, ctx->stream);
+    rc = launch_antideriv(ctx, m->d_x, m->D, m->N, Np, m->d_hp, d_a, d_b, mt, mtp, k1, Np);   // antideriv!  (:15-31)
+    if (rc) return rc;
+  }
+  {
+    Scope s(m->tm, GPR_T_PRED_MEAN, ctx->stream);
+    if (m->ny == 1) {
+      CK(cudaMemsetAsync(d_I, 0, sizeof(double) * mt, ctx->stream));
+      be.gemv('T', mt, Np, 1.0, k1, Np, m->d_wt, d_I);                                          // Iout = k1' wt  (:118-121)
+    } else {
+      be.gemm('T', 'N', mtp, m->nyp, Np, 1.0, k1, Np, m->d_wt, Np, 0.0, d_I, mtp, 0);
+    }
+    CK(cudaMemcpy2DAsync(Iout, sizeof(double) * ldI, d_I, sizeof(double) * mtp, sizeof(double) * mt, m->ny,
+                         cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  if (h_sq) {
+    Blocked<CudaBE> blk(be, m->d_dinv);
+    {
+      Scope s(m->tm, GPR_T_PRED_TRSM, ctx->stream);
+      blk.trsm_LUT(m->d_U, Np, Np, 0, k1, Np, mtp, 1.0);          // ldiv!(kchol.L, tt), L = U^T, every box at once  (:133-134)
+    }
+    {
+      Scope s(m->tm, GPR_T_PRED_ROWNORM, ctx->stream);
+      colsumsq_kernel<<<(unsigned)mt, 256, 0, ctx->stream>>>(k1, Np, Np, mt, 0.0, m->w_var.p);
+      ctx->launches++;
+      CK(cudaGetLastError());
+    }
+    CK(cudaMemcpyAsync(h_sq, m->w_var.p, sizeof(double) * mt, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  CK(cudaStreamSynchronize(ctx->stream));
+  return check_pending(ctx, "integrate_tile");
+}
+
 }  // namespace
 
 extern "C" {
@@ -1549,6 +1598,34 @@ int gpr_integrate(gpr_model* m, const double* a, const double* b, double* Iout, 
   if (rc) return rc;
   for (int e = 0; e < m->ny; ++e) Iout[e] = hI[e];
   if (var_out) var_out[0] = antideriv2_se(m->hp_host.data(), a, b, D) - hsq;
+  return GPR_OK;
+}
+
+// nbox boxes in tiles of predict_tile: one triangular solve with all of a tile's k1 columns instead of one trsv per box
+int gpr_integrate_batch(gpr_model* m, int64_t nbox, const double* a, const double* b, double* Iout, double* var_out) {
+  if (!m) return GPR_ERR_ARG;
+  gpr_ctx* ctx = m->ctx;
+  if (!a || !b || !Iout || nbox < 1) return fail(ctx, GPR_ERR_ARG, "NULL or empty argument");
+  if (!m->have_factor || m->factor_destroyed) return fail(ctx, GPR_ERR_STATE, "integrate: call gpr_update_cache first");
+  if (m->spec.type[0] == KT_NOISE) return fail(ctx, GPR_ERR_UNSUPPORTED, "integrate: the first component must be a SquaredExp (antideriv!, src/integrate.jl:15)");
+  CK(cudaSetDevice(ctx->device));
+  timer_reset_predict(m->tm);
+  const int D = m->D;
+  const int64_t MT = std::min<int64_t>(ctx->predict_tile, round_up(nbox, 128));
+  int rc = ensure(ctx, m->w_xp, (size_t)2 * D * MT);
+  if (rc) return rc;
+  double* d_a = m->w_xp.p;
+  double* d_b = d_a + (size_t)D * MT;
+  std::vector<double> hsq(var_out ? (size_t)MT : 0);
+  for (int64_t m0 = 0; m0 < nbox; m0 += MT) {
+    const int64_t mt = std::min(MT, nbox - m0);
+    CK(cudaMemcpyAsync(d_a, a + m0 * D, sizeof(double) * D * mt, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_b, b + m0 * D, sizeof(double) * D * mt, cudaMemcpyHostToDevice, ctx->stream));
+    rc = integrate_tile(m, d_a, d_b, mt, Iout + m0, nbox, var_out ? hsq.data() : nullptr);
+    if (rc) return rc;
+    if (var_out)   // k2 - |U^-T k1|^2, hsq holding the negated sum  (:131-136)
+      for (int64_t i = 0; i < mt; ++i) var_out[m0 + i] = antideriv2_se(m->hp_host.data(), a + (m0 + i) * D, b + (m0 + i) * D, D) + hsq[i];
+  }
   return GPR_OK;
 }
 

@@ -59,6 +59,7 @@ _SIGS = {
     "gpr_timings": (C.c_int, [_vp, _dp, C.c_int]),
     "gpr_model_route": (C.c_int, [_vp, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "gpr_integrate": (C.c_int, [_vp, _dp, _dp, _dp, _dp]),
+    "gpr_integrate_batch": (C.c_int, [_vp, _i64, _dp, _dp, _dp, _dp]),
     "gpr_sample_mvn": (C.c_int, [_vp, _ip, C.c_int, C.c_int, _dp, _dp, _i64, C.c_double, _dp, _dp, _dp, C.POINTER(_i64)]),
     "gpr_dbg_dgemm": (C.c_int, [_vp, C.c_char, C.c_char, C.c_int, C.c_int, C.c_int, C.c_double, _dp, _i64, _dp, _i64,
                                 C.c_double, _dp, _i64, C.c_int, C.c_int, _dp]),
@@ -290,12 +291,16 @@ class ModelHandle:
         return mean, var
 
     def integrate(self, a, b, want_var=True):
-        a, b = f64(np.asarray(a, dtype=np.float64).ravel()), f64(np.asarray(b, dtype=np.float64).ravel())
-        if a.size != self.D or b.size != self.D:
-            raise GPRError("integration bounds must have one entry per input dimension")
-        Iout = np.empty(self.ny)
-        var = np.empty(1) if want_var else None
-        self.ctx.check(lib().gpr_integrate(self.handle, dptr(a), dptr(b), dptr(Iout), dptr(var)))
+        """a, b of shape (D,): gpr_integrate, (Iout (ny,), var (1,)); of shape (D, nbox): gpr_integrate_batch,
+        (Iout (nbox, ny), var (nbox,)), one triangular solve per tile of boxes."""
+        a, b, nbox, single = _box_args(a, b, self.D)
+        var = np.empty(nbox) if want_var else None
+        if single:
+            Iout = np.empty(self.ny)
+            self.ctx.check(lib().gpr_integrate(self.handle, dptr(a), dptr(b), dptr(Iout), dptr(var)))
+            return Iout, var
+        Iout = np.empty((nbox, self.ny), order="F")
+        self.ctx.check(lib().gpr_integrate_batch(self.handle, nbox, dptr(a), dptr(b), dptr(Iout), dptr(var)))
         return Iout, var
 
     def route(self):
@@ -319,6 +324,16 @@ class ModelHandle:
             self.close()
         except Exception:
             pass
+
+
+def _box_args(a, b, D):
+    """(a, b, nbox, single) of the integrate entry points: bounds of shape (D,) (one box) or (D, nbox), the same for a and b,
+    as D x nbox column-major arrays"""
+    a, b = np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64)
+    if a.shape != b.shape or a.ndim not in (1, 2) or a.shape[0] != D or a.ndim == 2 and a.shape[1] < 1:
+        raise GPRError("integration bounds must be (D,) or (D, nbox) arrays of the same shape")
+    single, nbox = a.ndim == 1, 1 if a.ndim == 1 else int(a.shape[1])
+    return f64(a.reshape(D, nbox)), f64(b.reshape(D, nbox)), nbox, single
 
 
 def _split_args(xe, xq, var_range, want_var, mean_out, var_out):
@@ -564,11 +579,7 @@ class MultiModelHandle:
     def integrate(self, a, b, want_var=True):
         """gpr_mgpu_integrate.  a, b of shape (D,): (Iout (ny,), var (1,)) as ModelHandle.integrate; of shape (D, nbox):
         (Iout (nbox, ny), var (nbox,)), one pass over K^-1 for all boxes."""
-        a, b = np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64)
-        if a.shape != b.shape or a.ndim not in (1, 2) or a.shape[0] != self.D or a.ndim == 2 and a.shape[1] < 1:
-            raise GPRError("integration bounds must be (D,) or (D, nbox) arrays of the same shape")
-        single, nbox = a.ndim == 1, 1 if a.ndim == 1 else int(a.shape[1])
-        a, b = f64(a.reshape(self.D, nbox)), f64(b.reshape(self.D, nbox))
+        a, b, nbox, single = _box_args(a, b, self.D)
         Iout = np.empty((nbox, self.ny), order="F")
         var = np.empty(nbox) if want_var else None
         self.mctx.check(lib().gpr_mgpu_integrate(self.handle, nbox, dptr(a), dptr(b), dptr(Iout), dptr(var)))

@@ -950,7 +950,8 @@ def integrate(md, *args, sample_noise=None, ctx=None, cache=None):
     sample_noise, one row per box as the single-box call returns it.
     cache: a MultiGPUGradCache / MultiGPUPredictCache of md; the factorizations then run block-cyclic on its devices
     (update_cache_ on that cache) and all boxes go through gpr_mgpu_integrate in one pass over K^-1.  Without it, one
-    device: gpr_integrate once per box."""
+    device: gpr_integrate for a single box, and gpr_integrate_batch for all boxes of a D x nbox batch in one call per
+    factorization (one triangular solve per tile of boxes)."""
     if len(args) == 2:
         hp, (a, b) = md.params, args
     else:
@@ -962,12 +963,7 @@ def integrate(md, *args, sample_noise=None, ctx=None, cache=None):
 
     def once(eps):
         update_cache_(wc, hp, md, ϵ=eps)
-        if multi or not batched:
-            return wc.handle.integrate(a2, b2, want_var=True)
-        if a2.shape != b2.shape or a2.shape[1] < 1:
-            raise GPRError("integration bounds must be (D,) or (D, nbox) arrays of the same shape")
-        res = [wc.handle.integrate(a2[:, i], b2[:, i], want_var=True) for i in range(a2.shape[1])]
-        return np.stack([r[0] for r in res]), np.concatenate([r[1] for r in res])
+        return wc.handle.integrate(a2, b2, want_var=True)
 
     try:
         if sample_noise is None:

@@ -173,6 +173,17 @@ int gpr_model_route(gpr_model* model, int* digits, int* digits_inverse);
  * Iout[e] = wt[:, e]^T k1 (e < ny), k1 = antideriv!(SquaredExp(), x, hp, a, b) (:15-31, reads hp[1..D+1] of the model);
  * var_out[0] = antideriv2(hp, a, b) - |U^-T k1|^2 (:33-41,131-136). */
 int gpr_integrate(gpr_model* model, const double* a, const double* b, double* Iout, double* var_out);
+/* integrate!(Iout, var_Iout, md, hp, a, b, nothing, wc, ac) (src/integrate.jl:56-62,103-143) for nbox boxes at once: for each
+ * box what gpr_integrate returns for it, with its preconditions and refusals (GPR_ERR_STATE unless the model holds a factor, at
+ * that factorization's hp and eps; GPR_ERR_UNSUPPORTED for a WhiteNoise first component).  GPR_ERR_ARG for NULL a, b, Iout or
+ * nbox < 1.  a, b: D x nbox (box i is column i).  Iout: nbox x ny, box index fastest (the layout of gpr_mgpu_integrate),
+ * Iout[i + e nbox] = wt[:, e]^T k1_i.  var_out: NULL or nbox entries, var_i = antideriv2(hp, a_i, b_i) - |U^-T k1_i|^2, not
+ * clamped.  The boxes are the test points of gpr_predict with k1 in place of K(x, xp): tiles of "predict_tile" boxes
+ * (GPR_ERR_MEMORY if one does not fit), each one k1 build, one T,N product against wt and one left triangular solve with U^T
+ * for all its boxes (on the DMMA pipe or the INT8 route, as the prediction solves), so many boxes per call cost about as much
+ * as one.  Timings: PRED_KSTAR = the k1 tile, PRED_MEAN = the wt^T k1 product and its download, PRED_TRSM = the triangular
+ * solve, PRED_ROWNORM = the column sums. */
+int gpr_integrate_batch(gpr_model* model, int64_t nbox, const double* a, const double* b, double* Iout, double* var_out);
 
 /* sample(gp(x, theta)) / sample(::NormalDistribution): src/distributions.jl:20-45 (row f-5 of SURVEY.md 8f).
  * Sigma = kernel(cov, theta, x) .+ shift  -- the reference adds 1e-7 to EVERY entry, not to the diagonal --

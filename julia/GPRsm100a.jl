@@ -343,31 +343,53 @@ end
 # (the shift rides in the jitter argument of gpr_update_cache, divided by the number of non-noise components because
 # every such component adds its own jitter, src/compose_covar.jl:53-55) instead of the eigendecomposition of :72-80.
 # ---------------------------------------------------------------------------------------------------------
-function _integrate_once(h::Handle, hp::Vector{Float64}, a::Vector{Float64}, b::Vector{Float64}, eps::Float64, ny::Int)
+# The noise-level bookkeeping of both methods below: once(eps) factors at jitter eps and integrates every box, returning
+# Iout (nbox x ny) and var (nbox).  Each distinct noise level is factored once; vectors a, b (single) give the shapes of the
+# reference's integrate, matrices Iout nbox x ny and var nbox (nbox x ny with sample_noise).
+function _integrate_levels(once, covar, nbox::Int, ny::Int, single::Bool, sample_noise)
+    if sample_noise === nothing
+        I, v = once(1e-8)
+        return single ? (I[1, :], v) : (I, v)
+    end
+    nk = count(k -> !(k isa WhiteNoise), covar isa ComposedKernel ? covar.kernels : (covar,))
+    if sample_noise isa Real
+        I, v = once(1e-8 + sample_noise / nk)
+        return single ? (I[1, :], fill(v[1], ny)) : (I, repeat(v, 1, ny))
+    end
+    Iout = Matrix{Float64}(undef, nbox, ny); var = similar(Iout)
+    levels = Dict{Float64,Tuple{Matrix{Float64},Vector{Float64}}}()
+    for (i, e) in enumerate(sample_noise)
+        haskey(levels, e) || (levels[e] = once(1e-8 + e / nk))
+        I, v = levels[e]
+        Iout[:, i] = I[:, i]; var[:, i] = v
+    end
+    single ? (Iout[1, :], var[1, :]) : (Iout, var)
+end
+
+# a, b vectors: gpr_integrate for the one box; D x nbox matrices (box i = column i): gpr_integrate_batch for all boxes at
+# once, one triangular solve per tile of boxes instead of one per box.
+function _integrate_once(h::Handle, hp::Vector{Float64}, a::VecOrMat{Float64}, b::VecOrMat{Float64}, eps::Float64, ny::Int)
     info = Ref{Int64}(0)
     check(h.c, ccall((:gpr_update_cache, LIB), Cint, (Ptr{Cvoid}, Ptr{Float64}, Cint, Cdouble, Cint, Ref{Int64}),
         h.h, hp, length(hp), eps, 0, info), info[])
-    Iout = Vector{Float64}(undef, ny); v = Vector{Float64}(undef, 1)
-    check(h.c, ccall((:gpr_integrate, LIB), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
-        h.h, a, b, Iout, v))
-    Iout, v[1]
+    nbox = size(a, 2)
+    Iout = Matrix{Float64}(undef, nbox, ny); v = Vector{Float64}(undef, nbox)
+    if a isa Vector
+        check(h.c, ccall((:gpr_integrate, LIB), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+            h.h, a, b, Iout, v))
+    else
+        check(h.c, ccall((:gpr_integrate_batch, LIB), Cint,
+            (Ptr{Cvoid}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}), h.h, nbox, a, b, Iout, v))
+    end
+    Iout, v
 end
 function integrate_sm100(md::GPRModel, hp, a, b; sample_noise = nothing)
     h = Handle(md)                       # device model (x, y uploaded once), freed by its finalizer
     ny = size(md.y, 2)
-    nk = count(k -> !(k isa WhiteNoise), md.covar isa ComposedKernel ? md.covar.kernels : (md.covar,))
-    hpv, av, bv = Vector{Float64}(hp), Vector{Float64}(a), Vector{Float64}(b)
-    sample_noise === nothing && (r = _integrate_once(h, hpv, av, bv, 1e-8, ny); return r[1], [r[2]])
-    if sample_noise isa Real
-        I, v = _integrate_once(h, hpv, av, bv, 1e-8 + sample_noise / nk, ny)
-        return I, fill(v, ny)
-    end
-    Iout = Vector{Float64}(undef, ny); var = similar(Iout)
-    for (i, e) in enumerate(sample_noise)
-        I, v = _integrate_once(h, hpv, av, bv, 1e-8 + e / nk, ny)
-        Iout[i] = I[i]; var[i] = v
-    end
-    Iout, var
+    single = a isa AbstractVector
+    hpv = Vector{Float64}(hp)
+    av, bv = single ? (Vector{Float64}(a), Vector{Float64}(b)) : (Matrix{Float64}(a), Matrix{Float64}(b))
+    _integrate_levels(eps -> _integrate_once(h, hpv, av, bv, eps, ny), md.covar, size(av, 2), ny, single, sample_noise)
 end
 
 # The same on the distributed model of SM100Multi: one gpr_mgpu_update_cache per distinct noise level, then
@@ -386,26 +408,10 @@ end
 function integrate_sm100(s::SM100Multi, hp, a, b; sample_noise = nothing)
     h, _, _ = _multi_model(s.md, s.devices, s.nb)
     ny = size(s.md.y, 2)
-    nk = count(k -> !(k isa WhiteNoise), s.md.covar isa ComposedKernel ? s.md.covar.kernels : (s.md.covar,))
-    single = a isa AbstractVector
     hpv = Vector{Float64}(hp)
     am = Matrix{Float64}(reshape(a, size(a, 1), :)); bm = Matrix{Float64}(reshape(b, size(b, 1), :))
-    if sample_noise === nothing
-        I, v = _mintegrate_once(h, hpv, am, bm, 1e-8, ny)
-        return single ? (I[1, :], v) : (I, v)
-    end
-    if sample_noise isa Real
-        I, v = _mintegrate_once(h, hpv, am, bm, 1e-8 + sample_noise / nk, ny)
-        return single ? (I[1, :], fill(v[1], ny)) : (I, repeat(v, 1, ny))
-    end
-    Iout = Matrix{Float64}(undef, size(am, 2), ny); var = similar(Iout)
-    levels = Dict{Float64,Tuple{Matrix{Float64},Vector{Float64}}}()
-    for (i, e) in enumerate(sample_noise)
-        haskey(levels, e) || (levels[e] = _mintegrate_once(h, hpv, am, bm, 1e-8 + e / nk, ny))
-        I, v = levels[e]
-        Iout[:, i] = I[:, i]; var[:, i] = v
-    end
-    single ? (Iout[1, :], var[1, :]) : (Iout, var)
+    _integrate_levels(eps -> _mintegrate_once(h, hpv, am, bm, eps, ny), s.md.covar, size(am, 2), ny, a isa AbstractVector,
+                      sample_noise)
 end
 
 end # module
