@@ -14,7 +14,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libgpr_sm100a.so")
 SOURCES = ["gpr_api.cu"]
-DEPS = ["gpr_api.cu", "kbuild_tma.cuh", "dgemm_tma.cuh", "ozaki_i8.cuh", "fastexp.cuh", "mgpu_api.inl", "dist_blocked.hpp", "blocked.hpp", "cov_kernels.cuh", "dgemm_sm100.cuh", "leaf_kernels.cuh",
+DEPS = ["gpr_api.cu", "kbuild_tma.cuh", "dgemm_tma.cuh", "ozaki_i8.cuh", "fastexp.cuh", "mgpu_api.inl", "dist_blocked.hpp", "blocked.hpp", "cov_kernels.cuh", "grad_wide.cuh", "dgemm_sm100.cuh", "leaf_kernels.cuh",
         os.path.join(ROOT, "include", "gpr_sm100a.h")]
 NVCC_FLAGS = ["-shared", "-Xcompiler", "-fPIC", "-O3", "-std=c++17",
               "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo"]

@@ -69,10 +69,18 @@ __device__ __forceinline__ double kern_value(int type, double sig2, double dist)
   return sig2 * (1.0 + s5r + (5.0 / 3.0) * dist) * exp(-s5r);
 }
 
+// Coordinates per chunk of the wide covariance build and the pitch of its d-major point tiles (odd in doubles: the
+// staging stores, consecutive coordinates of one point, fall in distinct banks).
+constexpr int KBW_DC = 32;
+constexpr int KBW_P = KB_TILE + 1;
+
 // out[r + c*ldo] = sum_comp k_comp(x1[:,r], x2[:,c]) (+ jitter, + noise, padding)
-// smem: xs1[nk][D][64], xs2[nk][D][64] = inverse-length-scaled coordinates (the
-// reference scales x by l before taking differences: covariance.jl:90-92).
-template <int MODE>
+// WIDE = false: smem xs1[nk][D][64], xs2[nk][D][64] = inverse-length-scaled coordinates (the reference
+// scales x by l before taking differences: covariance.jl:90-92), all staged at once.
+// WIDE = true (the wide build): one component at a time, its scaled coordinates staged KBW_DC at a time
+// (smem xs1[KBW_DC][KBW_P], xs2[KBW_DC][KBW_P]), distances accumulated in registers in the same order over d, so any D
+// and any number of components fit.
+template <int MODE, bool WIDE = false>
 __global__ void __launch_bounds__(KB_THREADS) kbuild_kernel(const KBuildArgs a) {
   extern __shared__ __align__(16) double kb_smem[];
   const int D = a.D;
@@ -98,15 +106,17 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_kernel(const KBuildArgs a) 
     if (c < a.spec.ncomp && a.spec.type[c] != KT_NOISE) kidx[nk++] = c;
 
   double* xs1 = kb_smem;
-  double* xs2 = kb_smem + (size_t)nk * D * KB_TILE;
-  for (int idx = tid; idx < nk * D * KB_TILE; idx += KB_THREADS) {
-    const int p = idx % KB_TILE, d = (idx / KB_TILE) % D, k = idx / (KB_TILE * D);
-    const double l = a.hp[a.spec.hp_off[kidx[k]] + 1 + d];
-    const long long r = r0 + p, c = c0 + p;
-    xs1[idx] = (r < a.R) ? a.x1[d + r * D] * l : 0.0;
-    xs2[idx] = (c < a.C) ? a.x2[d + c * D] * l : 0.0;
+  double* xs2 = WIDE ? kb_smem + (size_t)KBW_DC * KBW_P : kb_smem + (size_t)nk * D * KB_TILE;
+  if constexpr (!WIDE) {
+    for (int idx = tid; idx < nk * D * KB_TILE; idx += KB_THREADS) {
+      const int p = idx % KB_TILE, d = (idx / KB_TILE) % D, k = idx / (KB_TILE * D);
+      const double l = a.hp[a.spec.hp_off[kidx[k]] + 1 + d];
+      const long long r = r0 + p, c = c0 + p;
+      xs1[idx] = (r < a.R) ? a.x1[d + r * D] * l : 0.0;
+      xs2[idx] = (c < a.C) ? a.x2[d + c * D] * l : 0.0;
+    }
+    __syncthreads();
   }
-  __syncthreads();
 
   double sum[4][4];
 #pragma unroll
@@ -123,22 +133,58 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_kernel(const KBuildArgs a) 
     for (int i = 0; i < 4; ++i)
 #pragma unroll
       for (int j = 0; j < 4; ++j) dist[i][j] = 0.0;
-    const double* p1 = xs1 + (size_t)k * D * KB_TILE;
-    const double* p2 = xs2 + (size_t)k * D * KB_TILE;
-    for (int d = 0; d < D; ++d) {
-      double u[4], v[4];
+    if constexpr (!WIDE) {
+      const double* p1 = xs1 + (size_t)k * D * KB_TILE;
+      const double* p2 = xs2 + (size_t)k * D * KB_TILE;
+      for (int d = 0; d < D; ++d) {
+        double u[4], v[4];
 #pragma unroll
-      for (int i = 0; i < 4; ++i) u[i] = p1[d * KB_TILE + tx + 16 * i];
+        for (int i = 0; i < 4; ++i) u[i] = p1[d * KB_TILE + tx + 16 * i];
 #pragma unroll
-      for (int j = 0; j < 4; ++j) v[j] = p2[d * KB_TILE + ty + 16 * j];
+        for (int j = 0; j < 4; ++j) v[j] = p2[d * KB_TILE + ty + 16 * j];
 #pragma unroll
-      for (int i = 0; i < 4; ++i)
+        for (int i = 0; i < 4; ++i)
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          if (MODE == DM_EUCLID) { const double df = u[i] - v[j]; dist[i][j] += df * df; }
-          else if (MODE == DM_SPLIT_A) dist[i][j] += v[j] * v[j] + 2.0 * u[i] * v[j];   // split_kernel.jl:114
-          else dist[i][j] += -2.0 * u[i] * v[j];                                       // split_kernel.jl:121
+          for (int j = 0; j < 4; ++j) {
+            if (MODE == DM_EUCLID) { const double df = u[i] - v[j]; dist[i][j] += df * df; }
+            else if (MODE == DM_SPLIT_A) dist[i][j] += v[j] * v[j] + 2.0 * u[i] * v[j];   // split_kernel.jl:114
+            else dist[i][j] += -2.0 * u[i] * v[j];                                       // split_kernel.jl:121
+          }
+      }
+    } else {
+      const double* lsc = a.hp + a.spec.hp_off[comp] + 1;
+      for (int d0 = 0; d0 < D; d0 += KBW_DC) {
+        const int nd = D - d0 < KBW_DC ? D - d0 : KBW_DC;
+        __syncthreads();   // the previous chunk has been read
+        // consecutive threads read consecutive coordinates of one point (coalesced)
+        for (int idx = tid; idx < 2 * KB_TILE * KBW_DC; idx += KB_THREADS) {
+          const int d = idx % KBW_DC, p = (idx / KBW_DC) % KB_TILE;
+          if (d >= nd) continue;
+          if (idx < KB_TILE * KBW_DC) {
+            const long long r = r0 + p;
+            xs1[d * KBW_P + p] = (r < a.R) ? a.x1[d0 + d + r * D] * lsc[d0 + d] : 0.0;
+          } else {
+            const long long c = c0 + p;
+            xs2[d * KBW_P + p] = (c < a.C) ? a.x2[d0 + d + c * D] * lsc[d0 + d] : 0.0;
+          }
         }
+        __syncthreads();
+        for (int d = 0; d < nd; ++d) {   // the same arithmetic as above, in the same order over d
+          double u[4], v[4];
+#pragma unroll
+          for (int i = 0; i < 4; ++i) u[i] = xs1[d * KBW_P + tx + 16 * i];
+#pragma unroll
+          for (int j = 0; j < 4; ++j) v[j] = xs2[d * KBW_P + ty + 16 * j];
+#pragma unroll
+          for (int i = 0; i < 4; ++i)
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+              if (MODE == DM_EUCLID) { const double df = u[i] - v[j]; dist[i][j] += df * df; }
+              else if (MODE == DM_SPLIT_A) dist[i][j] += v[j] * v[j] + 2.0 * u[i] * v[j];
+              else dist[i][j] += -2.0 * u[i] * v[j];
+            }
+        }
+      }
     }
 #pragma unroll
     for (int i = 0; i < 4; ++i)
@@ -217,6 +263,10 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_kernel(const KBuildArgs a) 
     }
   }
 }
+
+// dynamic shared memory of kbuild_kernel<MODE, true> (the fused-mean reductions reuse the point tiles)
+constexpr size_t KBW_SMEM_BYTES = (size_t)2 * KBW_DC * KBW_P * sizeof(double);
+static_assert(KBW_SMEM_BYTES >= (size_t)16 * (KB_TILE + 1) * sizeof(double), "fused-mean reduction buffer");
 
 // Dense dK/dtheta for ONE non-noise component (API parity with grad(cov,i,hp,x):
 // /root/reference/src/deriv_covar.jl:2-29).  li = local hyper-parameter index
@@ -422,28 +472,24 @@ __global__ void __launch_bounds__(GR_THREADS) grad_reduce_kernel(const GradArgs 
 
 // G[p] from the block partials.  sigma: -acc/|sigma| ; l_d: +l_d * acc ; noise: -sigma_n * acc_diag
 // (loss_grad.jl:43-52 with deriv_covar.jl:23,26,31).  log_scale: G .*= hp (cost.jl:65).
+// Every thread sums the slots it needs over the blocks in block order, so any P is taken.
 __global__ void grad_finalize_kernel(const double* __restrict__ partial, int nblocks, int P, const double* __restrict__ hp,
                                      KSpec spec, int D, int log_scale, double* __restrict__ G) {
-  __shared__ double tot[256];
-  const int tid = threadIdx.x;
-  for (int s = tid; s <= P && s < 256; s += blockDim.x) {
+  auto tot = [&](int s) {
     double v = 0.0;
     for (int b = 0; b < nblocks; ++b) v += partial[(size_t)b * (P + 1) + s];
-    tot[s] = v;
-  }
-  __syncthreads();
-  if (tid == 0) {
-    for (int c = 0; c < spec.ncomp; ++c) {
-      const int off = spec.hp_off[c];
-      if (spec.type[c] == KT_NOISE) {
-        G[off] = -hp[off] * tot[P];
-      } else {
-        G[off] = -tot[off] / fabs(hp[off]);
-        for (int d = 0; d < D; ++d) G[off + 1 + d] = hp[off + 1 + d] * tot[off + 1 + d];
-      }
-    }
-    if (log_scale)
-      for (int p = 0; p < P; ++p) G[p] *= hp[p];
+    return v;
+  };
+  for (int p = threadIdx.x; p < P; p += blockDim.x) {
+    int c = 0;
+    while (c + 1 < spec.ncomp && spec.hp_off[c + 1] <= p) ++c;
+    const int off = spec.hp_off[c];
+    double v;
+    if (spec.type[c] == KT_NOISE) v = -hp[off] * tot(P);
+    else if (p == off) v = -tot(off) / fabs(hp[off]);
+    else v = hp[p] * tot(p);
+    if (log_scale) v *= hp[p];
+    G[p] = v;
   }
 }
 
@@ -561,37 +607,79 @@ __device__ __forceinline__ double erf_between(double x, double y) {
 // rows >= n (padding of the factor) and columns >= nbox (padding of the tile) are zero.  Threads run along the training
 // index (coalesced stores); each CTA stages ANTIDERIV_BOXES boxes' bounds in shared memory (2 D ANTIDERIV_BOXES doubles of
 // dynamic shared memory) and walks the box chunks blockIdx.y, blockIdx.y + gridDim.y, ...
+// CHUNKED: the bounds are staged ANTIDERIV_DCH coordinates at a time (2 ANTIDERIV_DCH ANTIDERIV_BOXES doubles), the
+// products carried in registers across the chunks in the same order over i, for D whose bounds exceed shared memory.
 constexpr int ANTIDERIV_BOXES = 8;
+constexpr int ANTIDERIV_DCH = 1024;
+template <bool CHUNKED = false>
 __global__ void __launch_bounds__(256) antideriv_se_kernel(const double* __restrict__ x, int D, long long n, long long np,
                                                            const double* __restrict__ hp, const double* __restrict__ a,
                                                            const double* __restrict__ b, long long nbox, long long mtp,
                                                            double* __restrict__ k1, long long ldk) {
   extern __shared__ double sab[];   // [a | b] of the chunk, D x ANTIDERIV_BOXES each
   const long long j = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-  const int nab = D * ANTIDERIV_BOXES;
-  for (long long c0 = (long long)blockIdx.y * ANTIDERIV_BOXES; c0 < mtp; c0 += (long long)gridDim.y * ANTIDERIV_BOXES) {
-    __syncthreads();
-    for (int t = threadIdx.x; t < 2 * nab; t += blockDim.x) {
-      const long long o = c0 * D + (t % nab);
-      sab[t] = o < nbox * D ? (t < nab ? a[o] : b[o]) : 0.0;
-    }
-    __syncthreads();
-    if (j >= np) continue;
-    for (int cc = 0; cc < ANTIDERIV_BOXES && c0 + cc < mtp; ++cc) {
-      const long long c = c0 + cc;
-      double out = 0.0;
-      if (j < n && c < nbox) {
-        const double* ac = sab + cc * D;
-        const double* bc = sab + nab + cc * D;
-        double prefac = hp[0] * hp[0], v = 1.0;
-        for (int i = 0; i < D; ++i) {
-          const double l = hp[1 + i], xij = x[i + j * D];
-          prefac *= 0.88622692545275801365 / l;
-          v *= erf_between(l * (ac[i] - xij), l * (bc[i] - xij));
-        }
-        out = v * prefac;
+  if constexpr (!CHUNKED) {
+    const int nab = D * ANTIDERIV_BOXES;
+    for (long long c0 = (long long)blockIdx.y * ANTIDERIV_BOXES; c0 < mtp; c0 += (long long)gridDim.y * ANTIDERIV_BOXES) {
+      __syncthreads();
+      for (int t = threadIdx.x; t < 2 * nab; t += blockDim.x) {
+        const long long o = c0 * D + (t % nab);
+        sab[t] = o < nbox * D ? (t < nab ? a[o] : b[o]) : 0.0;
       }
-      k1[j + c * ldk] = out;
+      __syncthreads();
+      if (j >= np) continue;
+      for (int cc = 0; cc < ANTIDERIV_BOXES && c0 + cc < mtp; ++cc) {
+        const long long c = c0 + cc;
+        double out = 0.0;
+        if (j < n && c < nbox) {
+          const double* ac = sab + cc * D;
+          const double* bc = sab + nab + cc * D;
+          double prefac = hp[0] * hp[0], v = 1.0;
+          for (int i = 0; i < D; ++i) {
+            const double l = hp[1 + i], xij = x[i + j * D];
+            prefac *= 0.88622692545275801365 / l;
+            v *= erf_between(l * (ac[i] - xij), l * (bc[i] - xij));
+          }
+          out = v * prefac;
+        }
+        k1[j + c * ldk] = out;
+      }
+    }
+  } else {
+    const int nab = ANTIDERIV_DCH * ANTIDERIV_BOXES;   // sab: a[cc][i], b[cc][i] of coordinates d0 + i
+    for (long long c0 = (long long)blockIdx.y * ANTIDERIV_BOXES; c0 < mtp; c0 += (long long)gridDim.y * ANTIDERIV_BOXES) {
+      double prefac[ANTIDERIV_BOXES], v[ANTIDERIV_BOXES];
+#pragma unroll
+      for (int cc = 0; cc < ANTIDERIV_BOXES; ++cc) { prefac[cc] = hp[0] * hp[0]; v[cc] = 1.0; }
+      for (int d0 = 0; d0 < D; d0 += ANTIDERIV_DCH) {
+        const int nd = D - d0 < ANTIDERIV_DCH ? D - d0 : ANTIDERIV_DCH;
+        __syncthreads();
+        for (int t = threadIdx.x; t < 2 * nab; t += blockDim.x) {
+          const int cc = (t % nab) / ANTIDERIV_DCH, i = t % ANTIDERIV_DCH;
+          const long long c = c0 + cc;
+          sab[t] = (i < nd && c < nbox) ? (t < nab ? a : b)[c * D + d0 + i] : 0.0;
+        }
+        __syncthreads();
+        if (j >= n) continue;
+#pragma unroll
+        for (int cc = 0; cc < ANTIDERIV_BOXES; ++cc) {
+          if (c0 + cc >= nbox) continue;
+          const double* ac = sab + cc * ANTIDERIV_DCH;
+          const double* bc = sab + nab + cc * ANTIDERIV_DCH;
+          for (int i = 0; i < nd; ++i) {
+            const double l = hp[1 + d0 + i], xij = x[d0 + i + j * D];
+            prefac[cc] *= 0.88622692545275801365 / l;
+            v[cc] *= erf_between(l * (ac[i] - xij), l * (bc[i] - xij));
+          }
+        }
+      }
+      if (j >= np) continue;
+#pragma unroll
+      for (int cc = 0; cc < ANTIDERIV_BOXES; ++cc) {
+        const long long c = c0 + cc;
+        if (c >= mtp) break;
+        k1[j + c * ldk] = (j < n && c < nbox) ? v[cc] * prefac[cc] : 0.0;
+      }
     }
   }
 }

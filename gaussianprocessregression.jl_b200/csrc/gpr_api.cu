@@ -22,6 +22,7 @@
 #include "cov_kernels.cuh"
 #include "dgemm_sm100.cuh"
 #include "kbuild_tma.cuh"
+#include "grad_wide.cuh"
 #include "dgemm_tma.cuh"
 #include "ozaki_i8.cuh"
 #include "leaf_kernels.cuh"
@@ -315,6 +316,11 @@ int setup_kernel_attributes(gpr_ctx* ctx) {
   CK(cudaFuncSetAttribute(kbuild_gram_kernel<DM_SPLIT_C>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   CK(cudaFuncSetAttribute(grad_reduce_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   CK(cudaFuncSetAttribute(grad_reduce_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  CK(cudaFuncSetAttribute(kbuild_kernel<DM_EUCLID, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)KBW_SMEM_BYTES));
+  CK(cudaFuncSetAttribute(kbuild_kernel<DM_SPLIT_A, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)KBW_SMEM_BYTES));
+  CK(cudaFuncSetAttribute(kbuild_kernel<DM_SPLIT_C, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)KBW_SMEM_BYTES));
+  CK(cudaFuncSetAttribute(grad_reduce_wide_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GW_SMEM_BYTES));
+  CK(cudaFuncSetAttribute(grad_reduce_wide_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GW_SMEM_BYTES));
   return GPR_OK;
 }
 
@@ -352,15 +358,30 @@ int launch_kbuild(gpr_ctx* ctx, int mode, const KBuildArgs& a, const double* cen
   }
   size_t smem = (size_t)2 * nk * a.D * KB_TILE * sizeof(double);
   if (a.mean_w || a.mean_w_rows) smem = std::max(smem, (size_t)16 * (KB_TILE + 1) * sizeof(double));
-  if (smem > 200 * 1024) return fail(ctx, GPR_ERR_UNSUPPORTED, "covariance build: (#components x D) too large for shared memory");
   dim3 grid((unsigned)((a.Rp + KB_TILE - 1) / KB_TILE), (unsigned)((a.Cp + KB_TILE - 1) / KB_TILE));
   if (grid.y > 65535) return fail(ctx, GPR_ERR_UNSUPPORTED, "covariance build: too many column tiles");
-  if (mode == DM_EUCLID) kbuild_kernel<DM_EUCLID><<<grid, KB_THREADS, smem, ctx->stream>>>(a);
+  if (smem > 200 * 1024) {
+    // the scaled point tiles of all components do not fit: stage them one component and KBW_DC coordinates at a time
+    if (mode == DM_EUCLID) kbuild_kernel<DM_EUCLID, true><<<grid, KB_THREADS, KBW_SMEM_BYTES, ctx->stream>>>(a);
+    else if (mode == DM_SPLIT_A) kbuild_kernel<DM_SPLIT_A, true><<<grid, KB_THREADS, KBW_SMEM_BYTES, ctx->stream>>>(a);
+    else kbuild_kernel<DM_SPLIT_C, true><<<grid, KB_THREADS, KBW_SMEM_BYTES, ctx->stream>>>(a);
+  } else if (mode == DM_EUCLID) kbuild_kernel<DM_EUCLID><<<grid, KB_THREADS, smem, ctx->stream>>>(a);
   else if (mode == DM_SPLIT_A) kbuild_kernel<DM_SPLIT_A><<<grid, KB_THREADS, smem, ctx->stream>>>(a);
   else kbuild_kernel<DM_SPLIT_C><<<grid, KB_THREADS, smem, ctx->stream>>>(a);
   ctx->launches++;
   CK(cudaGetLastError());
   return GPR_OK;
+}
+
+// fused gradient reduction (partial[block][P+1], a.P and a.D set): grad_reduce_kernel where its per-thread accumulators and
+// point tiles fit in shared memory, the wide form (csrc/grad_wide.cuh: O(P) state per CTA, DMMA contractions over D in
+// chunks) otherwise.  Shared by the single-GPU and the block-cyclic multi-GPU gradient.
+template <bool DIST>
+cudaError_t launch_grad_reduce(cudaStream_t st, const GradArgs& a, int blocks) {
+  const size_t smem = ((size_t)(a.P + 1) * GR_THREADS + 2 * (size_t)a.D * GR_TILE + 2 * GR_TILE + 32) * sizeof(double);
+  if (smem <= 200 * 1024) grad_reduce_kernel<DIST><<<blocks, GR_THREADS, smem, st>>>(a);
+  else grad_reduce_wide_kernel<DIST><<<blocks, GR_THREADS, GW_SMEM_BYTES, st>>>(a);
+  return cudaGetLastError();
 }
 
 // rows of the output one CTA of the covariance build covers (the fused-mean partials are per CTA row tile)
@@ -507,13 +528,23 @@ double antideriv2_se(const double* hp, const double* a, const double* b, int D) 
   return k2;
 }
 
+// largest dynamic shared memory a CTA can opt in to on sm_100 (227 KB)
+constexpr size_t ANTIDERIV_SMEM_MAX = 227 * 1024;
+
 // k1 tile of nbox boxes on ctx's queue (antideriv_se_kernel: np x mtp, ld ldk; a, b D x nbox on the device)
 int launch_antideriv(gpr_ctx* ctx, const double* x, int D, int64_t n, int64_t np, const double* hp, const double* a,
                      const double* b, int64_t nbox, int64_t mtp, double* k1, int64_t ldk) {
   const size_t smem = sizeof(double) * 2 * D * ANTIDERIV_BOXES;
-  if (smem > 48 * 1024) CK(cudaFuncSetAttribute(antideriv_se_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const dim3 grid((unsigned)((np + 255) / 256), (unsigned)std::min<int64_t>((mtp + ANTIDERIV_BOXES - 1) / ANTIDERIV_BOXES, 65535));
-  antideriv_se_kernel<<<grid, 256, smem, ctx->stream>>>(x, D, n, np, hp, a, b, nbox, mtp, k1, ldk);
+  if (smem > ANTIDERIV_SMEM_MAX) {
+    // the bounds of D coordinates exceed the 227 KB a CTA can have: stage them ANTIDERIV_DCH coordinates at a time
+    const size_t smem_c = sizeof(double) * 2 * ANTIDERIV_DCH * ANTIDERIV_BOXES;
+    CK(cudaFuncSetAttribute(antideriv_se_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_c));
+    antideriv_se_kernel<true><<<grid, 256, smem_c, ctx->stream>>>(x, D, n, np, hp, a, b, nbox, mtp, k1, ldk);
+  } else {
+    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(antideriv_se_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    antideriv_se_kernel<false><<<grid, 256, smem, ctx->stream>>>(x, D, n, np, hp, a, b, nbox, mtp, k1, ldk);
+  }
   ctx->launches++;
   CK(cudaGetLastError());
   return GPR_OK;
@@ -685,10 +716,8 @@ int compute_grad(gpr_model* m, int log_scale, double* G_host) {
     a.Kinv = m->d_Kinv; a.ld = m->Np; a.alpha = m->d_wt + (int64_t)(m->train_axis - 1) * m->Np;
     a.x = m->d_x; a.D = m->D; a.N = m->N; a.hp = m->d_hp; a.spec = m->spec; a.P = m->P; a.eps = m->eps_host;
     a.partial = m->d_gpart;
-    const size_t smem = ((size_t)(m->P + 1) * GR_THREADS + 2 * (size_t)m->D * GR_TILE + 2 * GR_TILE + 32) * sizeof(double);
-    grad_reduce_kernel<false><<<m->gr_blocks, GR_THREADS, smem, ctx->stream>>>(a);
+    CK(launch_grad_reduce<false>(ctx->stream, a, m->gr_blocks));
     ctx->launches++;
-    CK(cudaGetLastError());
     grad_finalize_kernel<<<1, 256, 0, ctx->stream>>>(m->d_gpart, m->gr_blocks, m->P, m->d_hp, m->spec, m->D, log_scale, m->d_G);
     ctx->launches++;
     CK(cudaGetLastError());
@@ -846,7 +875,6 @@ int gpr_model_create(gpr_ctx* ctx, const int* comp_types, int ncomp, int D, int6
   m->ctx = ctx;
   int rc = make_spec(ctx, comp_types, ncomp, D, &m->spec, &m->P, &m->nk);
   if (rc) { delete m; return rc; }
-  if (m->P > 90) { delete m; return fail(ctx, GPR_ERR_UNSUPPORTED, "more than 90 hyper-parameters are not supported"); }
   timer_init(m->tm);
   m->types.assign(comp_types, comp_types + ncomp);
   m->ncomp = ncomp; m->D = D; m->N = N; m->Np = round_up(N, 128); m->ny = ny; m->train_axis = train_axis;

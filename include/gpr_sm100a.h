@@ -108,9 +108,11 @@ int64_t gpr_ctx_launch_count(gpr_ctx* ctx);        /* kernels launched by this c
 int gpr_dim_hp(const int* comp_types, int ncomp, int D);
 
 /* GPRModel(cov, hp, x, y; train_axis): src/models.jl:17-37.  train_axis is 1-based.
- * Limits of this implementation (the reference has none): at most 8 kernel components (GPR_ERR_ARG beyond) and at most 90
- * hyper-parameters in all (GPR_ERR_UNSUPPORTED beyond: the fused gradient reduction keeps one shared-memory accumulator per
- * hyper-parameter and thread).  Both fail at creation, never silently. */
+ * Limits of this implementation (the reference has none): at most 8 kernel components (GPR_ERR_ARG beyond, at creation).
+ * Any D and any hyper-parameter count are taken (tested up to D = 1024 with 8 components): shapes whose point tiles or
+ * per-thread gradient accumulators do not fit in shared memory run a covariance build that stages the coordinates in chunks
+ * and a gradient reduction with O(P) state per CTA instead; box integration stages its bounds in chunks of coordinates
+ * beyond D = 1816.  Tested up to D = 2048 for box integration. */
 int gpr_model_create(gpr_ctx* ctx, const int* comp_types, int ncomp, int D, int64_t N, const double* x,
                      const double* y, int ny, int train_axis, gpr_model** model);
 int gpr_model_destroy(gpr_model* model);
